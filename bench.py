@@ -2,6 +2,7 @@
 """Benchmark of the batched paint-simulation step (BASELINE.json metric: batched env steps/s).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c3|c3_late|c4|c5] [--impl reference]
+                    [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1), environments sharded by index, no collective on the
 step path.  A "step" is one `paintrl_step` over the whole per-GPU batch with random actions that
@@ -74,6 +75,7 @@ WORKLOADS = {
 METRIC = 'batched env steps/sec'
 UNIT = 'env-steps/s'
 N_SMS = 148
+DUMP_BYTES = 60 << 20      # --dump-outputs: the .npy files stay under 64 MB, headers included
 
 
 def measured_peaks():
@@ -181,6 +183,23 @@ def pin_to_gpu_numa_node(index):
     return None
 
 
+def dump_outputs(out_dir, arrays, env_axis=0):
+    """--dump-outputs: `arrays` (name -> device tensor, environments along `env_axis`) as out_dir/<name>.npy, float32
+    tensors and flags in float32, everything else in float64, and the environments written as env_ids.npy.  Above
+    DUMP_BYTES in all, a fixed seeded sample of the environments is written, the same one in every run."""
+    import torch
+    n_env = next(iter(arrays.values())).shape[env_axis]
+    as_f32 = {k: t.dtype in (torch.float32, torch.uint8, torch.bool) for k, t in arrays.items()}
+    per_env = 8 + sum((4 if as_f32[k] else 8) * (t.numel() // n_env) for k, t in arrays.items())
+    keep = min(n_env, DUMP_BYTES // per_env)
+    ids = np.arange(n_env) if keep == n_env else np.sort(np.random.default_rng(0).choice(n_env, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, 'env_ids.npy'), ids.astype(np.float64))
+    for k, t in arrays.items():
+        rows = t.index_select(env_axis, torch.as_tensor(ids, device=t.device)).cpu().numpy()
+        np.save(os.path.join(out_dir, k + '.npy'), rows.astype(np.float32 if as_f32[k] else np.float64))
+
+
 def workload_pack(workload, cfg, rasterizer='oracle'):
     """The part pack of a workload for the CPU legs (texels of synthetic textures from the oracle's own rasteriser)."""
     from paintrl_b200.partpack import PartPack
@@ -267,7 +286,7 @@ def run_reference(args, workload, rank, world_size):
     print(json.dumps(line), flush=True)
 
 
-def run_rollout(args, workload, env, cfg, rank, world_size, device, warmup):
+def run_rollout(args, workload, env, cfg, rank, world_size, device, warmup, dump_dir=None):
     """--rollout: fragments of 100 steps collected by paintrl_b200.rollout (policy obs->256->128->{logits, value}
     evaluated and sampled on the GPU, paint_ppo.py:179-190), one all-reduce of rollout statistics per fragment."""
     import torch
@@ -300,6 +319,10 @@ def run_rollout(args, workload, env, cfg, rank, world_size, device, warmup):
     if world_size > 1:
         dist.barrier()
     clocks = sampler.stop()
+    if dump_dir and rank == 0:
+        f = worker.frag
+        dump_outputs(dump_dir, {k: getattr(f, k) for k in ('obs', 'term_obs', 'actions', 'reward', 'penalty', 'actual', 'done',
+                                                          'new_texels', 'logp', 'value')}, env_axis=1)
     s1 = env.stats()
     t = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=device)
     if world_size > 1:
@@ -324,10 +347,32 @@ def run_rollout(args, workload, env, cfg, rank, world_size, device, warmup):
         dist.destroy_process_group()
 
 
-def measure(key, args, rank, local_rank, world_size, device, steps, warmup, e2e=True, parity_envs=128, rollout=False):
+def seeded_inputs(env, cfg, rank, device, steps, warmup, e2e):
+    """The step benchmark's inputs, seeded by rank: random actions [rows, n_env(, action_dim)] for the warm-up, timed
+    and e2e steps, and one start index per environment.  Returns (actions, start, e2e_steps)."""
+    import torch
+    n_env = env.num_envs
+    gen = torch.Generator(device=device)
+    gen.manual_seed(1234 + rank)
+    e2e_steps = max(10, min(steps, 200)) if e2e else 0
+    total = warmup + max(steps, e2e_steps)
+    if cfg.action_mode == 'discrete':
+        actions = torch.randint(0, cfg.discrete_granularity, (total, n_env), generator=gen, device=device,
+                                dtype=torch.int64)
+    else:
+        actions = torch.rand((total, n_env, cfg.action_dim), generator=gen, device=device, dtype=torch.float64) * 2 - 1
+    gs = torch.Generator(device=device)
+    gs.manual_seed(rank)
+    start = torch.randint(0, env.n_starts, (n_env,), generator=gs, device=device, dtype=torch.int32)
+    return actions, start, e2e_steps
+
+
+def measure(key, args, rank, local_rank, world_size, device, steps, warmup, e2e=True, parity_envs=128, rollout=False,
+            dump_dir=None):
     """One workload on this rank's GPU: W warm-up steps, `steps` timed steps (CUDA events per step, L2 flushed in
     between), the host-buffer (e2e) leg, the oracle replay of a sample of the timed run.  Every rank returns the
-    same reduced numbers; rank 0 also the roofline / parity details."""
+    same reduced numbers; rank 0 also the roofline / parity details, and writes what the last timed step returned
+    to `dump_dir` when one is given."""
     import torch
     import torch.distributed as dist
     from paintrl_b200 import sharding
@@ -341,20 +386,9 @@ def measure(key, args, rank, local_rank, world_size, device, steps, warmup, e2e=
     torch.cuda.synchronize(device)
     create_s = time.perf_counter() - t_create
     if rollout:
-        run_rollout(args, workload, env, cfg, rank, world_size, device, warmup)
+        run_rollout(args, workload, env, cfg, rank, world_size, device, warmup, dump_dir=dump_dir)
         return None
-    gen = torch.Generator(device=device)
-    gen.manual_seed(1234 + rank)
-    e2e_steps = max(10, min(steps, 200)) if e2e else 0
-    total = warmup + max(steps, e2e_steps)
-    if cfg.action_mode == 'discrete':
-        actions = torch.randint(0, cfg.discrete_granularity, (total, n_env), generator=gen, device=device,
-                                dtype=torch.int64)
-    else:
-        actions = torch.rand((total, n_env, cfg.action_dim), generator=gen, device=device, dtype=torch.float64) * 2 - 1
-    gs = torch.Generator(device=device)
-    gs.manual_seed(rank)
-    start = torch.randint(0, env.n_starts, (n_env,), generator=gs, device=device, dtype=torch.int32)
+    actions, start, e2e_steps = seeded_inputs(env, cfg, rank, device, steps, warmup, e2e)
     env.reset(start)
     flush = None if args.no_flush else torch.empty(512 << 20, dtype=torch.uint8, device=device)
     drain = torch.empty(256 << 20, dtype=torch.uint8, device=device) if (flush is not None and args.flush_mode == 'write+read') else None
@@ -406,6 +440,9 @@ def measure(key, args, rank, local_rank, world_size, device, steps, warmup, e2e=
     barrier()
     wall_s = time.perf_counter() - t_wall
     clocks = sampler.stop()
+    if dump_dir and rank == 0:        # before the legs below step the same environments again
+        dump_outputs(dump_dir, {'obs': env.obs, 'reward': env.reward, 'penalty': env.penalty, 'actual': env.actual,
+                                'done': env.done, 'new_texels': env.new_texels, 'next_obs': env.next_obs})
     s1 = env.stats()
     step_ms = np.array([a.elapsed_time(b) for a, b in zip(starts, stops)])
     dev_ms = float(step_ms.sum())
@@ -589,7 +626,12 @@ def main():
     ap.add_argument('--rollout', action='store_true',
                     help='time whole rollout fragments (on-GPU MLP policy + env step, paintrl_b200.rollout) instead of bare steps; '
                          '--steps counts fragments of 100 steps (BASELINE config C5 / paint_ppo.py sample_batch_size)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="after the timed steps, write what the last one returned (rank 0's environments; with --rollout the "
+                         'last fragment) as DIR/<name>.npy, under 64 MB: compares two builds run with the same arguments')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU path; --impl reference has none')
     workload = WORKLOADS[args.workload]
 
     from paintrl_b200 import sharding
@@ -610,7 +652,7 @@ def main():
 
     parity_envs = 0 if args.no_parity else 128
     res = measure(args.workload, args, rank, local_rank, world_size, device, args.steps, warmup, e2e=True,
-                  parity_envs=parity_envs, rollout=args.rollout)
+                  parity_envs=parity_envs, rollout=args.rollout, dump_dir=args.dump_outputs)
     if res is None:
         return
 

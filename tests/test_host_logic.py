@@ -56,6 +56,30 @@ def test_algorithmic_bytes_matches_survey_8d():
     assert bench.algorithmic_bytes(1, 9663, 2, 1, False, 0, 0.0) == 16 + 8 + 40 + 320
 
 
+def test_bench_dump_outputs_writes_a_fixed_sample_within_the_limit(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: every environment while the arrays fit the limit, a seeded sample (the same one in
+    every run) once they do not; flags and float32 tensors in float32, the rest in float64."""
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    arrays = {'obs': torch.arange(600, dtype=torch.float64).reshape(100, 6), 'done': torch.ones(100, dtype=torch.uint8),
+              'new_texels': torch.arange(100, dtype=torch.int32), 'value': torch.zeros(100, dtype=torch.float32)}
+    bench.dump_outputs(str(tmp_path / 'all'), arrays)
+    got = {k: np.load(str(tmp_path / 'all' / (k + '.npy'))) for k in list(arrays) + ['env_ids']}
+    assert np.array_equal(got['env_ids'], np.arange(100)) and np.array_equal(got['obs'], arrays['obs'].numpy())
+    assert got['obs'].dtype == np.float64 and got['new_texels'].dtype == np.float64
+    assert got['done'].dtype == np.float32 and got['value'].dtype == np.float32
+    monkeypatch.setattr(bench, 'DUMP_BYTES', 10 * (8 + 48 + 1 * 4 + 8 + 4))
+    for run in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / run), arrays)
+    ids = np.load(str(tmp_path / 'a' / 'env_ids.npy'))
+    assert len(ids) == 10 and np.all(np.diff(ids) > 0)
+    assert np.array_equal(ids, np.load(str(tmp_path / 'b' / 'env_ids.npy')))
+    assert np.array_equal(np.load(str(tmp_path / 'a' / 'obs.npy')), arrays['obs'].numpy()[ids.astype(np.int64)])
+    total = sum(os.path.getsize(str(tmp_path / 'a' / (k + '.npy'))) - 128 for k in list(arrays) + ['env_ids'])
+    assert total <= bench.DUMP_BYTES
+
+
 def test_shard_range_partitions_every_env_exactly_once():
     from paintrl_b200.sharding import shard_range
     for total in (0, 1, 7, 4096, 65536, 65537):

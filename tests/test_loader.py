@@ -4,8 +4,8 @@
   pack the REFERENCE made of it (oracle/make_golden.py pack100: PaintRL's own `load_part` under shims S1-S5).  The loader
   must reproduce every table bit for bit -- with the C oracle's rasteriser here, with the GPU rasteriser under `-m gpu`.
 * The reference's parts (door_test, square, door_rr, test: committed packs; door_lf, door_lr, door_rf, roof, bonnet,
-  door_rr_big: digests of reference-minted packs, tests/golden/pack_digests.json) are checked wherever the reference's
-  meshes are present (/root/reference: the build container, not the GPU box).
+  door_rr_big: digests of reference-minted packs, tests/golden/pack_digests.json) are checked when PAINTRL_REFERENCE
+  names a checkout of the reference, whose meshes this repository does not carry.
 """
 import json
 import os
@@ -20,9 +20,9 @@ from paintrl_b200.partpack import PART_DICT, PartPack
 HERE = os.path.dirname(os.path.abspath(__file__))
 BULGE_URDF = os.path.join(HERE, 'data', 'urdf', 'painting', 'bulge.urdf')
 BULGE_GOLDEN = os.path.join(HERE, 'golden', 'bulge_128x128.npz')
-REF_PARTS = os.environ.get('PAINTRL_REFERENCE', '/root/reference') + '/PaintRLEnv/urdf/painting'
-needs_reference = pytest.mark.skipif(not os.path.isfile(os.path.join(REF_PARTS, 'door_test.urdf')),
-                                     reason='the reference part meshes are not on this machine')
+REF_PARTS = os.path.join(os.environ.get('PAINTRL_REFERENCE', ''), 'PaintRLEnv', 'urdf', 'painting')
+needs_reference = pytest.mark.skipif(not os.environ.get('PAINTRL_REFERENCE') or not os.path.isfile(os.path.join(REF_PARTS, 'door_test.urdf')),
+                                     reason='PAINTRL_REFERENCE does not name a checkout of the reference with its part meshes')
 
 
 def oracle_rasterizer(*args):

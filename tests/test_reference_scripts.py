@@ -1,4 +1,5 @@
-"""Do the reference's own scripts resolve against this repository?  (CPU; needs the reference checkout.)
+"""Do the reference's own scripts resolve against this repository?  (CPU; needs a checkout of the reference, named by
+PAINTRL_REFERENCE: the scripts are not part of this repository.)
 
 zigzag.py, spiral.py, paint_*.py and param_test_*.py import `PaintRLEnv.robot_gym_env.PaintGymEnv` /
 `PaintRLEnv.param_test_env.ParamTestEnv` and drive them.  The scripts cannot be executed on the GPU box (the reference is
@@ -15,9 +16,10 @@ import textwrap
 
 import pytest
 
-REF = os.environ.get('PAINTRL_REFERENCE', '/root/reference')
+REF = os.environ.get('PAINTRL_REFERENCE', '')
 SCRIPTS = ['zigzag.py', 'spiral.py', 'paint_ppo.py', 'param_test_ppo.py']
-pytestmark = pytest.mark.skipif(not os.path.isfile(os.path.join(REF, 'zigzag.py')), reason='reference checkout not present')
+pytestmark = pytest.mark.skipif(not REF or not os.path.isfile(os.path.join(REF, 'zigzag.py')),
+                                reason='PAINTRL_REFERENCE does not name a checkout of the reference')
 
 
 def _calls_and_attributes(tree):
