@@ -191,6 +191,18 @@ int paintrl_step(PaintrlHandle h, const void *actions_dev, double *obs_dev, doub
                  int32_t *new_texels_dev, double *next_obs_dev,
                  const int32_t *reset_start_idx_dev, void *stream);
 
+/* paintrl_step for the environments env_ids_dev[0..n) (device int32, unique), or, when env_ids_dev is NULL,
+ * for env_lo .. env_lo + n - 1.  Every I/O buffer has n rows, row k = the k-th listed environment.
+ * What the step does to a listed environment is exactly what paintrl_step does to it (record, planes,
+ * counters, the seeded auto-reset stream); the other environments are not touched.  The kernel shape
+ * (one or two launches) follows n.  Ids outside [0, num_envs) are skipped by the device code; unique ids
+ * are the caller's contract.  PAINTRL_E_INVALID for n outside [1, num_envs], a range outside the batch or
+ * env_lo != 0 together with a list. */
+int paintrl_step_subset(PaintrlHandle h, const int32_t *env_ids_dev, int32_t env_lo, int32_t n,
+                        const void *actions_dev, double *obs_dev, double *reward_dev, double *penalty_dev,
+                        double *actual_dev, uint8_t *done_dev, int32_t *new_texels_dev, double *next_obs_dev,
+                        const int32_t *reset_start_idx_dev, void *stream);
+
 /* Same step with HOST buffers: copies the actions host->device, runs the step, copies
  * obs/reward/penalty/actual/done (and next_obs if given) device->host, and returns once they
  * have landed.  This is the call the gym / VectorEnv surface makes. */
@@ -208,6 +220,13 @@ int paintrl_step_host(PaintrlHandle h, const void *actions_host, double *obs_hos
 int paintrl_step_host_submit(PaintrlHandle h, int32_t slot, const void *actions_host, double *obs_host,
                              double *reward_host, double *penalty_host, double *actual_host,
                              uint8_t *done_host, double *next_obs_host, void *stream);
+/* paintrl_step_host_submit for the range env_lo .. env_lo + n - 1: host buffers of n rows; completed by
+ * paintrl_step_host_wait(slot).  Two slots = two groups in flight: a closed-loop host policy computes one group's
+ * next actions while the other group steps.  Results come back in the same obs | reward | penalty | actual |
+ * [next_obs] | done order, sized for n rows. */
+int paintrl_step_host_submit_range(PaintrlHandle h, int32_t slot, int32_t env_lo, int32_t n, const void *actions_host,
+                                   double *obs_host, double *reward_host, double *penalty_host, double *actual_host,
+                                   uint8_t *done_host, double *next_obs_host, void *stream);
 int paintrl_step_host_wait(PaintrlHandle h, int32_t slot);
 
 /* State access (the reference keeps it in Part.texels / Robot._pose,_orn / PaintGymEnv counters,

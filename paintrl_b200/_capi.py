@@ -101,8 +101,10 @@ SIGNATURES = {
     'paintrl_reset': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP]),
     'paintrl_set_pose': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP]),
     'paintrl_step': (ctypes.c_int, [_VP] * 11),
+    'paintrl_step_subset': (ctypes.c_int, [_VP, _VP, _I32, _I32] + [_VP] * 10),
     'paintrl_step_host': (ctypes.c_int, [_VP] * 9),
     'paintrl_step_host_submit': (ctypes.c_int, [_VP, _I32] + [_VP] * 8),
+    'paintrl_step_host_submit_range': (ctypes.c_int, [_VP, _I32, _I32, _I32] + [_VP] * 8),
     'paintrl_step_host_wait': (ctypes.c_int, [_VP, _I32]),
     'paintrl_get_state': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP, _VP]),
     'paintrl_set_state': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP, _VP]),

@@ -19,6 +19,78 @@ def _ptr(t):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+def check_subset(ids_or_range, num_envs):
+    """Validate a subset of a batch of `num_envs` environments once, so that stepping it needs no further check.
+
+    `ids_or_range` is a `range` with step 1 (a contiguous group: returns (None, lo, n)) or a list / array / tensor of
+    environment ids (returns (ids, 0, n), ids an int32 NumPy array, or an int32 tensor on the given CUDA tensor's
+    device).  Ids must be integers, in [0, num_envs) and unique, and the subset must not be empty: the kernels index
+    per-environment state with them, so a duplicate would race and an id out of range would touch no environment.
+    A CUDA tensor is checked with one reduction and one synchronisation."""
+    if isinstance(ids_or_range, range):
+        r = ids_or_range
+        if r.step != 1:
+            raise ValueError('a subset range must have step 1, got %d' % r.step)
+        if len(r) == 0:
+            raise ValueError('the subset range is empty')
+        if r.start < 0 or r.stop > num_envs:
+            raise IndexError('subset range [%d, %d) outside [0, %d)' % (r.start, r.stop, num_envs))
+        return None, r.start, len(r)
+    if isinstance(ids_or_range, torch.Tensor) and ids_or_range.is_cuda:
+        if ids_or_range.dtype.is_floating_point or ids_or_range.dtype.is_complex or ids_or_range.dtype == torch.bool:
+            raise ValueError('env ids must be integers')
+        ids = ids_or_range.reshape(-1)
+        n = int(ids.numel())
+        if n == 0:
+            raise ValueError('the subset is empty')
+        srt = torch.sort(ids.to(torch.int64)).values
+        lo, hi, dup = torch.stack([srt[0], srt[-1], (srt[1:] == srt[:-1]).sum()]).tolist()
+        host = None
+    else:
+        host = np.asarray(ids_or_range.cpu() if isinstance(ids_or_range, torch.Tensor) else ids_or_range).reshape(-1)
+        n = int(host.size)
+        if n == 0:
+            raise ValueError('the subset is empty')
+        if host.dtype.kind not in 'iu':
+            raise ValueError('env ids must be integers')
+        lo, hi = int(host.min()), int(host.max())
+        dup = n - np.unique(host).size
+    if lo < 0 or hi >= num_envs:
+        raise IndexError('env ids out of range [0, %d): min %d, max %d' % (num_envs, lo, hi))
+    if dup:
+        raise ValueError('env ids must be unique')
+    if host is None:
+        return ids_or_range.reshape(-1).to(torch.int32).contiguous(), 0, n
+    return host.astype(np.int32), 0, n
+
+
+class EnvSubset(object):
+    """A fixed subset of one `BatchedPaintEnv`'s environments (`BatchedPaintEnv.subset`): the device id list, or the
+    range lo .. lo + n - 1 (`ids` None), and compact output tensors of n rows of its own, row k = the k-th listed
+    environment, so that two subsets in flight never share buffers.  `env_ids` is the id of every row (int32, on the
+    environment's device)."""
+
+    def __init__(self, owner, ids, lo, n):
+        self.owner = owner
+        self.ids, self.lo, self.n = ids, lo, n
+        dev, f64 = owner.device, torch.float64
+        self.env_ids = ids if ids is not None else torch.arange(lo, lo + n, dtype=torch.int32, device=dev)
+        self.obs = torch.zeros(n, owner.obs_dim, dtype=f64, device=dev)
+        self.next_obs = torch.zeros(n, owner.obs_dim, dtype=f64, device=dev)
+        self.reward = torch.zeros(n, dtype=f64, device=dev)
+        self.penalty = torch.zeros(n, dtype=f64, device=dev)
+        self.actual = torch.zeros(n, dtype=f64, device=dev)
+        self.done = torch.zeros(n, dtype=torch.uint8, device=dev)
+        self.new_texels = torch.zeros(n, dtype=torch.int32, device=dev)
+
+    @property
+    def is_range(self):
+        return self.ids is None
+
+    def __len__(self):
+        return self.n
+
+
 class BatchedPaintEnv(object):
     """`num_envs` PaintGymEnv instances sharing one part and one configuration.
 
@@ -90,34 +162,13 @@ class BatchedPaintEnv(object):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
 
     def _ids(self, env_ids):
-        """Device list of environment indices for the by-index entry points, validated on the host: in range and
-        unique (the kernels index states / planes with them; a duplicate would race, an out-of-range id corrupt
-        another environment -- the device code also ignores ids out of range).  Host-side lists cost nothing to
-        check; a CUDA tensor is checked with one small reduction."""
+        """Device list of environment indices for the by-index entry points, validated on the host by
+        `check_subset`: in range and unique (the kernels index states / planes with them; a duplicate would race,
+        an out-of-range id corrupt another environment -- the device code also ignores ids out of range)."""
         if env_ids is None:
             return None, self.num_envs
-        if isinstance(env_ids, torch.Tensor) and env_ids.is_cuda:
-            ids = env_ids.to(device=self.device, dtype=torch.int32).reshape(-1).contiguous()
-            n = int(ids.numel())
-            if n == 0:
-                raise ValueError('env_ids is empty')
-            lo, hi = int(ids.min()), int(ids.max())
-            unique = n == 1 or int(torch.unique(ids).numel()) == n
-        else:
-            host = np.asarray(env_ids.cpu() if isinstance(env_ids, torch.Tensor) else env_ids).reshape(-1)
-            n = int(host.size)
-            if n == 0:
-                raise ValueError('env_ids is empty')
-            if host.dtype.kind not in 'iu':
-                raise ValueError('env_ids must be integers')
-            lo, hi = int(host.min()), int(host.max())
-            unique = n == 1 or np.unique(host).size == n
-            ids = torch.as_tensor(host.astype(np.int32), device=self.device).contiguous()
-        if lo < 0 or hi >= self.num_envs:
-            raise IndexError('env_ids out of range [0, %d): min %d, max %d' % (self.num_envs, lo, hi))
-        if not unique:
-            raise ValueError('env_ids must be unique')
-        return ids, n
+        ids, _, n = check_subset(list(env_ids) if isinstance(env_ids, range) else env_ids, self.num_envs)
+        return torch.as_tensor(ids, device=self.device).to(torch.int32).contiguous(), n
 
     # ------------------------------------------------------------------ reference call mirror
     def reset(self, start_index=None, env_ids=None):
@@ -147,36 +198,68 @@ class BatchedPaintEnv(object):
                                                self._stream()))
         return out
 
-    def step(self, actions, reset_start_index=None):
+    def subset(self, ids_or_range):
+        """An `EnvSubset` of this batch to pass as `subset=` to `step`, `step_into` and (ranges only)
+        `step_host_submit`: a `range` with step 1, or a list / array / tensor of unique environment ids.  Validated
+        here, once (see `check_subset`); stepping a fixed subset needs no host synchronisation, so it can be captured
+        in a CUDA graph."""
+        ids, lo, n = check_subset(ids_or_range, self.num_envs)
+        if ids is not None:
+            ids = torch.as_tensor(ids, device=self.device).to(torch.int32).contiguous()
+        return EnvSubset(self, ids, lo, n)
+
+    def _rows(self, subset):
+        if subset is None:
+            return self.num_envs
+        if not isinstance(subset, EnvSubset) or subset.owner is not self:
+            raise ValueError('subset must be an EnvSubset made by this environment\'s subset()')
+        return subset.n
+
+    def _step_call(self, subset, actions, obs, reward, penalty, actual, done, new_texels, next_obs, rs):
+        nxt = _ptr(next_obs) if self.cfg.auto_reset else None
+        if subset is None:
+            rc = self._lib.paintrl_step(self._h, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(penalty), _ptr(actual),
+                                        _ptr(done), _ptr(new_texels), nxt, _ptr(rs), self._stream())
+        else:
+            rc = self._lib.paintrl_step_subset(self._h, _ptr(subset.ids), subset.lo, subset.n, _ptr(actions), _ptr(obs),
+                                               _ptr(reward), _ptr(penalty), _ptr(actual), _ptr(done), _ptr(new_texels),
+                                               nxt, _ptr(rs), self._stream())
+        _capi.check(rc)
+
+    def step(self, actions, reset_start_index=None, subset=None):
         """PaintGymEnv.step for all environments (robot_gym_env.py:349-368), device tensors in and
         out, asynchronous on the current stream.  Returns (obs, actual_reward, done, info) where
-        info = {'reward', 'penalty'} like robot_gym_env.py:368 plus 'next_obs' / 'new_texels'."""
+        info = {'reward', 'penalty'} like robot_gym_env.py:368 plus 'next_obs' / 'new_texels'.
+        With `subset` (an `EnvSubset`) only its n environments step: actions, reset_start_index and every output
+        have n rows, row k = the k-th environment of the subset (info['env_ids'])."""
+        B = self._rows(subset)
         if self.cfg.action_mode == 'discrete':
             a = torch.as_tensor(actions, device=self.device).to(torch.int64).contiguous()
-            if a.numel() != self.num_envs:
-                raise ValueError('expected %d discrete actions' % self.num_envs)
+            if a.numel() != B:
+                raise ValueError('expected %d discrete actions' % B)
         else:
             a = torch.as_tensor(actions, device=self.device).to(torch.float64).contiguous()
-            if a.numel() != self.num_envs * self.action_dim:
-                raise ValueError('expected actions of shape [%d, %d]' % (self.num_envs, self.action_dim))
+            if a.numel() != B * self.action_dim:
+                raise ValueError('expected actions of shape [%d, %d]' % (B, self.action_dim))
         rs = None
         if reset_start_index is not None:
             rs = torch.as_tensor(reset_start_index, dtype=torch.int32, device=self.device).contiguous()
-            if rs.numel() != self.num_envs:
-                raise ValueError('reset_start_index must have one entry per environment (%d), got %d' % (self.num_envs, rs.numel()))
-        _capi.check(self._lib.paintrl_step(
-            self._h, _ptr(a), _ptr(self.obs), _ptr(self.reward), _ptr(self.penalty), _ptr(self.actual),
-            _ptr(self.done), _ptr(self.new_texels), _ptr(self.next_obs) if self.cfg.auto_reset else None,
-            _ptr(rs), self._stream()))
-        info = {'reward': self.reward, 'penalty': self.penalty, 'new_texels': self.new_texels,
-                'next_obs': self.next_obs if self.cfg.auto_reset else self.obs}
-        return self.obs, self.actual, self.done, info
+            if rs.numel() != B:
+                raise ValueError('reset_start_index must have one entry per environment (%d), got %d' % (B, rs.numel()))
+        o = self if subset is None else subset
+        self._step_call(subset, a, o.obs, o.reward, o.penalty, o.actual, o.done, o.new_texels, o.next_obs, rs)
+        info = {'reward': o.reward, 'penalty': o.penalty, 'new_texels': o.new_texels,
+                'next_obs': o.next_obs if self.cfg.auto_reset else o.obs}
+        if subset is not None:
+            info['env_ids'] = subset.env_ids
+        return o.obs, o.actual, o.done, info
 
-    def step_into(self, actions, obs, reward, penalty, actual, done, next_obs=None, new_texels=None):
+    def step_into(self, actions, obs, reward, penalty, actual, done, next_obs=None, new_texels=None, subset=None):
         """`step` writing straight into caller tensors (e.g. row t of a rollout fragment): contiguous
         CUDA tensors of this environment's device, float64 [B, obs_dim] / [B], uint8 [B], int32 [B];
-        `actions` int64 [B] or float64 [B, action_dim].  Nothing is returned and nothing is copied."""
-        B = self.num_envs
+        `actions` int64 [B] or float64 [B, action_dim].  Nothing is returned and nothing is copied.
+        With `subset`, B is the subset's size and row k belongs to its k-th environment."""
+        B = self._rows(subset)
         want = (torch.int64, B) if self.cfg.action_mode == 'discrete' else (torch.float64, B * self.action_dim)
         for t, (dt, n) in ((actions, want), (obs, (torch.float64, B * self.obs_dim)), (reward, (torch.float64, B)),
                            (penalty, (torch.float64, B)), (actual, (torch.float64, B)), (done, (torch.uint8, B)),
@@ -185,9 +268,7 @@ class BatchedPaintEnv(object):
                 continue
             if t.dtype != dt or t.numel() != n or not t.is_contiguous() or t.device != self.device:
                 raise ValueError('step_into: expected a contiguous %s tensor of %d elements on %s' % (dt, n, self.device))
-        _capi.check(self._lib.paintrl_step(
-            self._h, _ptr(actions), _ptr(obs), _ptr(reward), _ptr(penalty), _ptr(actual), _ptr(done), _ptr(new_texels),
-            _ptr(next_obs) if self.cfg.auto_reset else None, None, self._stream()))
+        self._step_call(subset, actions, obs, reward, penalty, actual, done, new_texels, next_obs, None)
         if next_obs is not None and not self.cfg.auto_reset:
             next_obs.copy_(obs)
 
@@ -215,18 +296,26 @@ class BatchedPaintEnv(object):
             _capi.check(rc)
         return out
 
-    def step_host_submit(self, actions, out, slot=0):
+    def step_host_submit(self, actions, out, slot=0, subset=None):
         """First half of `step_host` (paintrl_step_host_submit): queue the copy-in of `actions`, the step and the
         copy-out into `out` (from `host_buffers`) on staging slot 0 or 1 and return at once.  `actions` must stay
         untouched (and should be pinned) until `step_host_wait(slot)`.  Submitting step t + 1 on the other slot
-        before waiting for step t overlaps its copy-in and kernels with step t's copy-out and the host's wake-up."""
+        before waiting for step t overlaps its copy-in and kernels with step t's copy-out and the host's wake-up.
+        With `subset` (a range `EnvSubset`, paintrl_step_host_submit_range) only that group steps; `actions` and
+        `out` (`host_buffers(n=subset.n)`) have its n rows.  Two groups on the two slots let a closed-loop policy
+        compute one group's actions while the other steps."""
+        B = self._rows(subset)
+        if subset is not None and not subset.is_range:
+            raise ValueError('step_host_submit takes range subsets only (BatchedPaintEnv.subset(range(lo, hi)))')
         discrete = self.cfg.action_mode == 'discrete'
         want = np.int64 if discrete else np.float64
         a = actions
         if not (isinstance(a, np.ndarray) and a.dtype == want and a.flags.c_contiguous):
             a = np.ascontiguousarray(actions, dtype=want)
-        if a.size != (self.num_envs if discrete else self.num_envs * self.action_dim):
-            raise ValueError('expected %d actions' % self.num_envs)
+        if a.size != (B if discrete else B * self.action_dim):
+            raise ValueError('expected %d actions' % B)
+        if subset is not None and out['obs'].shape[0] != B:
+            raise ValueError('host buffers of %d rows for a step of %d environments' % (out['obs'].shape[0], B))
         ptrs = out.get('_ptrs')
         if ptrs is None:
             nxt = out.get('next_obs')
@@ -234,8 +323,13 @@ class BatchedPaintEnv(object):
                 nxt.ctypes.data if nxt is not None else None,)
         self._inflight = getattr(self, '_inflight', {})
         self._inflight[slot] = (a, out)          # keep the buffers alive until the wait
-        rc = self._lib.paintrl_step_host_submit(self._h, int(slot), a.ctypes.data, ptrs[0], ptrs[1], ptrs[2], ptrs[3], ptrs[4],
-                                                ptrs[5], torch.cuda.current_stream(self.device).cuda_stream)
+        stream = torch.cuda.current_stream(self.device).cuda_stream
+        if subset is None:
+            rc = self._lib.paintrl_step_host_submit(self._h, int(slot), a.ctypes.data, ptrs[0], ptrs[1], ptrs[2], ptrs[3],
+                                                    ptrs[4], ptrs[5], stream)
+        else:
+            rc = self._lib.paintrl_step_host_submit_range(self._h, int(slot), subset.lo, subset.n, a.ctypes.data, ptrs[0],
+                                                          ptrs[1], ptrs[2], ptrs[3], ptrs[4], ptrs[5], stream)
         if rc != 0:
             _capi.check(rc)
 
@@ -246,11 +340,12 @@ class BatchedPaintEnv(object):
             _capi.check(rc)
         return self._inflight.pop(slot)[1]
 
-    def host_buffers(self, pinned=True, next_obs=True):
+    def host_buffers(self, pinned=True, next_obs=True, n=None):
         """Host result buffers for `step_host`: views into ONE (pinned) allocation laid out
         obs | reward | penalty | actual | [next_obs] | done, the order `paintrl_step_host` stages its
-        results in, so that they come back with a single device->host copy."""
-        B, od = self.num_envs, self.obs_dim
+        results in, so that they come back with a single device->host copy.  `n`: rows (a group of
+        `step_host_submit(subset=...)`); default the whole batch."""
+        B, od = (self.num_envs if n is None else int(n)), self.obs_dim
         n_f64 = B * (od * (2 if next_obs else 1) + 3)
         raw = torch.zeros(n_f64 * 8 + B, dtype=torch.uint8, pin_memory=pinned)
         f64 = raw[:n_f64 * 8].view(torch.float64).numpy()

@@ -113,6 +113,7 @@ struct PaintrlEngine {
     // measured slower at C2 (the move phase loses L1 and issue slots to the co-resident paint warps).
     int carveout_percent = -1;
     bool carveout_set = false;       // the step kernels' shared-memory carveout has been requested on this device
+    bool carveout_set_subset = false;   // the same for their subset instantiations
     // staging for the host-buffer entry points
     void *stage_actions = nullptr;
     // paintrl_step_host: one contiguous block, laid out per call as obs | reward | penalty | actual | [next_obs] | done,
@@ -817,6 +818,228 @@ int launch_check(PaintrlEngine *e, const char *what) {
     return PAINTRL_OK;
 }
 
+// The I/O buffers of paintrl_step / paintrl_step_subset, checked and packed for the kernels.
+int step_io(PaintrlHandle h, const void *actions_dev, double *obs_dev, double *reward_dev, double *penalty_dev, double *actual_dev,
+            uint8_t *done_dev, int32_t *new_texels_dev, double *next_obs_dev, const int32_t *reset_start_idx_dev, StepIO *io) {
+    if (!actions_dev || !obs_dev || !reward_dev || !penalty_dev || !actual_dev || !done_dev)
+        return fail(PAINTRL_E_INVALID, "null I/O buffer");
+    {   // the kernels store 8-byte (4-byte for new_texels / start indices) elements: refuse misaligned buffers
+        const uintptr_t a8 = (uintptr_t)actions_dev | (uintptr_t)obs_dev | (uintptr_t)reward_dev | (uintptr_t)penalty_dev |
+                             (uintptr_t)actual_dev | (uintptr_t)next_obs_dev;
+        const uintptr_t a4 = (uintptr_t)new_texels_dev | (uintptr_t)reset_start_idx_dev;
+        if ((a8 & 7u) || (a4 & 3u)) return fail(PAINTRL_E_INVALID, "misaligned I/O buffer (float64 / int64 buffers need 8-byte alignment)");
+    }
+    io->actions = actions_dev; io->obs = obs_dev; io->reward = reward_dev; io->penalty = penalty_dev;
+    io->actual = actual_dev; io->done = done_dev; io->new_texels = new_texels_dev;
+    io->next_obs = h->cfg.auto_reset ? next_obs_dev : nullptr;
+    io->reset_start_idx = reset_start_idx_dev;
+    return PAINTRL_OK;
+}
+
+// The environments of a subset step: the list env_ids (env_lo must be 0) or the range env_lo .. env_lo + n - 1.
+int check_subset(PaintrlHandle h, const int32_t *env_ids, int32_t env_lo, int32_t n) {
+    if (n < 1 || n > h->num_envs) return fail(PAINTRL_E_INVALID, "bad env count: n must be in [1, num_envs]");
+    if (env_ids) {
+        if (env_lo != 0) return fail(PAINTRL_E_INVALID, "env_lo must be 0 when an env_ids list is given");
+        if ((uintptr_t)env_ids & 3u) return fail(PAINTRL_E_INVALID, "misaligned env_ids (int32 needs 4-byte alignment)");
+    } else if (env_lo < 0 || (int64_t)env_lo + n > h->num_envs) {
+        return fail(PAINTRL_E_INVALID, "env range [env_lo, env_lo + n) outside the batch");
+    }
+    return PAINTRL_OK;
+}
+
+// One step of the environments `sel` selects (SUBSET) or of the whole batch (!SUBSET, sel = {nullptr, 0, num_envs}),
+// I/O row k = the k-th selected environment.  The kernel shape follows the number of environments stepped.
+template <bool SUBSET>
+int launch_step(PaintrlHandle h, const EnvSel &sel, const StepIO &io, void *stream) {
+    const int n = sel.n;
+    const void *actions_dev = io.actions;
+    // the carveout is an attribute of each kernel: the whole-batch and the subset instantiations each ask once
+    bool &carveout_done = SUBSET ? h->carveout_set_subset : h->carveout_set;
+    CUDA_TRY(cudaSetDevice(h->device));
+    if (h->paint_normal) {
+        // Robot.PAINT_METHOD == 'normal': the generic move kernel (it also hands over the shots' poses), then the beam-fan
+        // paint kernel, one warp per environment
+        cudaStream_t ns = as_stream(stream);
+        const int threads = 128;
+        move_kernel<32, 4, false, SUBSET><<<(n * 32 + threads - 1) / threads, threads, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);
+        int rc = launch_check(h, "move_kernel");
+        if (rc != PAINTRL_OK) return rc;
+        if (h->color == 0) paint_normal_kernel<0, SUBSET><<<n, 32, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, io, (const ColdArgs *)h->cold_args, sel);
+        else paint_normal_kernel<1, SUBSET><<<n, 32, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, io, (const ColdArgs *)h->cold_args, sel);
+        cudaError_t nerr = cudaGetLastError();
+        if (nerr != cudaSuccess) {
+            cudaMemsetAsync(h->ready, 0, sizeof(unsigned) * (size_t)h->num_envs, ns);
+            return fail(PAINTRL_E_CUDA, std::string("paint_normal_kernel: ") + cudaGetErrorString(nerr));
+        }
+        h->launches++;
+        return PAINTRL_OK;
+    }
+    const bool use_fused = h->fused >= 0 ? h->fused == 1 : n < kFusedBelowEnvs;
+    if (use_fused) {
+        // one launch, one warp per environment for the whole step (paintrl_kernels.cuh step_fused_kernel)
+        const bool staged_f = h->pk.n_words_pad <= kStageWords && !h->force_unstaged;
+        const bool ax12f = h->pk.axis0 == 1 && h->pk.axis1 == 2, disc = h->cfg.action_mode == 0;
+        const EnvArrays fea = env_arrays(h);
+        const ColdArgs *cold = (const ColdArgs *)h->cold_args;
+        cudaStream_t fs = as_stream(stream);
+#define PAINTRL_FUSED_K(C, ST, AX, DI) step_fused_kernel<C, ST, AX, DI, SUBSET><<<(n + PAINTRL_FUSED_WPB - 1) / PAINTRL_FUSED_WPB, 32 * PAINTRL_FUSED_WPB, 0, fs>>>(h->pk, h->cfg, fea, h->num_envs, io, cold, sel)
+#define PAINTRL_FUSED_AD(C, ST)                                                        \
+    do {                                                                               \
+        if (ax12f && disc) PAINTRL_FUSED_K(C, ST, true, true);                         \
+        else if (ax12f) PAINTRL_FUSED_K(C, ST, true, false);                           \
+        else if (disc) PAINTRL_FUSED_K(C, ST, false, true);                            \
+        else PAINTRL_FUSED_K(C, ST, false, false);                                     \
+    } while (0)
+        if (h->color == 0) { if (staged_f) PAINTRL_FUSED_AD(0, true); else PAINTRL_FUSED_AD(0, false); }
+        else { if (staged_f) PAINTRL_FUSED_AD(1, true); else PAINTRL_FUSED_AD(1, false); }
+#undef PAINTRL_FUSED_AD
+#undef PAINTRL_FUSED_K
+        return launch_check(h, "step_fused_kernel");
+    }
+    {   // lanes per environment in the move phase: fewer when there are enough environments to fill the GPU
+        const int threads = h->move_warps * 32;
+        cudaStream_t ms = as_stream(stream);
+        const int L = h->move_lanes;
+        const int mblocks = (int)(((long long)n * L + threads - 1) / threads);
+        const bool ax12m = h->pk.axis0 == 1 && h->pk.axis1 == 2;
+#define PAINTRL_MOVE(G, MINB)                                                                                              \
+    do {                                                                                                                   \
+        if (!carveout_done && h->carveout_percent >= 0) {                                                                \
+            cudaFuncSetAttribute(move_kernel<G, MINB, true, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent);  \
+            cudaFuncSetAttribute(move_kernel<G, MINB, false, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent); \
+        }                                                                                                                  \
+        if (ax12m) move_kernel<G, MINB, true, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);  \
+        else move_kernel<G, MINB, false, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);       \
+    } while (0)
+#define PAINTRL_MOVE_FAST(G)                                                                                               \
+    do {                                                                                                                   \
+        if (ax12m && discrete) move_fast_kernel<G, true, true, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);   \
+        else if (ax12m) move_fast_kernel<G, true, false, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);         \
+        else if (discrete) move_fast_kernel<G, false, true, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);      \
+        else move_fast_kernel<G, false, false, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);                   \
+    } while (0)
+        const bool discrete = h->cfg.action_mode == 0;
+        if (h->move_fast) {
+            // the lean kernel: rays decided by their move cell alone; the rest is handed to the paint warps (kReadyBailed)
+            if (L == 8) PAINTRL_MOVE_FAST(8); else if (L == 16) PAINTRL_MOVE_FAST(16); else PAINTRL_MOVE_FAST(32);
+        } else if (h->move_minb == 7) {
+            if (L == 8) PAINTRL_MOVE(8, 7); else if (L == 16) PAINTRL_MOVE(16, 7); else PAINTRL_MOVE(32, 7);
+        } else {
+            if (L == 8) PAINTRL_MOVE(8, 4); else if (L == 16) PAINTRL_MOVE(16, 4); else PAINTRL_MOVE(32, 4);
+        }
+#undef PAINTRL_MOVE_FAST
+#undef PAINTRL_MOVE
+    }
+    int rc = launch_check(h, "move_kernel");
+    if (rc != PAINTRL_OK) return rc;
+    const bool staged = h->pk.n_words_pad <= kStageWords && !h->force_unstaged;
+    const int pw = h->paint_warps;
+    const dim3 grid((n + pw - 1) / pw), block(pw * 32);
+    cudaStream_t s = as_stream(stream);
+    const bool ax12 = h->pk.axis0 == 1 && h->pk.axis1 == 2;
+    // programmatic dependent launch after move_kernel (see griddepcontrol.* in the kernels)
+    cudaLaunchConfig_t lc{};
+    lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = 0; lc.stream = s;
+    cudaLaunchAttribute lattr[1];
+    lattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    lattr[0].val.programmaticStreamSerializationAllowed = 1;
+    lc.attrs = lattr; lc.numAttrs = 1;
+    const EnvArrays pea = env_arrays(h);
+    cudaError_t perr = cudaSuccess;
+#define PAINTRL_PAINT_W(C, ST, W)                                                                           \
+    do {                                                                                                    \
+        if (!carveout_done && h->carveout_percent >= 0) {                                                 \
+            cudaFuncSetAttribute(paint_kernel<C, ST, true, W, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent);  \
+            cudaFuncSetAttribute(paint_kernel<C, ST, false, W, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent); \
+        }                                                                                                   \
+        if (ax12) perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, true, W, SUBSET>, h->pk, h->cfg, pea, h->num_envs, io, (const ColdArgs *)h->cold_args, sel);  \
+        else perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, false, W, SUBSET>, h->pk, h->cfg, pea, h->num_envs, io, (const ColdArgs *)h->cold_args, sel);      \
+    } while (0)
+#define PAINTRL_PAINT(C, ST)                                                                 \
+    do {                                                                                     \
+        if (pw == 1) PAINTRL_PAINT_W(C, ST, 1); else if (pw == 2) PAINTRL_PAINT_W(C, ST, 2); \
+        else PAINTRL_PAINT_W(C, ST, 4);                                                      \
+    } while (0)
+    if (h->color == 0) {
+        if (staged) PAINTRL_PAINT(0, true); else PAINTRL_PAINT(0, false);
+    } else {
+        if (staged) PAINTRL_PAINT(1, true); else PAINTRL_PAINT(1, false);
+    }
+#undef PAINTRL_PAINT
+#undef PAINTRL_PAINT_W
+    carveout_done = true;
+    if (perr == cudaSuccess) perr = cudaGetLastError();
+    if (perr != cudaSuccess) {
+        // the move grid is already in flight and will raise the hand-off flags nobody consumes: clear them behind it,
+        // or the next step's paint warps would pass their acquire on stale move outputs
+        cudaGetLastError();
+        cudaMemsetAsync(h->ready, 0, sizeof(unsigned) * (size_t)h->num_envs, s);
+        return fail(PAINTRL_E_CUDA, std::string("paint_kernel: ") + cudaGetErrorString(perr));
+    }
+    h->launches++;
+    return PAINTRL_OK;
+}
+
+// paintrl_step_host_submit (subset == false, the whole batch) and paintrl_step_host_submit_range (the environments
+// env_lo .. env_lo + n - 1): host buffers of n rows, staged in the slot's device buffers in the same order.
+int host_submit(PaintrlHandle h, int32_t slot, bool subset, int32_t env_lo, int32_t n, const void *actions_host, double *obs_host,
+                double *reward_host, double *penalty_host, double *actual_host, uint8_t *done_host, double *next_obs_host,
+                void *stream) {
+    if (slot < 0 || slot > 1) return fail(PAINTRL_E_INVALID, "slot must be 0 or 1");
+    if (!actions_host || !obs_host || !reward_host || !penalty_host || !actual_host || !done_host)
+        return fail(PAINTRL_E_INVALID, "null I/O buffer");
+    CUDA_TRY(cudaSetDevice(h->device));
+    cudaStream_t s = as_stream(stream);
+    const size_t nenv = (size_t)n;
+    const size_t abytes = (h->cfg.action_mode == 0 ? sizeof(long long) : sizeof(double) * h->cfg.action_shape) * nenv;
+    const size_t obytes = sizeof(double) * h->cfg.obs_dim * nenv;
+    const bool want_next = next_obs_host != nullptr, dev_next = want_next && h->cfg.auto_reset;
+    // a slot that is submitted again before it was waited for: its previous copy-out must have drained first
+    if (h->slot_pending[slot]) {
+        CUDA_TRY(cudaStreamWaitEvent(h->copy_in, h->ev_done[slot], 0));
+        CUDA_TRY(cudaStreamWaitEvent(s, h->ev_done[slot], 0));
+    }
+    // copy-in stream: the actions, then the step on the caller's stream behind it
+    CUDA_TRY(cudaMemcpyAsync(h->slot_actions[slot], actions_host, abytes, cudaMemcpyHostToDevice, h->copy_in));
+    CUDA_TRY(cudaEventRecord(h->ev_in[slot], h->copy_in));
+    CUDA_TRY(cudaStreamWaitEvent(s, h->ev_in[slot], 0));
+    unsigned char *d = h->slot_out[slot];
+    double *d_obs = reinterpret_cast<double *>(d);
+    double *d_sc = reinterpret_cast<double *>(d + obytes);
+    double *d_next = dev_next ? reinterpret_cast<double *>(d + obytes + 3 * sizeof(double) * nenv) : nullptr;
+    uint8_t *d_done = d + obytes + 3 * sizeof(double) * nenv + (dev_next ? obytes : 0);
+    int rc = subset ? paintrl_step_subset(h, nullptr, env_lo, n, h->slot_actions[slot], d_obs, d_sc, d_sc + nenv, d_sc + 2 * nenv,
+                                          d_done, nullptr, d_next, nullptr, stream)
+                    : paintrl_step(h, h->slot_actions[slot], d_obs, d_sc, d_sc + nenv, d_sc + 2 * nenv, d_done, nullptr, d_next, nullptr, stream);
+    if (rc != PAINTRL_OK) return rc;
+    CUDA_TRY(cudaEventRecord(h->ev_step[slot], s));
+    // copy-out stream: the results, as one copy when the host buffers are carved from one allocation in staging order
+    CUDA_TRY(cudaStreamWaitEvent(h->copy_out, h->ev_step[slot], 0));
+    struct Seg { void *dst; const void *src; size_t n; };
+    Seg segs[7] = {};
+    int ns = 0;
+    auto push = [&](void *dst, const void *src, size_t n) {
+        if (ns > 0 && (const char *)segs[ns - 1].src + segs[ns - 1].n == (const char *)src &&
+            (char *)segs[ns - 1].dst + segs[ns - 1].n == (char *)dst) {
+            segs[ns - 1].n += n;
+        } else {
+            segs[ns].dst = dst; segs[ns].src = src; segs[ns].n = n; ++ns;
+        }
+    };
+    push(obs_host, d_obs, obytes);
+    push(reward_host, d_sc, sizeof(double) * nenv);
+    push(penalty_host, d_sc + nenv, sizeof(double) * nenv);
+    push(actual_host, d_sc + 2 * nenv, sizeof(double) * nenv);
+    if (dev_next) push(next_obs_host, d_next, obytes);
+    push(done_host, d_done, nenv);
+    if (want_next && !dev_next) push(next_obs_host, d_obs, obytes);
+    for (int i = 0; i < ns; ++i) CUDA_TRY(cudaMemcpyAsync(segs[i].dst, segs[i].src, segs[i].n, cudaMemcpyDeviceToHost, h->copy_out));
+    CUDA_TRY(cudaEventRecord(h->ev_done[slot], h->copy_out));
+    h->slot_pending[slot] = true;
+    return PAINTRL_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -1391,142 +1614,24 @@ int paintrl_step(PaintrlHandle h, const void *actions_dev, double *obs_dev, doub
                  double *actual_dev, uint8_t *done_dev, int32_t *new_texels_dev, double *next_obs_dev,
                  const int32_t *reset_start_idx_dev, void *stream) {
     if (!h) return fail(PAINTRL_E_INVALID, "null handle");
-    if (!actions_dev || !obs_dev || !reward_dev || !penalty_dev || !actual_dev || !done_dev)
-        return fail(PAINTRL_E_INVALID, "null I/O buffer");
-    {   // the kernels store 8-byte (4-byte for new_texels / start indices) elements: refuse misaligned buffers
-        const uintptr_t a8 = (uintptr_t)actions_dev | (uintptr_t)obs_dev | (uintptr_t)reward_dev | (uintptr_t)penalty_dev |
-                             (uintptr_t)actual_dev | (uintptr_t)next_obs_dev;
-        const uintptr_t a4 = (uintptr_t)new_texels_dev | (uintptr_t)reset_start_idx_dev;
-        if ((a8 & 7u) || (a4 & 3u)) return fail(PAINTRL_E_INVALID, "misaligned I/O buffer (float64 / int64 buffers need 8-byte alignment)");
-    }
-    CUDA_TRY(cudaSetDevice(h->device));
     StepIO io;
-    io.actions = actions_dev; io.obs = obs_dev; io.reward = reward_dev; io.penalty = penalty_dev;
-    io.actual = actual_dev; io.done = done_dev; io.new_texels = new_texels_dev;
-    io.next_obs = h->cfg.auto_reset ? next_obs_dev : nullptr;
-    io.reset_start_idx = reset_start_idx_dev;
-    if (h->paint_normal) {
-        // Robot.PAINT_METHOD == 'normal': the generic move kernel (it also hands over the shots' poses), then the beam-fan
-        // paint kernel, one warp per environment
-        cudaStream_t ns = as_stream(stream);
-        const int threads = 128;
-        move_kernel<32, 4, false><<<(h->num_envs * 32 + threads - 1) / threads, threads, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev);
-        int rc = launch_check(h, "move_kernel");
-        if (rc != PAINTRL_OK) return rc;
-        if (h->color == 0) paint_normal_kernel<0><<<h->num_envs, 32, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, io, (const ColdArgs *)h->cold_args);
-        else paint_normal_kernel<1><<<h->num_envs, 32, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, io, (const ColdArgs *)h->cold_args);
-        cudaError_t nerr = cudaGetLastError();
-        if (nerr != cudaSuccess) {
-            cudaMemsetAsync(h->ready, 0, sizeof(unsigned) * (size_t)h->num_envs, ns);
-            return fail(PAINTRL_E_CUDA, std::string("paint_normal_kernel: ") + cudaGetErrorString(nerr));
-        }
-        h->launches++;
-        return PAINTRL_OK;
-    }
-    const bool use_fused = h->fused >= 0 ? h->fused == 1 : h->num_envs < kFusedBelowEnvs;
-    if (use_fused) {
-        // one launch, one warp per environment for the whole step (paintrl_kernels.cuh step_fused_kernel)
-        const bool staged_f = h->pk.n_words_pad <= kStageWords && !h->force_unstaged;
-        const bool ax12f = h->pk.axis0 == 1 && h->pk.axis1 == 2, disc = h->cfg.action_mode == 0;
-        const EnvArrays fea = env_arrays(h);
-        const ColdArgs *cold = (const ColdArgs *)h->cold_args;
-        cudaStream_t fs = as_stream(stream);
-#define PAINTRL_FUSED_K(C, ST, AX, DI) step_fused_kernel<C, ST, AX, DI><<<(h->num_envs + PAINTRL_FUSED_WPB - 1) / PAINTRL_FUSED_WPB, 32 * PAINTRL_FUSED_WPB, 0, fs>>>(h->pk, h->cfg, fea, h->num_envs, io, cold)
-#define PAINTRL_FUSED_AD(C, ST)                                                        \
-    do {                                                                               \
-        if (ax12f && disc) PAINTRL_FUSED_K(C, ST, true, true);                         \
-        else if (ax12f) PAINTRL_FUSED_K(C, ST, true, false);                           \
-        else if (disc) PAINTRL_FUSED_K(C, ST, false, true);                            \
-        else PAINTRL_FUSED_K(C, ST, false, false);                                     \
-    } while (0)
-        if (h->color == 0) { if (staged_f) PAINTRL_FUSED_AD(0, true); else PAINTRL_FUSED_AD(0, false); }
-        else { if (staged_f) PAINTRL_FUSED_AD(1, true); else PAINTRL_FUSED_AD(1, false); }
-#undef PAINTRL_FUSED_AD
-#undef PAINTRL_FUSED_K
-        return launch_check(h, "step_fused_kernel");
-    }
-    {   // lanes per environment in the move phase: fewer when there are enough environments to fill the GPU
-        const int threads = h->move_warps * 32;
-        cudaStream_t ms = as_stream(stream);
-        const int L = h->move_lanes;
-        const int mblocks = (int)(((long long)h->num_envs * L + threads - 1) / threads);
-        const bool ax12m = h->pk.axis0 == 1 && h->pk.axis1 == 2;
-#define PAINTRL_MOVE(G, MINB)                                                                                              \
-    do {                                                                                                                   \
-        if (!h->carveout_set && h->carveout_percent >= 0) {                                                                \
-            cudaFuncSetAttribute(move_kernel<G, MINB, true>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent);  \
-            cudaFuncSetAttribute(move_kernel<G, MINB, false>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent); \
-        }                                                                                                                  \
-        if (ax12m) move_kernel<G, MINB, true><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev);  \
-        else move_kernel<G, MINB, false><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev);       \
-    } while (0)
-#define PAINTRL_MOVE_FAST(G)                                                                                               \
-    do {                                                                                                                   \
-        if (ax12m && discrete) move_fast_kernel<G, true, true><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev);   \
-        else if (ax12m) move_fast_kernel<G, true, false><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev);         \
-        else if (discrete) move_fast_kernel<G, false, true><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev);      \
-        else move_fast_kernel<G, false, false><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev);                   \
-    } while (0)
-        const bool discrete = h->cfg.action_mode == 0;
-        if (h->move_fast) {
-            // the lean kernel: rays decided by their move cell alone; the rest is handed to the paint warps (kReadyBailed)
-            if (L == 8) PAINTRL_MOVE_FAST(8); else if (L == 16) PAINTRL_MOVE_FAST(16); else PAINTRL_MOVE_FAST(32);
-        } else if (h->move_minb == 7) {
-            if (L == 8) PAINTRL_MOVE(8, 7); else if (L == 16) PAINTRL_MOVE(16, 7); else PAINTRL_MOVE(32, 7);
-        } else {
-            if (L == 8) PAINTRL_MOVE(8, 4); else if (L == 16) PAINTRL_MOVE(16, 4); else PAINTRL_MOVE(32, 4);
-        }
-#undef PAINTRL_MOVE_FAST
-#undef PAINTRL_MOVE
-    }
-    int rc = launch_check(h, "move_kernel");
+    const int rc = step_io(h, actions_dev, obs_dev, reward_dev, penalty_dev, actual_dev, done_dev, new_texels_dev, next_obs_dev,
+                           reset_start_idx_dev, &io);
     if (rc != PAINTRL_OK) return rc;
-    const bool staged = h->pk.n_words_pad <= kStageWords && !h->force_unstaged;
-    const int pw = h->paint_warps;
-    const dim3 grid((h->num_envs + pw - 1) / pw), block(pw * 32);
-    cudaStream_t s = as_stream(stream);
-    const bool ax12 = h->pk.axis0 == 1 && h->pk.axis1 == 2;
-    // programmatic dependent launch after move_kernel (see griddepcontrol.* in the kernels)
-    cudaLaunchConfig_t lc{};
-    lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = 0; lc.stream = s;
-    cudaLaunchAttribute lattr[1];
-    lattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    lattr[0].val.programmaticStreamSerializationAllowed = 1;
-    lc.attrs = lattr; lc.numAttrs = 1;
-    const EnvArrays pea = env_arrays(h);
-    cudaError_t perr = cudaSuccess;
-#define PAINTRL_PAINT_W(C, ST, W)                                                                           \
-    do {                                                                                                    \
-        if (!h->carveout_set && h->carveout_percent >= 0) {                                                 \
-            cudaFuncSetAttribute(paint_kernel<C, ST, true, W>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent);  \
-            cudaFuncSetAttribute(paint_kernel<C, ST, false, W>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent); \
-        }                                                                                                   \
-        if (ax12) perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, true, W>, h->pk, h->cfg, pea, h->num_envs, io, (const ColdArgs *)h->cold_args);  \
-        else perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, false, W>, h->pk, h->cfg, pea, h->num_envs, io, (const ColdArgs *)h->cold_args);      \
-    } while (0)
-#define PAINTRL_PAINT(C, ST)                                                                 \
-    do {                                                                                     \
-        if (pw == 1) PAINTRL_PAINT_W(C, ST, 1); else if (pw == 2) PAINTRL_PAINT_W(C, ST, 2); \
-        else PAINTRL_PAINT_W(C, ST, 4);                                                      \
-    } while (0)
-    if (h->color == 0) {
-        if (staged) PAINTRL_PAINT(0, true); else PAINTRL_PAINT(0, false);
-    } else {
-        if (staged) PAINTRL_PAINT(1, true); else PAINTRL_PAINT(1, false);
-    }
-#undef PAINTRL_PAINT
-#undef PAINTRL_PAINT_W
-    h->carveout_set = true;
-    if (perr == cudaSuccess) perr = cudaGetLastError();
-    if (perr != cudaSuccess) {
-        // the move grid is already in flight and will raise the hand-off flags nobody consumes: clear them behind it,
-        // or the next step's paint warps would pass their acquire on stale move outputs
-        cudaGetLastError();
-        cudaMemsetAsync(h->ready, 0, sizeof(unsigned) * (size_t)h->num_envs, s);
-        return fail(PAINTRL_E_CUDA, std::string("paint_kernel: ") + cudaGetErrorString(perr));
-    }
-    h->launches++;
-    return PAINTRL_OK;
+    return launch_step<false>(h, EnvSel{nullptr, 0, h->num_envs}, io, stream);
+}
+
+int paintrl_step_subset(PaintrlHandle h, const int32_t *env_ids_dev, int32_t env_lo, int32_t n, const void *actions_dev,
+                        double *obs_dev, double *reward_dev, double *penalty_dev, double *actual_dev, uint8_t *done_dev,
+                        int32_t *new_texels_dev, double *next_obs_dev, const int32_t *reset_start_idx_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    int rc = check_subset(h, env_ids_dev, env_lo, n);
+    if (rc != PAINTRL_OK) return rc;
+    StepIO io;
+    rc = step_io(h, actions_dev, obs_dev, reward_dev, penalty_dev, actual_dev, done_dev, new_texels_dev, next_obs_dev,
+                 reset_start_idx_dev, &io);
+    if (rc != PAINTRL_OK) return rc;
+    return launch_step<true>(h, EnvSel{env_ids_dev, env_lo, n}, io, stream);
 }
 
 int paintrl_step_host(PaintrlHandle h, const void *actions_host, double *obs_host, double *reward_host,
@@ -1577,56 +1682,18 @@ int paintrl_step_host(PaintrlHandle h, const void *actions_host, double *obs_hos
 int paintrl_step_host_submit(PaintrlHandle h, int32_t slot, const void *actions_host, double *obs_host, double *reward_host,
                              double *penalty_host, double *actual_host, uint8_t *done_host, double *next_obs_host, void *stream) {
     if (!h) return fail(PAINTRL_E_INVALID, "null handle");
-    if (slot < 0 || slot > 1) return fail(PAINTRL_E_INVALID, "slot must be 0 or 1");
-    if (!actions_host || !obs_host || !reward_host || !penalty_host || !actual_host || !done_host)
-        return fail(PAINTRL_E_INVALID, "null I/O buffer");
-    CUDA_TRY(cudaSetDevice(h->device));
-    cudaStream_t s = as_stream(stream);
-    const size_t nenv = (size_t)h->num_envs;
-    const size_t abytes = (h->cfg.action_mode == 0 ? sizeof(long long) : sizeof(double) * h->cfg.action_shape) * nenv;
-    const size_t obytes = sizeof(double) * h->cfg.obs_dim * nenv;
-    const bool want_next = next_obs_host != nullptr, dev_next = want_next && h->cfg.auto_reset;
-    // a slot that is submitted again before it was waited for: its previous copy-out must have drained first
-    if (h->slot_pending[slot]) {
-        CUDA_TRY(cudaStreamWaitEvent(h->copy_in, h->ev_done[slot], 0));
-        CUDA_TRY(cudaStreamWaitEvent(s, h->ev_done[slot], 0));
-    }
-    // copy-in stream: the actions, then the step on the caller's stream behind it
-    CUDA_TRY(cudaMemcpyAsync(h->slot_actions[slot], actions_host, abytes, cudaMemcpyHostToDevice, h->copy_in));
-    CUDA_TRY(cudaEventRecord(h->ev_in[slot], h->copy_in));
-    CUDA_TRY(cudaStreamWaitEvent(s, h->ev_in[slot], 0));
-    unsigned char *d = h->slot_out[slot];
-    double *d_obs = reinterpret_cast<double *>(d);
-    double *d_sc = reinterpret_cast<double *>(d + obytes);
-    double *d_next = dev_next ? reinterpret_cast<double *>(d + obytes + 3 * sizeof(double) * nenv) : nullptr;
-    uint8_t *d_done = d + obytes + 3 * sizeof(double) * nenv + (dev_next ? obytes : 0);
-    int rc = paintrl_step(h, h->slot_actions[slot], d_obs, d_sc, d_sc + nenv, d_sc + 2 * nenv, d_done, nullptr, d_next, nullptr, stream);
+    return host_submit(h, slot, false, 0, h->num_envs, actions_host, obs_host, reward_host, penalty_host, actual_host, done_host,
+                       next_obs_host, stream);
+}
+
+int paintrl_step_host_submit_range(PaintrlHandle h, int32_t slot, int32_t env_lo, int32_t n, const void *actions_host,
+                                   double *obs_host, double *reward_host, double *penalty_host, double *actual_host,
+                                   uint8_t *done_host, double *next_obs_host, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    const int rc = check_subset(h, nullptr, env_lo, n);
     if (rc != PAINTRL_OK) return rc;
-    CUDA_TRY(cudaEventRecord(h->ev_step[slot], s));
-    // copy-out stream: the results, as one copy when the host buffers are carved from one allocation in staging order
-    CUDA_TRY(cudaStreamWaitEvent(h->copy_out, h->ev_step[slot], 0));
-    struct Seg { void *dst; const void *src; size_t n; };
-    Seg segs[7] = {};
-    int ns = 0;
-    auto push = [&](void *dst, const void *src, size_t n) {
-        if (ns > 0 && (const char *)segs[ns - 1].src + segs[ns - 1].n == (const char *)src &&
-            (char *)segs[ns - 1].dst + segs[ns - 1].n == (char *)dst) {
-            segs[ns - 1].n += n;
-        } else {
-            segs[ns].dst = dst; segs[ns].src = src; segs[ns].n = n; ++ns;
-        }
-    };
-    push(obs_host, d_obs, obytes);
-    push(reward_host, d_sc, sizeof(double) * nenv);
-    push(penalty_host, d_sc + nenv, sizeof(double) * nenv);
-    push(actual_host, d_sc + 2 * nenv, sizeof(double) * nenv);
-    if (dev_next) push(next_obs_host, d_next, obytes);
-    push(done_host, d_done, nenv);
-    if (want_next && !dev_next) push(next_obs_host, d_obs, obytes);
-    for (int i = 0; i < ns; ++i) CUDA_TRY(cudaMemcpyAsync(segs[i].dst, segs[i].src, segs[i].n, cudaMemcpyDeviceToHost, h->copy_out));
-    CUDA_TRY(cudaEventRecord(h->ev_done[slot], h->copy_out));
-    h->slot_pending[slot] = true;
-    return PAINTRL_OK;
+    return host_submit(h, slot, true, env_lo, n, actions_host, obs_host, reward_host, penalty_host, actual_host, done_host,
+                       next_obs_host, stream);
 }
 
 int paintrl_step_host_wait(PaintrlHandle h, int32_t slot) {

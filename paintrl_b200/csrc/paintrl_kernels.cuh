@@ -35,6 +35,24 @@ struct StepIO {
     const int32_t *reset_start_idx;
 };
 
+// The environments a subset step serves (SUBSET instantiations of the step kernels): the k-th warp / move group steps
+// environment ids[k] (ids != nullptr) or lo + k, for k < n.  Row k of every StepIO buffer belongs to it.
+struct EnvSel {
+    const int32_t *ids;
+    int lo, n;
+};
+
+// `env` = the environment of the k-th warp / move group; false when it has none.  Without SUBSET the k-th environment
+// (env is k itself, so the whole-batch kernels compile as they did before subsets existed).  Ids outside [0, num_envs)
+// are skipped (the host validates them; the device never indexes out of bounds).
+template <bool SUBSET>
+__device__ __forceinline__ bool step_env(const EnvSel &sel, int k, int num_envs, int &env) {
+    if (!SUBSET) { env = k; return k < num_envs; }
+    if (k >= sel.n) return false;
+    env = sel.ids ? __ldg(&sel.ids[k]) : sel.lo + k;
+    return (unsigned)env < (unsigned)num_envs;
+}
+
 // Per-environment dynamic arrays.
 struct EnvArrays {
     EnvState *states;
@@ -1013,7 +1031,7 @@ __device__ __forceinline__ void stamp_normal(const DevPack &pk, const DevConfig 
 // Robot._get_actions (robot.py:302-329): action -> direction, five guided sub-steps.
 // G lanes per environment (the plane / vertex / triangle lists of a sub-step are short).
 template <int G, bool AX12>
-__device__ __forceinline__ void move_body(const DevPack &pk, const DevConfig &cfg, const EnvArrays &ea, int env, const void *actions) {
+__device__ __forceinline__ void move_body(const DevPack &pk, const DevConfig &cfg, const EnvArrays &ea, int env, int row, const void *actions) {
     const Ax ax = make_ax<AX12>(pk.axis0, pk.axis1);
     const int lane = threadIdx.x & 31;
     const Grp grp = make_grp<G>(lane);
@@ -1030,13 +1048,13 @@ __device__ __forceinline__ void move_body(const DevPack &pk, const DevConfig &cf
     // ---- action -> direction (robot_gym_env.py:342-347, robot.py:390-398, 352-358)
     double u1, u2, new_angle;
     if (cfg.action_mode == 0) {
-        long long a = reinterpret_cast<const long long *>(actions)[env];
+        long long a = reinterpret_cast<const long long *>(actions)[row];
         int ai = (int)min(max(a, 0ll), (long long)cfg.discrete_granularity);   // out-of-range actions are clipped, not rejected (robot.py:390-393)
         u1 = __ldg(&cfg.discrete_table[3 * ai]);
         u2 = __ldg(&cfg.discrete_table[3 * ai + 1]);
         new_angle = __ldg(&cfg.discrete_table[3 * ai + 2]);
     } else {
-        const double *a = reinterpret_cast<const double *>(actions) + (size_t)env * cfg.action_shape;
+        const double *a = reinterpret_cast<const double *>(actions) + (size_t)row * cfg.action_shape;
         double a0 = a[0];
         if (!(-1.0 <= a0 && a0 <= 1.0)) a0 = a0 < -1.0 ? -1.0 : 1.0;   // robot.py:391-393 (a NaN ends up at 1 there too)
         if (cfg.action_shape == 1) {
@@ -1142,14 +1160,15 @@ __device__ __forceinline__ void move_body(const DevPack &pk, const DevConfig &cf
 #endif
 }
 
-template <int G, int MINB, bool AX12>
+template <int G, int MINB, bool AX12, bool SUBSET = false>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, MINB)
-move_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, const void *actions) {
+move_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, const void *actions, EnvSel sel) {
     // programmatic dependent launch: let the paint kernel's CTAs be scheduled as this grid drains
     asm volatile("griddepcontrol.launch_dependents;");
-    const int env = (blockIdx.x * blockDim.x + threadIdx.x) / G;   // launched with 32, 64 or 128 threads per block
-    if (env >= num_envs) return;
-    move_body<G, AX12>(pk, cfg, ea, env, actions);
+    const int k = (blockIdx.x * blockDim.x + threadIdx.x) / G;   // launched with 32, 64 or 128 threads per block
+    int env;
+    if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
+    move_body<G, AX12>(pk, cfg, ea, env, k, actions);
 }
 
 // ------------------------------------------------------------------------------ move, fast path
@@ -1323,7 +1342,7 @@ __device__ __forceinline__ int ray_fast(const DevPack &pk, const Ax &ax, const V
 // scratch `sst` / `smv` instead of global memory and no flag is published; returns true when the environment left
 // the fast path (then nothing of `sst` has been changed).
 template <int G, bool AX12, bool DISCRETE, bool FUSED>
-__device__ __forceinline__ bool move_fast_body(const DevPack &pk, const DevConfig &cfg, const EnvArrays &ea, int env, const void *actions,
+__device__ __forceinline__ bool move_fast_body(const DevPack &pk, const DevConfig &cfg, const EnvArrays &ea, int env, int row, const void *actions,
                                                EnvState *sst, MoveOut *smv) {
     const Ax ax = make_ax<AX12>(pk.axis0, pk.axis1);
     const int lane = threadIdx.x & 31;
@@ -1345,13 +1364,13 @@ __device__ __forceinline__ bool move_fast_body(const DevPack &pk, const DevConfi
     // ---- action -> direction (robot_gym_env.py:342-347, robot.py:390-398, 352-358), as in move_body
     double u1, u2, new_angle;
     if (DISCRETE) {
-        const long long a = reinterpret_cast<const long long *>(actions)[env];
+        const long long a = reinterpret_cast<const long long *>(actions)[row];
         const int ai = (int)min(max(a, 0ll), (long long)cfg.discrete_granularity);
         u1 = __ldg(&cfg.discrete_table[3 * ai]);
         u2 = __ldg(&cfg.discrete_table[3 * ai + 1]);
         new_angle = __ldg(&cfg.discrete_table[3 * ai + 2]);
     } else {
-        const double *a = reinterpret_cast<const double *>(actions) + (size_t)env * cfg.action_shape;
+        const double *a = reinterpret_cast<const double *>(actions) + (size_t)row * cfg.action_shape;
         double a0 = a[0];
         if (!(-1.0 <= a0 && a0 <= 1.0)) a0 = a0 < -1.0 ? -1.0 : 1.0;
         if (cfg.action_shape == 1) {
@@ -1447,32 +1466,34 @@ __device__ __forceinline__ bool move_fast_body(const DevPack &pk, const DevConfi
 #ifndef PAINTRL_MOVE_FAST_MINB
 #define PAINTRL_MOVE_FAST_MINB 7
 #endif
-template <int G, bool AX12, bool DISCRETE>
+template <int G, bool AX12, bool DISCRETE, bool SUBSET = false>
 __global__ void __launch_bounds__(kWarpsPerBlock * 32, PAINTRL_MOVE_FAST_MINB)
-move_fast_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, const void *actions) {
+move_fast_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, const void *actions, EnvSel sel) {
     asm volatile("griddepcontrol.launch_dependents;");
-    const int env = (blockIdx.x * blockDim.x + threadIdx.x) / G;
-    if (env >= num_envs) return;
+    const int k = (blockIdx.x * blockDim.x + threadIdx.x) / G;
+    int env;
+    if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
     if (cfg.debug_bail_mod > 0 && env % cfg.debug_bail_mod == 0) {      // tests: exercise the hand-over to the paint warp
         if ((threadIdx.x & (G - 1)) == 0) asm volatile("st.release.gpu.global.u32 [%0], %1;" ::"l"(ea.ready + env), "r"(kReadyBailed) : "memory");
         return;
     }
-    move_fast_body<G, AX12, DISCRETE, false>(pk, cfg, ea, env, actions, nullptr, nullptr);
+    move_fast_body<G, AX12, DISCRETE, false>(pk, cfg, ea, env, k, actions, nullptr, nullptr);
 }
 
 // The generic move of ONE environment, called by its paint warp when the fast move kernel bailed out.  Deliberately a
 // real call (noinline) on a copy of the kernel arguments in global memory: the cold path's registers and spills stay
-// out of the paint kernel's own allocation.
+// out of the paint kernel's own allocation.  `row`: the environment's row of the actions.
 struct ColdArgs { DevPack pk; DevConfig cfg; EnvArrays ea; };
-__device__ __noinline__ void move_generic_cold(const ColdArgs *ca, int env, const void *actions) {
-    move_body<32, false>(ca->pk, ca->cfg, ca->ea, env, actions);
+__device__ __noinline__ void move_generic_cold(const ColdArgs *ca, int env, int row, const void *actions) {
+    move_body<32, false>(ca->pk, ca->cfg, ca->ea, env, row, actions);
 }
 
 // Everything after the move: stamp, score, observe, auto-reset.  (STAGED) the environment's flip bits
 // come in through a TMA bulk copy issued before the warp waits for its environment's hand-off flag and go
-// back the same way; the record and the move kernel's output follow the flag with L2 loads.
+// back the same way; the record and the move kernel's output follow the flag with L2 loads.  State is indexed by
+// `env`, the I/O buffers of `io` by `row` (the same in a whole-batch step).
 template <int COLOR, bool STAGED, bool AX12, bool FUSED = false, bool DISCRETE = false, bool NORMAL = false>
-__device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &cfg, const EnvArrays &ea, int env, const StepIO &io,
+__device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &cfg, const EnvArrays &ea, int env, int row, const StepIO &io,
                                            WarpScratch<STAGED> &ws, const ColdArgs *cold, NormalScratch *ns = nullptr) {
     const Ax ax = make_ax<AX12>(pk.axis0, pk.axis1);
     typedef WarpScratch<STAGED> WS;
@@ -1499,7 +1520,7 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
         if (lane < 8) reinterpret_cast<double2 *>(&ws.st)[lane] = __ldcg(reinterpret_cast<const double2 *>(&ea.states[env]) + lane);
         __syncwarp();
         if (cfg.debug_bail_mod > 0 && env % cfg.debug_bail_mod == 0) bailed = 1;      // tests: force the generic path
-        else bailed = move_fast_body<32, AX12, DISCRETE, true>(pk, cfg, ea, env, io.actions, &ws.st, &ws.mv) ? 1 : 0;
+        else bailed = move_fast_body<32, AX12, DISCRETE, true>(pk, cfg, ea, env, row, io.actions, &ws.st, &ws.mv) ? 1 : 0;
         __syncwarp();
     } else {
         // Launched with programmatic stream serialization: this grid's CTAs start as soon as every CTA of the
@@ -1523,7 +1544,7 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
     if (bailed) {
         // the fast move phase could not decide one of this environment's rays from its move cell alone and wrote
         // nothing: run the generic move here (verify pass / full plane scan / vertex-grid search), then paint
-        move_generic_cold(cold, env, io.actions);
+        move_generic_cold(cold, env, row, io.actions);
         __threadfence();
         if (lane == 0) ea.ready[env] = 0u;      // move_body published 1: consumed
     }
@@ -1649,8 +1670,8 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
 
     // ---- write the observation (robot_gym_env.py:306-319)
     const bool resetting = done && cfg.auto_reset;
-    double *obs = io.obs + (size_t)env * cfg.obs_dim;
-    double *next_obs = io.next_obs ? io.next_obs + (size_t)env * cfg.obs_dim : nullptr;
+    double *obs = io.obs + (size_t)row * cfg.obs_dim;
+    double *next_obs = io.next_obs ? io.next_obs + (size_t)row * cfg.obs_dim : nullptr;
     if (resetting) next_obs = nullptr;
     if (fast4) {
         if (lane >= 2 && lane < 6) {
@@ -1671,15 +1692,15 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
     } else {
         write_observation(pk, ax, cfg, bits, grid_cnt, cur_p, lane, ws, obs, next_obs PAINTRL_PROF_PASS);
     }
-    if (io.next_obs) next_obs = io.next_obs + (size_t)env * cfg.obs_dim;
+    if (io.next_obs) next_obs = io.next_obs + (size_t)row * cfg.obs_dim;
     __syncwarp();
     PAINTRL_PROF(25, lane == 0);
     if (lane == 0) {
-        io.reward[env] = reward;
-        io.penalty[env] = penalty;
-        io.actual[env] = actual;
-        io.done[env] = done ? 1 : 0;
-        if (io.new_texels) io.new_texels[env] = n_new;
+        io.reward[row] = reward;
+        io.penalty[row] = penalty;
+        io.actual[row] = actual;
+        io.done[row] = done ? 1 : 0;
+        if (io.new_texels) io.new_texels[row] = n_new;
         EnvStat *es = &ea.env_stats[env];       // no other thread touches this record: plain reductions, no return value
         if (done) atomicAdd(&es->episodes_ended, 1ull);
         if (n_possible) atomicAdd(&es->footprint_texels, (unsigned long long)n_possible);
@@ -1699,7 +1720,7 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
 
     // ---- same-step auto-reset: `obs` keeps the terminal observation, `next_obs` gets reset()'s
     if (resetting) {
-        int idx = io.reset_start_idx ? io.reset_start_idx[env] : auto_start_index(pk, cfg, env, st.episode);
+        int idx = io.reset_start_idx ? io.reset_start_idx[row] : auto_start_index(pk, cfg, env, st.episode);
         idx = min(max(idx, 0), pk.n_starts - 1);
         clear_planes(pk, bits, gbits, thick, grid_cnt, lane);
         if (ea.last_mask)
@@ -1725,25 +1746,27 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
 #ifndef PAINTRL_PAINT_OCC
 #define PAINTRL_PAINT_OCC 28
 #endif
-template <int COLOR, bool STAGED, bool AX12, int WPB>
+template <int COLOR, bool STAGED, bool AX12, int WPB, bool SUBSET = false>
 __global__ void __launch_bounds__(WPB * 32, (STAGED ? PAINTRL_PAINT_OCC : 16) / WPB)
-paint_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold) {
+paint_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold, EnvSel sel) {
     __shared__ WarpScratch<STAGED> scratch[WPB];
     const int warp = threadIdx.x >> 5;
-    const int env = blockIdx.x * WPB + warp;
-    if (env >= num_envs) return;
-    paint_body<COLOR, STAGED, AX12>(pk, cfg, ea, env, io, scratch[warp], cold);
+    const int k = blockIdx.x * WPB + warp;
+    int env;
+    if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
+    paint_body<COLOR, STAGED, AX12>(pk, cfg, ea, env, k, io, scratch[warp], cold);
 }
 
 // Paint kernel of the normal paint method (staged plane, generic axes; one warp per block).
-template <int COLOR>
+template <int COLOR, bool SUBSET = false>
 __global__ void __launch_bounds__(32, 14)   // 15 KB of shared memory per warp: 14 warps per SM
-paint_normal_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold) {
+paint_normal_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold, EnvSel sel) {
     __shared__ WarpScratch<true> scratch[1];
     __shared__ NormalScratch nscratch[1];
-    const int env = blockIdx.x;
-    if (env >= num_envs) return;
-    paint_body<COLOR, true, false, false, false, true>(pk, cfg, ea, env, io, scratch[0], cold, &nscratch[0]);
+    const int k = blockIdx.x;
+    int env;
+    if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
+    paint_body<COLOR, true, false, false, false, true>(pk, cfg, ea, env, k, io, scratch[0], cold, &nscratch[0]);
 }
 
 // The whole step of one environment in one warp (batches that cannot fill the GPU twice over: the two-kernel step
@@ -1751,15 +1774,16 @@ paint_normal_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepI
 #ifndef PAINTRL_FUSED_WPB
 #define PAINTRL_FUSED_WPB 1      // warps (= environments) per CTA of the one-kernel step
 #endif
-template <int COLOR, bool STAGED, bool AX12, bool DISCRETE>
+template <int COLOR, bool STAGED, bool AX12, bool DISCRETE, bool SUBSET = false>
 __global__ void __launch_bounds__(32 * PAINTRL_FUSED_WPB, (STAGED ? PAINTRL_PAINT_OCC : 16) / PAINTRL_FUSED_WPB)
-step_fused_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold) {
+step_fused_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold, EnvSel sel) {
     __shared__ WarpScratch<STAGED> scratch[PAINTRL_FUSED_WPB];
     const int warp = threadIdx.x >> 5;
-    const int env = blockIdx.x * PAINTRL_FUSED_WPB + warp;
-    if (env >= num_envs) return;
+    const int k = blockIdx.x * PAINTRL_FUSED_WPB + warp;
+    int env;
+    if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
     l2_prefetch_tables(pk, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
-    paint_body<COLOR, STAGED, AX12, true, DISCRETE>(pk, cfg, ea, env, io, scratch[warp], cold);
+    paint_body<COLOR, STAGED, AX12, true, DISCRETE>(pk, cfg, ea, env, k, io, scratch[warp], cold);
 }
 
 // PaintGymEnv.reset / Robot.reset(pose) for the listed environments, with their first observation.
