@@ -348,6 +348,48 @@ void paintrl_policy_destroy(PaintrlPolicyHandle h);
 int paintrl_policy_act(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, void *actions_dev, float *logp_dev,
                        float *value_dev, float *logits_dev, int32_t sample, void *stream);
 
+/*
+ * Training the policy on the GPU: the PPO learner of the reference's training script (RLlib PPO, ray 0.x).
+ * Parameters travel as one flat FP32 device vector, w1 | b1 | w2 | b2 | w3 | b3, each row-major as in
+ * PaintrlPolicyConfig; paintrl_policy_num_params gives its length (PAINTRL_E_INVALID for shapes the kernels do not take).
+ * paintrl_policy_set_params packs such a vector into the policy engine's device weights on `stream`, at the addresses
+ * the engine already uses: a CUDA graph captured around paintrl_policy_act samples with the new weights on its next replay.
+ */
+int32_t paintrl_policy_num_params(int32_t obs_dim, int32_t n_out);
+int paintrl_policy_set_params(PaintrlPolicyHandle h, const float *params_dev, void *stream);
+
+typedef struct PaintrlPpoConfig {
+    int32_t abi_version;
+    int32_t obs_dim, n_out, discrete;   /* as PaintrlPolicyConfig */
+    int32_t max_minibatch;              /* largest n of paintrl_ppo_grad (sizes the partial-gradient workspace) */
+    float clip_param;                   /* surrogate clip epsilon (RLlib default 0.3) */
+    float vf_clip_param;                /* value clip (RLlib default 10) */
+    float vf_loss_coeff;                /* RLlib default 1 */
+    float entropy_coeff;                /* RLlib default 0 */
+} PaintrlPpoConfig;
+typedef struct PaintrlPpoEngine *PaintrlPpoHandle;
+
+int paintrl_ppo_create(const PaintrlPpoConfig *cfg, int32_t device, PaintrlPpoHandle *out);
+void paintrl_ppo_destroy(PaintrlPpoHandle h);
+/* The loss gradient of one minibatch, asynchronous on `stream` (two launches, no synchronisation).  Row k of the
+ * minibatch is row idx_dev[k] of the flattened fragment (idx int32 [n]; the indices are the caller's contract):
+ * obs float64 [rows][obs_dim], actions int64 [rows] (discrete) or float64 [rows][n_out], logp_old / value_old / adv /
+ * vtarg float32 [rows], logits_old float32 [rows][n_out + 1] (the act kernel's logits output).  Loss, averaged over the
+ * n rows: -min(A r, A clip(r, 1 +- clip)) + kl_coeff KL(old || new) + vf_loss_coeff max((v - R)^2, (v_old + clip(v -
+ * v_old, +-vf_clip) - R)^2) - entropy_coeff H.  Writes grad_dev float32 [num_params] (overwritten, not accumulated) and
+ * stats_dev float32 [6]: policy loss, value loss, KL, entropy, clip fraction, mean ratio.  Bitwise reproducible. */
+int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                     const void *actions_dev, const float *logp_old_dev, const float *value_old_dev, const float *logits_old_dev,
+                     const float *adv_dev, const float *vtarg_dev, float kl_coeff, float *grad_dev, float *stats_dev, void *stream);
+/* The learner kernel's forward pass alone: out_dev float32 [n][n_out + 1], logits | means, then the value -- equal to
+ * paintrl_policy_act's logits output for the same weights, bit for bit. */
+int paintrl_ppo_forward(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                        float *out_dev, void *stream);
+/* Adam (torch.optim.Adam's arithmetic, bias-corrected, no gradient clipping) over n_params FP32 values; m / v are the
+ * caller's moment buffers (zero before step 1); step counts from 1. */
+int paintrl_adam_step(float *params_dev, const float *grad_dev, float *m_dev, float *v_dev, int32_t n_params, float lr,
+                      float beta1, float beta2, float eps, int32_t step, void *stream);
+
 const char *paintrl_last_error(void);
 int32_t paintrl_abi_version(void);
 

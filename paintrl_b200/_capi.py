@@ -85,6 +85,12 @@ class PaintrlPolicyConfig(ctypes.Structure):
                 ('capacity', ctypes.c_int32), ('seed', ctypes.c_uint64)] + [(k, ctypes.POINTER(ctypes.c_float)) for k in ('w1', 'b1', 'w2', 'b2', 'w3', 'b3')]
 
 
+class PaintrlPpoConfig(ctypes.Structure):
+    _fields_ = [('abi_version', ctypes.c_int32), ('obs_dim', ctypes.c_int32), ('n_out', ctypes.c_int32), ('discrete', ctypes.c_int32),
+                ('max_minibatch', ctypes.c_int32), ('clip_param', ctypes.c_float), ('vf_clip_param', ctypes.c_float),
+                ('vf_loss_coeff', ctypes.c_float), ('entropy_coeff', ctypes.c_float)]
+
+
 # name -> (restype, argtypes); every symbol include/paintrl.h declares
 _VP = ctypes.c_void_p
 _I32 = ctypes.c_int32
@@ -123,6 +129,13 @@ SIGNATURES = {
     'paintrl_policy_create': (ctypes.c_int, [ctypes.POINTER(PaintrlPolicyConfig), _I32, ctypes.POINTER(_VP)]),
     'paintrl_policy_destroy': (None, [_VP]),
     'paintrl_policy_act': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP, _I32, _VP]),
+    'paintrl_policy_num_params': (_I32, [_I32, _I32]),
+    'paintrl_policy_set_params': (ctypes.c_int, [_VP, _VP, _VP]),
+    'paintrl_ppo_create': (ctypes.c_int, [ctypes.POINTER(PaintrlPpoConfig), _I32, ctypes.POINTER(_VP)]),
+    'paintrl_ppo_destroy': (None, [_VP]),
+    'paintrl_ppo_grad': (ctypes.c_int, [_VP, _VP, _VP, _I32] + [_VP] * 7 + [ctypes.c_float, _VP, _VP, _VP]),
+    'paintrl_ppo_forward': (ctypes.c_int, [_VP, _VP, _VP, _I32, _VP, _VP, _VP]),
+    'paintrl_adam_step': (ctypes.c_int, [_VP, _VP, _VP, _VP, _I32, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _I32, _VP]),
     'paintrl_last_error': (ctypes.c_char_p, []),
     'paintrl_abi_version': (_I32, []),
 }

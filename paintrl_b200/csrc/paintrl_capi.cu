@@ -14,6 +14,7 @@
 #include "paintrl_raster.cuh"
 #include "paintrl_param.cuh"
 #include "paintrl_policy.cuh"
+#include "paintrl_learn.cuh"
 
 using namespace paintrl;
 
@@ -1319,6 +1320,145 @@ int paintrl_policy_act(PaintrlPolicyHandle h, const double *obs_dev, int32_t bat
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("policy_act_kernel: ") + cudaGetErrorString(err));
     h->launches++;
+    return PAINTRL_OK;
+}
+
+/* ---- the PPO learner, see paintrl_learn.cuh ---- */
+int32_t paintrl_policy_num_params(int32_t obs_dim, int32_t n_out) {
+    if (obs_dim <= 0 || obs_dim > kPolMaxObs || n_out <= 0 || n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the policy kernel takes observations of 1..32 entries and 1..15 action outputs");
+    return ppo_num_params(obs_dim, n_out);
+}
+
+int paintrl_policy_set_params(PaintrlPolicyHandle h, const float *params_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (!params_dev) return fail(PAINTRL_E_INVALID, "null parameter buffer");
+    CUDA_TRY(cudaSetDevice(h->device));
+    const PolicyParams &pp = h->pp;
+    const int n = ppo_num_params(pp.obs_dim, pp.n_out);
+    policy_pack_kernel<<<(n + 255) / 256, 256, 0, as_stream(stream)>>>(params_dev, pp.obs_dim, pp.n_out, const_cast<float *>(pp.w1),
+                                                                        const_cast<float *>(pp.b1), const_cast<__nv_bfloat16 *>(pp.w2_packed),
+                                                                        const_cast<float *>(pp.b2), const_cast<float *>(pp.w3), const_cast<float *>(pp.b3));
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("policy_pack_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
+}
+
+struct PaintrlPpoEngine {
+    int device = 0;
+    PaintrlPpoConfig cfg{};
+    int nparams = 0, max_ctas = 0;
+    float *partial = nullptr, *partial_stats = nullptr;
+    DeviceArena arena;
+};
+
+int paintrl_ppo_create(const PaintrlPpoConfig *cfg, int32_t device, PaintrlPpoHandle *out) {
+    if (!cfg || !out) return fail(PAINTRL_E_INVALID, "null argument");
+    if (cfg->abi_version != PAINTRL_ABI_VERSION) return fail(PAINTRL_E_INVALID, "ABI version mismatch");
+    if (cfg->obs_dim <= 0 || cfg->obs_dim > kPolMaxObs) return fail(PAINTRL_E_INVALID, "the learner kernel takes observations of 1..32 entries");
+    if (cfg->n_out <= 0 || cfg->n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the learner kernel takes 1..15 action outputs");
+    if (cfg->max_minibatch <= 0) return fail(PAINTRL_E_INVALID, "max_minibatch must be positive");
+    if (!(cfg->clip_param > 0.f) || !(cfg->vf_clip_param > 0.f) || !(cfg->vf_loss_coeff >= 0.f) || !(cfg->entropy_coeff >= 0.f))
+        return fail(PAINTRL_E_INVALID, "clip_param and vf_clip_param must be positive, vf_loss_coeff and entropy_coeff non-negative");
+    int count = 0;
+    cudaError_t err = cudaGetDeviceCount(&count);
+    if (err != cudaSuccess || count == 0)
+        return fail(PAINTRL_E_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(err));
+    if (device < 0 || device >= count) return fail(PAINTRL_E_INVALID, "device index out of range");
+    CUDA_TRY(cudaSetDevice(device));
+    PaintrlPpoEngine *e = new PaintrlPpoEngine();
+    e->device = device;
+    e->cfg = *cfg;
+    e->nparams = ppo_num_params(cfg->obs_dim, cfg->n_out);
+    e->max_ctas = (cfg->max_minibatch + kPolRows - 1) / kPolRows;
+    bool ok = e->arena.alloc((void **)&e->partial, sizeof(float) * (size_t)e->max_ctas * e->nparams) == cudaSuccess &&
+              e->arena.alloc((void **)&e->partial_stats, sizeof(float) * (size_t)e->max_ctas * kLrnStatStride) == cudaSuccess;
+    if (ok) ok = cudaFuncSetAttribute(ppo_grad_kernel<8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<8, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<32, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess;
+    if (!ok) { delete e; cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the learner failed (allocation / shared memory opt-in)"); }
+    *out = e;
+    return PAINTRL_OK;
+}
+
+void paintrl_ppo_destroy(PaintrlPpoHandle h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    cudaDeviceSynchronize();
+    delete h;
+}
+
+static int ppo_launch(const PpoGradArgs &a, void *stream) {
+    const dim3 grid((a.n + kPolRows - 1) / kPolRows);
+    const bool small_obs = a.obs_dim <= 8, small_out = a.n_out + 1 <= 8;
+    cudaStream_t s = as_stream(stream);
+    if (small_obs && small_out) ppo_grad_kernel<8, 8><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    else if (small_obs) ppo_grad_kernel<8, 16><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    else if (small_out) ppo_grad_kernel<32, 8><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    else ppo_grad_kernel<32, 16><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_grad_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
+}
+
+static void ppo_args(PaintrlPpoHandle h, PpoGradArgs &a, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev) {
+    a = PpoGradArgs{};
+    a.obs_dim = h->cfg.obs_dim; a.n_out = h->cfg.n_out; a.discrete = h->cfg.discrete ? 1 : 0; a.n = n; a.nparams = h->nparams;
+    a.params = params_dev; a.idx = idx_dev; a.obs = obs_dev;
+    a.partial = h->partial; a.partial_stats = h->partial_stats;
+}
+
+int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                     const void *actions_dev, const float *logp_old_dev, const float *value_old_dev, const float *logits_old_dev,
+                     const float *adv_dev, const float *vtarg_dev, float kl_coeff, float *grad_dev, float *stats_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (!params_dev || !idx_dev || !obs_dev || !actions_dev || !logp_old_dev || !value_old_dev || !logits_old_dev || !adv_dev ||
+        !vtarg_dev || !grad_dev || !stats_dev)
+        return fail(PAINTRL_E_INVALID, "null buffer");
+    if (n <= 0 || n > h->cfg.max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+    if (!(kl_coeff >= 0.f)) return fail(PAINTRL_E_INVALID, "kl_coeff must be non-negative");
+    CUDA_TRY(cudaSetDevice(h->device));
+    PpoGradArgs a;
+    ppo_args(h, a, params_dev, idx_dev, n, obs_dev);
+    a.actions = actions_dev; a.logp_old = logp_old_dev; a.value_old = value_old_dev; a.logits_old = logits_old_dev;
+    a.adv = adv_dev; a.vtarg = vtarg_dev;
+    a.clip = h->cfg.clip_param; a.vf_clip = h->cfg.vf_clip_param; a.vf_coeff = h->cfg.vf_loss_coeff; a.ent_coeff = h->cfg.entropy_coeff;
+    a.kl_coeff = kl_coeff; a.inv_n = 1.f / (float)n;
+    int rc = ppo_launch(a, stream);
+    if (rc != PAINTRL_OK) return rc;
+    const int nparts = (n + kPolRows - 1) / kPolRows;
+    ppo_reduce_kernel<<<(h->nparams + 255) / 256, 256, 0, as_stream(stream)>>>(h->partial, nparts, h->nparams, grad_dev, h->partial_stats,
+                                                                                a.inv_n, stats_dev);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_reduce_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
+}
+
+int paintrl_ppo_forward(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                        float *out_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (!params_dev || !idx_dev || !obs_dev || !out_dev) return fail(PAINTRL_E_INVALID, "null buffer");
+    if (n <= 0 || n > h->cfg.max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+    CUDA_TRY(cudaSetDevice(h->device));
+    PpoGradArgs a;
+    ppo_args(h, a, params_dev, idx_dev, n, obs_dev);
+    a.forward_only = 1;
+    a.fwd_out = out_dev;
+    return ppo_launch(a, stream);
+}
+
+int paintrl_adam_step(float *params_dev, const float *grad_dev, float *m_dev, float *v_dev, int32_t n_params, float lr, float beta1,
+                      float beta2, float eps, int32_t step, void *stream) {
+    if (!params_dev || !grad_dev || !m_dev || !v_dev) return fail(PAINTRL_E_INVALID, "null buffer");
+    if (n_params <= 0) return fail(PAINTRL_E_INVALID, "n_params must be positive");
+    if (step < 1) return fail(PAINTRL_E_INVALID, "step counts from 1");
+    if (!(lr >= 0.f) || !(beta1 >= 0.f && beta1 < 1.f) || !(beta2 >= 0.f && beta2 < 1.f) || !(eps > 0.f))
+        return fail(PAINTRL_E_INVALID, "lr >= 0, beta1 / beta2 in [0, 1) and eps > 0 are required");
+    const double bc1 = 1.0 - std::pow((double)beta1, (double)step), bc2 = 1.0 - std::pow((double)beta2, (double)step);
+    adam_kernel<<<(n_params + 255) / 256, 256, 0, as_stream(stream)>>>(params_dev, grad_dev, m_dev, v_dev, n_params, (float)(lr / bc1), beta1,
+                                                                        beta2, eps, (float)std::sqrt(bc2));
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("adam_kernel: ") + cudaGetErrorString(err));
     return PAINTRL_OK;
 }
 

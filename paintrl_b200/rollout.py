@@ -61,6 +61,13 @@ class NativePolicy(object):
         _capi.check(self._lib.paintrl_policy_act(self._h, p(obs), B, p(actions), p(logp), p(value), p(logits), int(bool(sample)),
                                                  ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
 
+    def set_params(self, params):
+        """Pack a flat FP32 parameter vector (w1 | b1 | w2 | b2 | w3 | b3, a contiguous CUDA tensor of this device) into
+        this engine's device weights, in place and on the current stream: a captured rollout graph samples with the new
+        weights on its next replay."""
+        _capi.check(self._lib.paintrl_policy_set_params(self._h, ctypes.c_void_p(params.data_ptr()),
+                                                        ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+
 
 class MlpPolicy(object):
     """Fully connected policy of paint_ppo.py:179-183: obs -> 256 -> 128 -> {logits | mean, value},
@@ -136,7 +143,7 @@ class MlpPolicy(object):
 class RolloutFragment(object):
     """Time-major buffers of one fragment: T steps of B environments, all on the device."""
 
-    def __init__(self, T, B, obs_dim, action_shape, device):
+    def __init__(self, T, B, obs_dim, action_shape, device, logits_dim=None):
         f64, f32 = torch.float64, torch.float32
         self.T, self.B = T, B
         self.obs = torch.zeros(T + 1, B, obs_dim, dtype=f64, device=device)     # obs[t] is what the policy saw at step t
@@ -150,25 +157,33 @@ class RolloutFragment(object):
         self.new_texels = torch.zeros(T, B, dtype=torch.int32, device=device)
         self.logp = torch.zeros(T, B, dtype=f32, device=device)
         self.value = torch.zeros(T + 1, B, dtype=f32, device=device)
+        # the policy's logits | means and value at step t (the PPO learner's KL term); only with keep_logits
+        self.logits = torch.zeros(T, B, logits_dim, dtype=f32, device=device) if logits_dim else None
 
 
 class RolloutWorker(object):
     """Collects fragments from a `BatchedPaintEnv` created with `auto_reset=True`."""
 
-    def __init__(self, env, policy, fragment_length=100, use_cuda_graph=False, use_native_policy=True):
+    def __init__(self, env, policy, fragment_length=100, use_cuda_graph=False, use_native_policy=True, keep_logits=False):
         """`use_cuda_graph`: after one eager fragment, capture the whole T-step loop (policy kernels and the
         two step kernels per step, ~25 launches each) into one CUDA graph and replay it per fragment -- the
         fragment buffers are persistent, so every address in the loop is static.  Small batches are
-        launch-bound without it."""
+        launch-bound without it.
+        `keep_logits`: the policy kernel also writes its logits | means and value into `fragment.logits`
+        [T, B, n_out + 1] (what `ppo.PPOLearner` needs for the KL term); needs the native policy."""
         if not env.cfg.auto_reset:
             raise ValueError('RolloutWorker needs an environment created with auto_reset=True')
         self.env, self.policy, self.T = env, policy, int(fragment_length)
         if use_native_policy and hasattr(policy, 'enable_native'):
             policy.enable_native(env.num_envs)
+        self.keep_logits = bool(keep_logits)
+        if self.keep_logits and getattr(policy, 'native', None) is None:
+            raise ValueError('keep_logits needs the native policy kernel (obs_dim <= 32, n_out <= 15, hidden layers 256, 128)')
         self.use_cuda_graph = bool(use_cuda_graph)
         self._graph, self._eager_fragments, self.graph_error = None, 0, None
         shape = () if env.cfg.action_mode == 'discrete' else (env.action_dim,)
-        self.frag = RolloutFragment(self.T, env.num_envs, env.obs_dim, shape, env.device)
+        self.frag = RolloutFragment(self.T, env.num_envs, env.obs_dim, shape, env.device,
+                                    logits_dim=policy.n_out + 1 if self.keep_logits else None)
         dev, B = env.device, env.num_envs
         # running per-episode totals (the reference's on_episode_step / on_episode_end callbacks)
         self.ep_reward = torch.zeros(B, dtype=torch.float64, device=dev)
@@ -194,7 +209,7 @@ class RolloutWorker(object):
         for t in range(self.T):
             if native is not None:
                 # one launch: obs[t] -> actions[t], logp[t], value[t] written in place (no torch kernels in the loop)
-                native.act_into(f.obs[t], f.actions[t], f.logp[t], f.value[t])
+                native.act_into(f.obs[t], f.actions[t], f.logp[t], f.value[t], logits=None if f.logits is None else f.logits[t])
             else:
                 a, logp, value = pol.act(f.obs[t])
                 f.actions[t].copy_(a)
