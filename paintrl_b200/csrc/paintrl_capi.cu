@@ -1604,6 +1604,7 @@ int paintrl_create(const PaintrlPartPack *pack, const PaintrlConfig *cfg, int32_
         e->paint_normal = true;
     }
     { const char *bm = getenv("PAINTRL_DEBUG_BAIL_MOD"); c.debug_bail_mod = bm ? std::max(0, atoi(bm)) : 0; }
+    { const char *so = getenv("PAINTRL_START_ORDER"); c.start_order = so ? (atoi(so) != 0 ? 1 : 0) : 1; }
     c.seed = cfg->seed;
 
     const size_t bits_bytes = (size_t)num_envs * e->pk.n_words_pad * sizeof(unsigned);

@@ -242,6 +242,8 @@ struct DevConfig {
     int n_beams;
     const double *beam_plain;       // [n_beams][3] Robot._paint_plain, ray end points in the TCP frame
     int debug_bail_mod;             // PAINTRL_DEBUG_BAIL_MOD=n (tests): every n-th environment leaves the fast move kernel at once
+    int start_order;                // PAINTRL_START_ORDER (default 1): the one-kernel step loads the record before the L2 sweep and
+                                    // copies the bit-plane in after the move phase; 0: sweep, copy, record (results are the same)
     unsigned long long seed;
 };
 

@@ -1504,11 +1504,20 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
     unsigned *gbits = bits_of(pk, ea, env), *grid_cnt = grid_cnt_of(pk, ea, env);
     int16_t *thick = thick_of(pk, ea, env);
     const unsigned plane_bytes = (unsigned)pk.n_words_pad * 4u;
-    if (STAGED && lane == 0) {
-        mbar_init(&ws.bar, 1);
-        mbar_expect_tx(&ws.bar, plane_bytes);
-        bulk_g2s(ws.sbits, gbits, plane_bytes, &ws.bar);   // not written by the move kernel
-    }
+    // The bit-plane copy in, issued exactly once per step before mbar_wait.  One-kernel step with start_order: the
+    // plane is not needed before the stamp, so its copy goes out after the move phase (before the generic move when
+    // the fast one bails) instead of queueing in front of the record load and the move's first table lookups.
+    const bool late_copy = FUSED && STAGED && !NORMAL && cfg.start_order;
+    auto issue_copy = [&]() {
+        if (STAGED && lane == 0) {
+            mbar_init(&ws.bar, 1);
+            mbar_expect_tx(&ws.bar, plane_bytes);
+            bulk_g2s(ws.sbits, gbits, plane_bytes, &ws.bar);   // not written by the move phase
+        }
+    };
+    const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x, nthreads = gridDim.x * blockDim.x;
+    if (FUSED && !cfg.start_order) l2_prefetch_tables(pk, tid, nthreads);
+    if (!late_copy) issue_copy();
     // Launched with programmatic stream serialization: this grid's CTAs start as soon as every CTA of the
     // move kernel has started, and each warp waits only for ITS environment's move phase (acquire of the
     // flag the move warp released) -- not for the whole grid: a slow environment of the move phase delays
@@ -1518,10 +1527,15 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
         // One warp runs the whole step of its environment: the record comes into the scratch, the fast move phase
         // works on that copy (the bit-plane copy issued above lands meanwhile), the paint phase continues on it.
         if (lane < 8) reinterpret_cast<double2 *>(&ws.st)[lane] = __ldcg(reinterpret_cast<const double2 *>(&ea.states[env]) + lane);
+        // start_order: the record load is every warp's first dependent load, so it goes out before the sweep's prefetches
+        if (cfg.start_order) l2_prefetch_tables(pk, tid, nthreads);
         __syncwarp();
         if (cfg.debug_bail_mod > 0 && env % cfg.debug_bail_mod == 0) bailed = 1;      // tests: force the generic path
         else bailed = move_fast_body<32, AX12, DISCRETE, true>(pk, cfg, ea, env, row, io.actions, &ws.st, &ws.mv) ? 1 : 0;
         __syncwarp();
+        // after the move, not inside it: a copy issued inside the sub-step loop keeps its operands live there (+40 / +96
+        // bytes of spill stores / loads in the C2 kernel)
+        if (late_copy) issue_copy();
     } else {
         // Launched with programmatic stream serialization: this grid's CTAs start as soon as every CTA of the
         // move kernel has started, and each warp waits only for ITS environment's move phase (acquire of the
@@ -1560,7 +1574,7 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
         }
         __syncwarp();
     }
-    if (STAGED) mbar_wait(&ws.bar, 0);
+    if (STAGED && !late_copy) mbar_wait(&ws.bar, 0);      // a late copy is waited for after the row ranks below
     PAINTRL_TRACE_MARK(env, 4, lane == 0);
     PAINTRL_PROF(16, lane == 0);
     const Bits<STAGED> bits = {gbits, ws.sbits};
@@ -1578,6 +1592,7 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
             for (int k = lane; k < 2 * (w1 - w0); k += 32) prefetch_l1(ky + (size_t)k * 128);
         }
     }
+    if (STAGED && late_copy) mbar_wait(&ws.bar, 0);
     PAINTRL_PROF(15, lane == 0);
 
     // ---- stamp the 5 shots (bullet_paint_wrapper.py:568-577)
@@ -1782,8 +1797,7 @@ step_fused_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO 
     const int k = blockIdx.x * PAINTRL_FUSED_WPB + warp;
     int env;
     if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
-    l2_prefetch_tables(pk, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
-    paint_body<COLOR, STAGED, AX12, true, DISCRETE>(pk, cfg, ea, env, k, io, scratch[warp], cold);
+    paint_body<COLOR, STAGED, AX12, true, DISCRETE>(pk, cfg, ea, env, k, io, scratch[warp], cold);   // sweeps the tables into L2
 }
 
 // PaintGymEnv.reset / Robot.reset(pose) for the listed environments, with their first observation.
