@@ -43,7 +43,7 @@ def build(force=False, verbose=False):
         return LIB
     extra = ['-DPAINTRL_PROFILE'] if os.environ.get('PAINTRL_PROFILE') else []   # phase timing build (profiles/)
     extra += ['-DPAINTRL_TRACE'] if os.environ.get('PAINTRL_TRACE') else []     # per-warp timeline build (profiles/timeline.py)
-    extra += os.environ.get('PAINTRL_NVCC_EXTRA', '').split()                    # experiments, e.g. -DPAINTRL_PAINT_OCC=32
+    extra += os.environ.get('PAINTRL_NVCC_EXTRA', '').split()                    # experiments, e.g. -Xptxas=-O3
     cmd = [nvcc_path()] + NVCC_FLAGS + extra + (['-Xptxas', '-v'] if verbose else []) + SOURCES + ['-o', LIB]
     res = subprocess.run(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)
     if verbose or res.returncode != 0:

@@ -109,12 +109,6 @@ struct PaintrlEngine {
     bool paint_normal = false;
     unsigned *ready = nullptr;       // [num_envs] per-environment move -> paint hand-off flags: 1 = this step's move output is published;
                                      // the paint warp clears it.  All steps of one handle must be issued on ONE stream (or ordered streams).
-    // PAINTRL_CARVEOUT=<percent>: ask for the same L1 / shared-memory split for both step kernels, so that paint CTAs can
-    // share an SM with the move kernel's last wave (CTAs of kernels with different carveouts cannot).  Off by default:
-    // measured slower at C2 (the move phase loses L1 and issue slots to the co-resident paint warps).
-    int carveout_percent = -1;
-    bool carveout_set = false;       // the step kernels' shared-memory carveout has been requested on this device
-    bool carveout_set_subset = false;   // the same for their subset instantiations
     // staging for the host-buffer entry points
     void *stage_actions = nullptr;
     // paintrl_step_host: one contiguous block, laid out per call as obs | reward | penalty | actual | [next_obs] | done,
@@ -129,12 +123,9 @@ struct PaintrlEngine {
     bool slot_pending[2] = {false, false};
     unsigned long long launches = 0;
     double move_cell_planes_mean = 0.0, move_cell_verts_mean = 0.0;
-    int move_lanes = 32;             // lanes per environment in move_kernel (8, 16 or 32)
-    int move_warps = 4, paint_warps = 1;   // warps per block of the two step kernels (1, 2 or 4)
-    int move_minb = 4;               // its __launch_bounds__ min blocks per SM (4: 128 registers, 7: 72)
+    int move_lanes = 32;             // lanes per environment in move_fast_kernel of the two-kernel step (8 or 32)
     void *cold_args = nullptr;       // device copy of {pk, cfg, env arrays} for the paint warps' generic-move call (ColdArgs)
     int fused = -1;                  // PAINTRL_FUSED: 1 / 0 force the one-kernel / two-kernel step; -1: by batch size
-    bool move_fast = true;           // PAINTRL_MOVE_FAST=0: the generic move kernel instead of the lean fast-path one
     bool force_unstaged = false;     // PAINTRL_FORCE_UNSTAGED: run the global-memory bit-plane path (tests)
 };
 
@@ -819,6 +810,19 @@ int launch_check(PaintrlEngine *e, const char *what) {
     return PAINTRL_OK;
 }
 
+// launch_check for a step's second launch.  On failure the move grid is already in flight and will raise hand-off flags
+// nobody consumes: clear them behind it, or the next step's paint warps would pass their acquire on stale move outputs.
+int paint_check(PaintrlEngine *e, const char *what, cudaError_t err, cudaStream_t s) {
+    if (err == cudaSuccess) err = cudaGetLastError();
+    if (err != cudaSuccess) {
+        cudaGetLastError();
+        cudaMemsetAsync(e->ready, 0, sizeof(unsigned) * (size_t)e->num_envs, s);
+        return fail(PAINTRL_E_CUDA, std::string(what) + ": " + cudaGetErrorString(err));
+    }
+    e->launches++;
+    return PAINTRL_OK;
+}
+
 // The I/O buffers of paintrl_step / paintrl_step_subset, checked and packed for the kernels.
 int step_io(PaintrlHandle h, const void *actions_dev, double *obs_dev, double *reward_dev, double *penalty_dev, double *actual_dev,
             uint8_t *done_dev, int32_t *new_texels_dev, double *next_obs_dev, const int32_t *reset_start_idx_dev, StepIO *io) {
@@ -850,136 +854,72 @@ int check_subset(PaintrlHandle h, const int32_t *env_ids, int32_t env_lo, int32_
 }
 
 // One step of the environments `sel` selects (SUBSET) or of the whole batch (!SUBSET, sel = {nullptr, 0, num_envs}),
-// I/O row k = the k-th selected environment.  The kernel shape follows the number of environments stepped.
+// I/O row k = the k-th selected environment.  The kernel shape follows the paint method and the number of environments
+// stepped: the beam-fan method, else the one-kernel step, else the two-kernel step.
 template <bool SUBSET>
 int launch_step(PaintrlHandle h, const EnvSel &sel, const StepIO &io, void *stream) {
-    const int n = sel.n;
-    const void *actions_dev = io.actions;
-    // the carveout is an attribute of each kernel: the whole-batch and the subset instantiations each ask once
-    bool &carveout_done = SUBSET ? h->carveout_set_subset : h->carveout_set;
     CUDA_TRY(cudaSetDevice(h->device));
+    const int n = sel.n, threads = kWarpsPerBlock * 32;
+    cudaStream_t s = as_stream(stream);
+    const EnvArrays ea = env_arrays(h);
+    const ColdArgs *cold = (const ColdArgs *)h->cold_args;
     if (h->paint_normal) {
         // Robot.PAINT_METHOD == 'normal': the generic move kernel (it also hands over the shots' poses), then the beam-fan
         // paint kernel, one warp per environment
-        cudaStream_t ns = as_stream(stream);
-        const int threads = 128;
-        move_kernel<32, 4, false, SUBSET><<<(n * 32 + threads - 1) / threads, threads, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);
+        move_kernel<SUBSET><<<(n * 32 + threads - 1) / threads, threads, 0, s>>>(h->pk, h->cfg, ea, h->num_envs, io.actions, sel);
         int rc = launch_check(h, "move_kernel");
         if (rc != PAINTRL_OK) return rc;
-        if (h->color == 0) paint_normal_kernel<0, SUBSET><<<n, 32, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, io, (const ColdArgs *)h->cold_args, sel);
-        else paint_normal_kernel<1, SUBSET><<<n, 32, 0, ns>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, io, (const ColdArgs *)h->cold_args, sel);
-        cudaError_t nerr = cudaGetLastError();
-        if (nerr != cudaSuccess) {
-            cudaMemsetAsync(h->ready, 0, sizeof(unsigned) * (size_t)h->num_envs, ns);
-            return fail(PAINTRL_E_CUDA, std::string("paint_normal_kernel: ") + cudaGetErrorString(nerr));
-        }
-        h->launches++;
-        return PAINTRL_OK;
+        if (h->color == 0) paint_normal_kernel<0, SUBSET><<<n, 32, 0, s>>>(h->pk, h->cfg, ea, h->num_envs, io, cold, sel);
+        else paint_normal_kernel<1, SUBSET><<<n, 32, 0, s>>>(h->pk, h->cfg, ea, h->num_envs, io, cold, sel);
+        return paint_check(h, "paint_normal_kernel", cudaSuccess, s);
     }
-    const bool use_fused = h->fused >= 0 ? h->fused == 1 : n < kFusedBelowEnvs;
-    if (use_fused) {
-        // one launch, one warp per environment for the whole step (paintrl_kernels.cuh step_fused_kernel)
-        const bool staged_f = h->pk.n_words_pad <= kStageWords && !h->force_unstaged;
-        const bool ax12f = h->pk.axis0 == 1 && h->pk.axis1 == 2, disc = h->cfg.action_mode == 0;
-        const EnvArrays fea = env_arrays(h);
-        const ColdArgs *cold = (const ColdArgs *)h->cold_args;
-        cudaStream_t fs = as_stream(stream);
-#define PAINTRL_FUSED_K(C, ST, AX, DI) step_fused_kernel<C, ST, AX, DI, SUBSET><<<(n + PAINTRL_FUSED_WPB - 1) / PAINTRL_FUSED_WPB, 32 * PAINTRL_FUSED_WPB, 0, fs>>>(h->pk, h->cfg, fea, h->num_envs, io, cold, sel)
-#define PAINTRL_FUSED_AD(C, ST)                                                        \
-    do {                                                                               \
-        if (ax12f && disc) PAINTRL_FUSED_K(C, ST, true, true);                         \
-        else if (ax12f) PAINTRL_FUSED_K(C, ST, true, false);                           \
-        else if (disc) PAINTRL_FUSED_K(C, ST, false, true);                            \
-        else PAINTRL_FUSED_K(C, ST, false, false);                                     \
+    const bool staged = h->pk.n_words_pad <= kStageWords && !h->force_unstaged;
+    const bool ax12 = h->pk.axis0 == 1 && h->pk.axis1 == 2, discrete = h->cfg.action_mode == 0;
+    // K(args..., AX12, DISCRETE) with the part's axes and the action mode as compile-time constants
+#define PAINTRL_AX_DI(K, ...)                                                                                       \
+    do {                                                                                                            \
+        if (ax12 && discrete) K(__VA_ARGS__, true, true);                                                           \
+        else if (ax12) K(__VA_ARGS__, true, false);                                                                 \
+        else if (discrete) K(__VA_ARGS__, false, true);                                                             \
+        else K(__VA_ARGS__, false, false);                                                                          \
     } while (0)
-        if (h->color == 0) { if (staged_f) PAINTRL_FUSED_AD(0, true); else PAINTRL_FUSED_AD(0, false); }
-        else { if (staged_f) PAINTRL_FUSED_AD(1, true); else PAINTRL_FUSED_AD(1, false); }
-#undef PAINTRL_FUSED_AD
-#undef PAINTRL_FUSED_K
+    if (h->fused >= 0 ? h->fused == 1 : n < kFusedBelowEnvs) {
+        // one launch, one warp per environment for the whole step (paintrl_kernels.cuh step_fused_kernel)
+#define PAINTRL_STEP_FUSED(C, ST, AX, DI)                                                                           \
+    step_fused_kernel<C, ST, AX, DI, SUBSET><<<(n + kFusedWarpsPerBlock - 1) / kFusedWarpsPerBlock,                \
+                                               32 * kFusedWarpsPerBlock, 0, s>>>(h->pk, h->cfg, ea, h->num_envs, io, cold, sel)
+        if (h->color == 0) { if (staged) PAINTRL_AX_DI(PAINTRL_STEP_FUSED, 0, true); else PAINTRL_AX_DI(PAINTRL_STEP_FUSED, 0, false); }
+        else { if (staged) PAINTRL_AX_DI(PAINTRL_STEP_FUSED, 1, true); else PAINTRL_AX_DI(PAINTRL_STEP_FUSED, 1, false); }
+#undef PAINTRL_STEP_FUSED
         return launch_check(h, "step_fused_kernel");
     }
-    {   // lanes per environment in the move phase: fewer when there are enough environments to fill the GPU
-        const int threads = h->move_warps * 32;
-        cudaStream_t ms = as_stream(stream);
-        const int L = h->move_lanes;
-        const int mblocks = (int)(((long long)n * L + threads - 1) / threads);
-        const bool ax12m = h->pk.axis0 == 1 && h->pk.axis1 == 2;
-#define PAINTRL_MOVE(G, MINB)                                                                                              \
-    do {                                                                                                                   \
-        if (!carveout_done && h->carveout_percent >= 0) {                                                                \
-            cudaFuncSetAttribute(move_kernel<G, MINB, true, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent);  \
-            cudaFuncSetAttribute(move_kernel<G, MINB, false, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent); \
-        }                                                                                                                  \
-        if (ax12m) move_kernel<G, MINB, true, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);  \
-        else move_kernel<G, MINB, false, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);       \
-    } while (0)
-#define PAINTRL_MOVE_FAST(G)                                                                                               \
-    do {                                                                                                                   \
-        if (ax12m && discrete) move_fast_kernel<G, true, true, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);   \
-        else if (ax12m) move_fast_kernel<G, true, false, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);         \
-        else if (discrete) move_fast_kernel<G, false, true, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);      \
-        else move_fast_kernel<G, false, false, SUBSET><<<mblocks, threads, 0, ms>>>(h->pk, h->cfg, env_arrays(h), h->num_envs, actions_dev, sel);                   \
-    } while (0)
-        const bool discrete = h->cfg.action_mode == 0;
-        if (h->move_fast) {
-            // the lean kernel: rays decided by their move cell alone; the rest is handed to the paint warps (kReadyBailed)
-            if (L == 8) PAINTRL_MOVE_FAST(8); else if (L == 16) PAINTRL_MOVE_FAST(16); else PAINTRL_MOVE_FAST(32);
-        } else if (h->move_minb == 7) {
-            if (L == 8) PAINTRL_MOVE(8, 7); else if (L == 16) PAINTRL_MOVE(16, 7); else PAINTRL_MOVE(32, 7);
-        } else {
-            if (L == 8) PAINTRL_MOVE(8, 4); else if (L == 16) PAINTRL_MOVE(16, 4); else PAINTRL_MOVE(32, 4);
-        }
-#undef PAINTRL_MOVE_FAST
-#undef PAINTRL_MOVE
-    }
-    int rc = launch_check(h, "move_kernel");
+    // The lean move kernel, h->move_lanes lanes per environment: rays decided by their move cell alone; the rest is
+    // handed to the paint warps (kReadyBailed).
+    const int mblocks = (int)(((long long)n * h->move_lanes + threads - 1) / threads);
+#define PAINTRL_STEP_MOVE(G, AX, DI) move_fast_kernel<G, AX, DI, SUBSET><<<mblocks, threads, 0, s>>>(h->pk, h->cfg, ea, h->num_envs, io.actions, sel)
+    if (h->move_lanes == 8) PAINTRL_AX_DI(PAINTRL_STEP_MOVE, 8); else PAINTRL_AX_DI(PAINTRL_STEP_MOVE, 32);
+#undef PAINTRL_STEP_MOVE
+#undef PAINTRL_AX_DI
+    int rc = launch_check(h, "move_fast_kernel");
     if (rc != PAINTRL_OK) return rc;
-    const bool staged = h->pk.n_words_pad <= kStageWords && !h->force_unstaged;
-    const int pw = h->paint_warps;
-    const dim3 grid((n + pw - 1) / pw), block(pw * 32);
-    cudaStream_t s = as_stream(stream);
-    const bool ax12 = h->pk.axis0 == 1 && h->pk.axis1 == 2;
-    // programmatic dependent launch after move_kernel (see griddepcontrol.* in the kernels)
+    // the paint kernel, one warp per block, as a programmatic dependent launch after the move kernel (see
+    // griddepcontrol.* in the kernels)
     cudaLaunchConfig_t lc{};
-    lc.gridDim = grid; lc.blockDim = block; lc.dynamicSmemBytes = 0; lc.stream = s;
+    lc.gridDim = dim3(n); lc.blockDim = dim3(32); lc.dynamicSmemBytes = 0; lc.stream = s;
     cudaLaunchAttribute lattr[1];
     lattr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     lattr[0].val.programmaticStreamSerializationAllowed = 1;
     lc.attrs = lattr; lc.numAttrs = 1;
-    const EnvArrays pea = env_arrays(h);
-    cudaError_t perr = cudaSuccess;
-#define PAINTRL_PAINT_W(C, ST, W)                                                                           \
-    do {                                                                                                    \
-        if (!carveout_done && h->carveout_percent >= 0) {                                                 \
-            cudaFuncSetAttribute(paint_kernel<C, ST, true, W, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent);  \
-            cudaFuncSetAttribute(paint_kernel<C, ST, false, W, SUBSET>, cudaFuncAttributePreferredSharedMemoryCarveout, h->carveout_percent); \
-        }                                                                                                   \
-        if (ax12) perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, true, W, SUBSET>, h->pk, h->cfg, pea, h->num_envs, io, (const ColdArgs *)h->cold_args, sel);  \
-        else perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, false, W, SUBSET>, h->pk, h->cfg, pea, h->num_envs, io, (const ColdArgs *)h->cold_args, sel);      \
+    cudaError_t perr;
+#define PAINTRL_STEP_PAINT(C, ST)                                                                                   \
+    do {                                                                                                            \
+        if (ax12) perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, true, SUBSET>, h->pk, h->cfg, ea, h->num_envs, io, cold, sel);  \
+        else perr = cudaLaunchKernelEx(&lc, paint_kernel<C, ST, false, SUBSET>, h->pk, h->cfg, ea, h->num_envs, io, cold, sel);      \
     } while (0)
-#define PAINTRL_PAINT(C, ST)                                                                 \
-    do {                                                                                     \
-        if (pw == 1) PAINTRL_PAINT_W(C, ST, 1); else if (pw == 2) PAINTRL_PAINT_W(C, ST, 2); \
-        else PAINTRL_PAINT_W(C, ST, 4);                                                      \
-    } while (0)
-    if (h->color == 0) {
-        if (staged) PAINTRL_PAINT(0, true); else PAINTRL_PAINT(0, false);
-    } else {
-        if (staged) PAINTRL_PAINT(1, true); else PAINTRL_PAINT(1, false);
-    }
-#undef PAINTRL_PAINT
-#undef PAINTRL_PAINT_W
-    carveout_done = true;
-    if (perr == cudaSuccess) perr = cudaGetLastError();
-    if (perr != cudaSuccess) {
-        // the move grid is already in flight and will raise the hand-off flags nobody consumes: clear them behind it,
-        // or the next step's paint warps would pass their acquire on stale move outputs
-        cudaGetLastError();
-        cudaMemsetAsync(h->ready, 0, sizeof(unsigned) * (size_t)h->num_envs, s);
-        return fail(PAINTRL_E_CUDA, std::string("paint_kernel: ") + cudaGetErrorString(perr));
-    }
-    h->launches++;
-    return PAINTRL_OK;
+    if (h->color == 0) { if (staged) PAINTRL_STEP_PAINT(0, true); else PAINTRL_STEP_PAINT(0, false); }
+    else { if (staged) PAINTRL_STEP_PAINT(1, true); else PAINTRL_STEP_PAINT(1, false); }
+#undef PAINTRL_STEP_PAINT
+    return paint_check(h, "paint_kernel", perr, s);
 }
 
 // paintrl_step_host_submit (subset == false, the whole batch) and paintrl_step_host_submit_range (the environments
@@ -1604,7 +1544,6 @@ int paintrl_create(const PaintrlPartPack *pack, const PaintrlConfig *cfg, int32_
         e->paint_normal = true;
     }
     { const char *bm = getenv("PAINTRL_DEBUG_BAIL_MOD"); c.debug_bail_mod = bm ? std::max(0, atoi(bm)) : 0; }
-    { const char *so = getenv("PAINTRL_START_ORDER"); c.start_order = so ? (atoi(so) != 0 ? 1 : 0) : 1; }
     c.seed = cfg->seed;
 
     const size_t bits_bytes = (size_t)num_envs * e->pk.n_words_pad * sizeof(unsigned);
@@ -1656,20 +1595,10 @@ int paintrl_create(const PaintrlPartPack *pack, const PaintrlConfig *cfg, int32_
         // (the phase is latency-bound there), 8 lanes once it can (then instruction issue is the limit)
         const char *ml = getenv("PAINTRL_MOVE_LANES");
         int lanes = ml ? atoi(ml) : (num_envs < 16384 ? 32 : 8);   // measured: 4096 envs 60 vs 103 us, 16384 envs 292 vs 249 us (32 vs 8 lanes)
-        e->move_lanes = (lanes == 16 || lanes == 8) ? lanes : 32;
+        e->move_lanes = lanes == 8 ? 8 : 32;
         e->force_unstaged = getenv("PAINTRL_FORCE_UNSTAGED") != nullptr;
-        const char *mw = getenv("PAINTRL_MOVE_WARPS"), *pwv = getenv("PAINTRL_PAINT_WARPS");
-        const int mwi = mw ? atoi(mw) : 4, pwi = pwv ? atoi(pwv) : 1;
-        e->move_warps = (mwi == 1 || mwi == 2) ? mwi : 4;
-        e->paint_warps = (pwi == 4 || pwi == 2) ? pwi : 1;   // one warp per block: a finished environment frees its slot at once
-        const char *co = getenv("PAINTRL_CARVEOUT");
-        e->carveout_percent = co ? std::min(100, std::max(-1, atoi(co))) : -1;
         const char *fu = getenv("PAINTRL_FUSED");
         e->fused = fu ? (atoi(fu) != 0 ? 1 : 0) : -1;
-        const char *mf = getenv("PAINTRL_MOVE_FAST");
-        e->move_fast = !(mf && atoi(mf) == 0);
-        const char *mb = getenv("PAINTRL_MOVE_MINB");
-        e->move_minb = (mb && atoi(mb) >= 7) ? 7 : 4;     // 4: 128 registers, two waves at 4096 envs; 7: 72 registers (spills), one wave
     }
     err = cudaStreamCreateWithFlags(&e->copy_in, cudaStreamNonBlocking);
     if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&e->copy_out, cudaStreamNonBlocking);
@@ -1680,11 +1609,10 @@ int paintrl_create(const PaintrlPartPack *pack, const PaintrlConfig *cfg, int32_
     }
     if (err != cudaSuccess) { delete e; return fail(PAINTRL_E_CUDA, std::string("creating the copy streams: ") + cudaGetErrorString(err)); }
     {
-        // L2 prefetch ranges of the static tables (PAINTRL_L2_PREFETCH=0 switches the pass off; tables beyond 48 MB --
-        // multi-megapixel textures -- are left to demand loads)
-        const char *pf = getenv("PAINTRL_L2_PREFETCH");
+        // L2 prefetch ranges of the static tables (tables beyond 48 MB -- multi-megapixel textures -- are left to
+        // demand loads)
         e->pk.pf_n = 0;
-        if (!(pf && atoi(pf) == 0) && e->arena.static_bytes() <= (size_t(48) << 20) && e->arena.slabs.size() <= 4) {
+        if (e->arena.static_bytes() <= (size_t(48) << 20) && e->arena.slabs.size() <= 4) {
             for (const DeviceArena::Slab &s : e->arena.slabs) {
                 e->pk.pf_base[e->pk.pf_n] = s.base;
                 e->pk.pf_lines[e->pk.pf_n] = (unsigned)((s.used + 127) / 128);

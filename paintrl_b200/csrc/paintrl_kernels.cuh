@@ -1160,15 +1160,16 @@ __device__ __forceinline__ void move_body(const DevPack &pk, const DevConfig &cf
 #endif
 }
 
-template <int G, int MINB, bool AX12, bool SUBSET = false>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, MINB)
+// The generic move kernel: the first launch of the beam-fan step (its paint kernel needs every shot's pose).
+template <bool SUBSET>
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, 4)
 move_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, const void *actions, EnvSel sel) {
     // programmatic dependent launch: let the paint kernel's CTAs be scheduled as this grid drains
     asm volatile("griddepcontrol.launch_dependents;");
-    const int k = (blockIdx.x * blockDim.x + threadIdx.x) / G;   // launched with 32, 64 or 128 threads per block
+    const int k = (blockIdx.x * blockDim.x + threadIdx.x) / 32;
     int env;
     if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
-    move_body<G, AX12>(pk, cfg, ea, env, k, actions);
+    move_body<32, false>(pk, cfg, ea, env, k, actions);
 }
 
 // ------------------------------------------------------------------------------ move, fast path
@@ -1463,11 +1464,9 @@ __device__ __forceinline__ bool move_fast_body(const DevPack &pk, const DevConfi
     return false;
 }
 
-#ifndef PAINTRL_MOVE_FAST_MINB
-#define PAINTRL_MOVE_FAST_MINB 7
-#endif
+constexpr int kMoveFastMinBlocks = 7;   // 72 registers, 28 warps per SM: 4096 environments x 32 lanes in one wave
 template <int G, bool AX12, bool DISCRETE, bool SUBSET = false>
-__global__ void __launch_bounds__(kWarpsPerBlock * 32, PAINTRL_MOVE_FAST_MINB)
+__global__ void __launch_bounds__(kWarpsPerBlock * 32, kMoveFastMinBlocks)
 move_fast_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, const void *actions, EnvSel sel) {
     asm volatile("griddepcontrol.launch_dependents;");
     const int k = (blockIdx.x * blockDim.x + threadIdx.x) / G;
@@ -1504,10 +1503,10 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
     unsigned *gbits = bits_of(pk, ea, env), *grid_cnt = grid_cnt_of(pk, ea, env);
     int16_t *thick = thick_of(pk, ea, env);
     const unsigned plane_bytes = (unsigned)pk.n_words_pad * 4u;
-    // The bit-plane copy in, issued exactly once per step before mbar_wait.  One-kernel step with start_order: the
-    // plane is not needed before the stamp, so its copy goes out after the move phase (before the generic move when
-    // the fast one bails) instead of queueing in front of the record load and the move's first table lookups.
-    const bool late_copy = FUSED && STAGED && !NORMAL && cfg.start_order;
+    // The bit-plane copy in, issued exactly once per step before mbar_wait.  One-kernel step: the plane is not needed
+    // before the stamp, so its copy goes out after the move phase (before the generic move when the fast one bails)
+    // instead of queueing in front of the record load and the move's first table lookups.
+    const bool late_copy = FUSED && STAGED && !NORMAL;
     auto issue_copy = [&]() {
         if (STAGED && lane == 0) {
             mbar_init(&ws.bar, 1);
@@ -1515,8 +1514,6 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
             bulk_g2s(ws.sbits, gbits, plane_bytes, &ws.bar);   // not written by the move phase
         }
     };
-    const unsigned tid = blockIdx.x * blockDim.x + threadIdx.x, nthreads = gridDim.x * blockDim.x;
-    if (FUSED && !cfg.start_order) l2_prefetch_tables(pk, tid, nthreads);
     if (!late_copy) issue_copy();
     // Launched with programmatic stream serialization: this grid's CTAs start as soon as every CTA of the
     // move kernel has started, and each warp waits only for ITS environment's move phase (acquire of the
@@ -1527,8 +1524,8 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
         // One warp runs the whole step of its environment: the record comes into the scratch, the fast move phase
         // works on that copy (the bit-plane copy issued above lands meanwhile), the paint phase continues on it.
         if (lane < 8) reinterpret_cast<double2 *>(&ws.st)[lane] = __ldcg(reinterpret_cast<const double2 *>(&ea.states[env]) + lane);
-        // start_order: the record load is every warp's first dependent load, so it goes out before the sweep's prefetches
-        if (cfg.start_order) l2_prefetch_tables(pk, tid, nthreads);
+        // the record load is every warp's first dependent load, so it goes out before the sweep's prefetches
+        l2_prefetch_tables(pk, blockIdx.x * blockDim.x + threadIdx.x, gridDim.x * blockDim.x);
         __syncwarp();
         if (cfg.debug_bail_mod > 0 && env % cfg.debug_bail_mod == 0) bailed = 1;      // tests: force the generic path
         else bailed = move_fast_body<32, AX12, DISCRETE, true>(pk, cfg, ea, env, row, io.actions, &ws.st, &ws.mv) ? 1 : 0;
@@ -1758,18 +1755,16 @@ __device__ __forceinline__ void paint_body(const DevPack &pk, const DevConfig &c
     PAINTRL_TRACE_MARK(env, 5, lane == 0);
 }
 
-#ifndef PAINTRL_PAINT_OCC
-#define PAINTRL_PAINT_OCC 28
-#endif
-template <int COLOR, bool STAGED, bool AX12, int WPB, bool SUBSET = false>
-__global__ void __launch_bounds__(WPB * 32, (STAGED ? PAINTRL_PAINT_OCC : 16) / WPB)
+constexpr int kPaintOcc = 28;   // staged warps per SM (72 registers): 24 (80 registers) took 66 us at C2, a second wave
+// One warp per block: a finished environment frees its slot at once.
+template <int COLOR, bool STAGED, bool AX12, bool SUBSET = false>
+__global__ void __launch_bounds__(32, STAGED ? kPaintOcc : 16)
 paint_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold, EnvSel sel) {
-    __shared__ WarpScratch<STAGED> scratch[WPB];
-    const int warp = threadIdx.x >> 5;
-    const int k = blockIdx.x * WPB + warp;
+    __shared__ WarpScratch<STAGED> scratch[1];
+    const int k = blockIdx.x;
     int env;
     if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
-    paint_body<COLOR, STAGED, AX12>(pk, cfg, ea, env, k, io, scratch[warp], cold);
+    paint_body<COLOR, STAGED, AX12>(pk, cfg, ea, env, k, io, scratch[0], cold);
 }
 
 // Paint kernel of the normal paint method (staged plane, generic axes; one warp per block).
@@ -1786,15 +1781,13 @@ paint_normal_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepI
 
 // The whole step of one environment in one warp (batches that cannot fill the GPU twice over: the two-kernel step
 // pays the move grid's drain before the paint grid's warps get their slots; here a warp goes straight on).
-#ifndef PAINTRL_FUSED_WPB
-#define PAINTRL_FUSED_WPB 1      // warps (= environments) per CTA of the one-kernel step
-#endif
+constexpr int kFusedWarpsPerBlock = 1;   // warps (= environments) per CTA: 2 / 4 took 55.1 / 54.3 us at C2 against 54.0
 template <int COLOR, bool STAGED, bool AX12, bool DISCRETE, bool SUBSET = false>
-__global__ void __launch_bounds__(32 * PAINTRL_FUSED_WPB, (STAGED ? PAINTRL_PAINT_OCC : 16) / PAINTRL_FUSED_WPB)
+__global__ void __launch_bounds__(32 * kFusedWarpsPerBlock, (STAGED ? kPaintOcc : 16) / kFusedWarpsPerBlock)
 step_fused_kernel(DevPack pk, DevConfig cfg, EnvArrays ea, int num_envs, StepIO io, const ColdArgs *cold, EnvSel sel) {
-    __shared__ WarpScratch<STAGED> scratch[PAINTRL_FUSED_WPB];
+    __shared__ WarpScratch<STAGED> scratch[kFusedWarpsPerBlock];
     const int warp = threadIdx.x >> 5;
-    const int k = blockIdx.x * PAINTRL_FUSED_WPB + warp;
+    const int k = blockIdx.x * kFusedWarpsPerBlock + warp;
     int env;
     if (!step_env<SUBSET>(sel, k, num_envs, env)) return;
     paint_body<COLOR, STAGED, AX12, true, DISCRETE>(pk, cfg, ea, env, k, io, scratch[warp], cold);   // sweeps the tables into L2

@@ -8,6 +8,5 @@ for F in 1 0; do
 EXTRA="--workload c2"; run fused${F}_write PAINTRL_FUSED=$F
 EXTRA="--workload c2 --no-flush"; run fused${F}_noflush PAINTRL_FUSED=$F
 done
-EXTRA="--workload c2"; run generic_two PAINTRL_FUSED=0 PAINTRL_MOVE_FAST=0
 ncu --metrics gpu__time_duration.sum --clock-control none -s 10 -c 30 --csv --log-file gpurun_out/launches_fused.csv env PAINTRL_FUSED=1 python bench.py --steps 20 --warmup 5 --no-extra --no-cpu-baseline --no-parity --e2e-sync > /dev/null 2>&1
 grep -E "step_fused|fill" gpurun_out/launches_fused.csv | head -12

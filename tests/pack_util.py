@@ -2,7 +2,7 @@
 
 `permuted_pack` re-expresses a part in a coordinate frame whose principal axes are not (1, 2) --
 both reference parts have principal axes (1, 2) (bullet_paint_wrapper.py:1294-1300), so the kernels'
-generic-axes instantiations (`move_kernel<..., false>` / `paint_kernel<..., false, ...>`) are otherwise
+generic-axes instantiations (`move_fast_kernel<G, false, ...>` / `paint_kernel<C, ST, false, ...>`) are otherwise
 never reached.  The oracle and the engine both consume the transformed pack, so the comparison stays
 like against like; derived per-triangle constants (d00 ...) are kept as they are.
 """
