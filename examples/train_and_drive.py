@@ -5,7 +5,9 @@
     python examples/train_and_drive.py [checkpoint.pt]
 
 Without an argument it trains for 10 iterations of 4096 environments x 100 steps (about 4 M env-steps, a few seconds
-on a B200) and writes /tmp/paintrl_door_ppo.pt; with one it loads that checkpoint instead.
+on a B200) and writes /tmp/paintrl_door_ppo.pt; with one it loads that checkpoint instead, PPO or DQN
+(`python -m paintrl_b200.train --algo dqn ...`): for a DQN policy the argmax of the head's first n_out columns is the
+greedy Q action, up to the tie rule.
 """
 import os
 import sys

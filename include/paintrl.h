@@ -390,6 +390,45 @@ int paintrl_ppo_forward(PaintrlPpoHandle h, const float *params_dev, const int32
 int paintrl_adam_step(float *params_dev, const float *grad_dev, float *m_dev, float *v_dev, int32_t n_params, float lr,
                       float beta1, float beta2, float eps, int32_t step, void *stream);
 
+/*
+ * Double DQN with a dueling head on the same network (RLlib DQN's dueling combination, without its extra hidden layer
+ * per stream): the n_out head outputs are the advantages A, the value column is V, and Q(s, a) = V + A_a - mean_o A_o.
+ * "Greedy" is the first maximum of Q (the lowest action index on ties), in the act kernel and in the target alike.
+ *
+ * paintrl_policy_act_epsilon: epsilon-greedy actions of a discrete policy engine (PAINTRL_E_INVALID for a continuous
+ * one).  epsilon_dev is one float32 in device memory, read by the kernel on every launch, so a CUDA graph captured
+ * around this call follows an exploration schedule written into it between replays.  Per environment and launch the
+ * engine's counter ctr gives the draws pol_uniform(seed, env, ctr, k) of paintrl_policy.cuh: k = 0 explores when it is
+ * < epsilon, k = 1 then picks the action min(floor(u * n_out), n_out - 1); the counter advances by one either way.
+ * value_dev float32 [batch]; logits_dev float32 [batch, n_out + 1] or NULL, the same bits as paintrl_policy_act's.
+ */
+int paintrl_policy_act_epsilon(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, void *actions_dev, float *value_dev,
+                               float *logits_dev, const float *epsilon_dev, void *stream);
+
+typedef struct PaintrlDqnConfig {
+    int32_t abi_version;
+    int32_t obs_dim, n_out;             /* as PaintrlPolicyConfig (discrete actions only) */
+    int32_t max_minibatch;              /* largest n of paintrl_dqn_grad (sizes the partial-gradient and s' workspaces) */
+    float gamma;                        /* discount, in (0, 1] */
+} PaintrlDqnConfig;
+typedef struct PaintrlDqnEngine *PaintrlDqnHandle;
+
+int paintrl_dqn_create(const PaintrlDqnConfig *cfg, int32_t device, PaintrlDqnHandle *out);
+void paintrl_dqn_destroy(PaintrlDqnHandle h);
+/* The double-DQN loss gradient of one minibatch, asynchronous on `stream` (four launches, no synchronisation).  Row k
+ * of the minibatch is row idx_dev[k] of the transition arrays (idx int32 [n]): obs / next_obs float64 [rows][obs_dim],
+ * actions int64 [rows], reward float32 [rows], done uint8 [rows].  y = r + gamma (1 - done) Q_target(s', argmax_o
+ * Q_online(s', o)) with Q_online from params_dev and Q_target from target_params_dev; loss = mean Huber(Q(s, a) - y),
+ * delta 1.  Writes grad_dev float32 [num_params] (overwritten) and stats_dev float32 [4]: mean Huber loss, mean |td|,
+ * mean Q(s, a), mean y.  Bitwise reproducible. */
+int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
+                     const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
+                     const uint8_t *done_dev, float *grad_dev, float *stats_dev, void *stream);
+/* Global-norm clipping of n float32 values in place (torch.nn.utils.clip_grad_norm_'s rule: scaled by
+ * max_norm / (norm + 1e-6) only when the L2 norm exceeds max_norm, untouched otherwise).  norm_out_dev float32 [1]
+ * receives the norm before clipping.  Fixed-order reduction: the same norm on every run. */
+int paintrl_clip_grad_norm(float *grad_dev, int32_t n, float max_norm, float *norm_out_dev, void *stream);
+
 const char *paintrl_last_error(void);
 int32_t paintrl_abi_version(void);
 

@@ -91,6 +91,11 @@ class PaintrlPpoConfig(ctypes.Structure):
                 ('vf_loss_coeff', ctypes.c_float), ('entropy_coeff', ctypes.c_float)]
 
 
+class PaintrlDqnConfig(ctypes.Structure):
+    _fields_ = [('abi_version', ctypes.c_int32), ('obs_dim', ctypes.c_int32), ('n_out', ctypes.c_int32),
+                ('max_minibatch', ctypes.c_int32), ('gamma', ctypes.c_float)]
+
+
 # name -> (restype, argtypes); every symbol include/paintrl.h declares
 _VP = ctypes.c_void_p
 _I32 = ctypes.c_int32
@@ -136,6 +141,11 @@ SIGNATURES = {
     'paintrl_ppo_grad': (ctypes.c_int, [_VP, _VP, _VP, _I32] + [_VP] * 7 + [ctypes.c_float, _VP, _VP, _VP]),
     'paintrl_ppo_forward': (ctypes.c_int, [_VP, _VP, _VP, _I32, _VP, _VP, _VP]),
     'paintrl_adam_step': (ctypes.c_int, [_VP, _VP, _VP, _VP, _I32, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _I32, _VP]),
+    'paintrl_policy_act_epsilon': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP, _VP]),
+    'paintrl_dqn_create': (ctypes.c_int, [ctypes.POINTER(PaintrlDqnConfig), _I32, ctypes.POINTER(_VP)]),
+    'paintrl_dqn_destroy': (None, [_VP]),
+    'paintrl_dqn_grad': (ctypes.c_int, [_VP, _VP, _VP, _VP, _I32] + [_VP] * 8),
+    'paintrl_clip_grad_norm': (ctypes.c_int, [_VP, _I32, ctypes.c_float, _VP, _VP]),
     'paintrl_last_error': (ctypes.c_char_p, []),
     'paintrl_abi_version': (_I32, []),
 }

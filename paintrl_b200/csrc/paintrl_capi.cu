@@ -1227,7 +1227,11 @@ int paintrl_policy_create(const PaintrlPolicyConfig *cfg, int32_t device, Paintr
     if (ok) ok = cudaFuncSetAttribute(policy_act_kernel<8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
                  cudaFuncSetAttribute(policy_act_kernel<8, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
                  cudaFuncSetAttribute(policy_act_kernel<32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<32, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess;
+                 cudaFuncSetAttribute(policy_act_kernel<32, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(policy_act_kernel<8, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(policy_act_kernel<8, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(policy_act_kernel<32, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(policy_act_kernel<32, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess;
     if (!ok) { delete e; cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the policy engine failed (allocation / shared memory opt-in)"); }
     *out = e;
     return PAINTRL_OK;
@@ -1257,6 +1261,29 @@ int paintrl_policy_act(PaintrlPolicyHandle h, const double *obs_dev, int32_t bat
     else if (small_obs) policy_act_kernel<8, 16><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
     else if (small_out) policy_act_kernel<32, 8><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
     else policy_act_kernel<32, 16><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("policy_act_kernel: ") + cudaGetErrorString(err));
+    h->launches++;
+    return PAINTRL_OK;
+}
+
+int paintrl_policy_act_epsilon(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, void *actions_dev, float *value_dev,
+                               float *logits_dev, const float *epsilon_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (!h->pp.discrete) return fail(PAINTRL_E_INVALID, "epsilon-greedy actions need a discrete policy engine");
+    if (!obs_dev || !actions_dev || !value_dev || !epsilon_dev) return fail(PAINTRL_E_INVALID, "null I/O buffer");
+    if (batch <= 0 || batch > h->capacity) return fail(PAINTRL_E_INVALID, "batch exceeds the policy engine's capacity");
+    CUDA_TRY(cudaSetDevice(h->device));
+    PolicyIO io{};
+    io.obs = obs_dev; io.batch = batch;
+    io.act_discrete = reinterpret_cast<long long *>(actions_dev);
+    io.value = value_dev; io.logits = logits_dev; io.sample = 1; io.epsilon = epsilon_dev;
+    const dim3 pgrid((batch + kPolRows - 1) / kPolRows);
+    const bool small_obs = h->pp.obs_dim <= 8, small_out = h->pp.n_out + 1 <= 8;
+    if (small_obs && small_out) policy_act_kernel<8, 8, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
+    else if (small_obs) policy_act_kernel<8, 16, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
+    else if (small_out) policy_act_kernel<32, 8, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
+    else policy_act_kernel<32, 16, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("policy_act_kernel: ") + cudaGetErrorString(err));
     h->launches++;
@@ -1328,11 +1355,16 @@ void paintrl_ppo_destroy(PaintrlPpoHandle h) {
     delete h;
 }
 
-static int ppo_launch(const PpoGradArgs &a, void *stream) {
+static int ppo_launch(const PpoGradArgs &a, void *stream, int loss = kLossPpo) {
     const dim3 grid((a.n + kPolRows - 1) / kPolRows);
     const bool small_obs = a.obs_dim <= 8, small_out = a.n_out + 1 <= 8;
     cudaStream_t s = as_stream(stream);
-    if (small_obs && small_out) ppo_grad_kernel<8, 8><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    if (loss == kLossDqn) {
+        if (small_obs && small_out) ppo_grad_kernel<8, 8, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+        else if (small_obs) ppo_grad_kernel<8, 16, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+        else if (small_out) ppo_grad_kernel<32, 8, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+        else ppo_grad_kernel<32, 16, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    } else if (small_obs && small_out) ppo_grad_kernel<8, 8><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
     else if (small_obs) ppo_grad_kernel<8, 16><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
     else if (small_out) ppo_grad_kernel<32, 8><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
     else ppo_grad_kernel<32, 16><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
@@ -1368,7 +1400,7 @@ int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t 
     if (rc != PAINTRL_OK) return rc;
     const int nparts = (n + kPolRows - 1) / kPolRows;
     ppo_reduce_kernel<<<(h->nparams + 255) / 256, 256, 0, as_stream(stream)>>>(h->partial, nparts, h->nparams, grad_dev, h->partial_stats,
-                                                                                a.inv_n, stats_dev);
+                                                                                a.inv_n, stats_dev, kLrnStats);
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_reduce_kernel: ") + cudaGetErrorString(err));
     return PAINTRL_OK;
@@ -1399,6 +1431,101 @@ int paintrl_adam_step(float *params_dev, const float *grad_dev, float *m_dev, fl
                                                                         beta2, eps, (float)std::sqrt(bc2));
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("adam_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
+}
+
+/* ---- double DQN on the learner kernel's loss template, see paintrl_learn.cuh ---- */
+struct PaintrlDqnEngine {
+    int device = 0;
+    PaintrlDqnConfig cfg{};
+    int nparams = 0, max_ctas = 0;
+    float *partial = nullptr, *partial_stats = nullptr;
+    float *next_online = nullptr, *next_target = nullptr;   // [max_minibatch][n_out + 1]: the head on s'
+    DeviceArena arena;
+};
+
+int paintrl_dqn_create(const PaintrlDqnConfig *cfg, int32_t device, PaintrlDqnHandle *out) {
+    if (!cfg || !out) return fail(PAINTRL_E_INVALID, "null argument");
+    if (cfg->abi_version != PAINTRL_ABI_VERSION) return fail(PAINTRL_E_INVALID, "ABI version mismatch");
+    if (cfg->obs_dim <= 0 || cfg->obs_dim > kPolMaxObs) return fail(PAINTRL_E_INVALID, "the learner kernel takes observations of 1..32 entries");
+    if (cfg->n_out <= 0 || cfg->n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the learner kernel takes 1..15 action outputs");
+    if (cfg->max_minibatch <= 0) return fail(PAINTRL_E_INVALID, "max_minibatch must be positive");
+    if (!(cfg->gamma > 0.f && cfg->gamma <= 1.f)) return fail(PAINTRL_E_INVALID, "gamma must be in (0, 1]");
+    int count = 0;
+    cudaError_t err = cudaGetDeviceCount(&count);
+    if (err != cudaSuccess || count == 0)
+        return fail(PAINTRL_E_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(err));
+    if (device < 0 || device >= count) return fail(PAINTRL_E_INVALID, "device index out of range");
+    CUDA_TRY(cudaSetDevice(device));
+    PaintrlDqnEngine *e = new PaintrlDqnEngine();
+    e->device = device;
+    e->cfg = *cfg;
+    e->nparams = ppo_num_params(cfg->obs_dim, cfg->n_out);
+    e->max_ctas = (cfg->max_minibatch + kPolRows - 1) / kPolRows;
+    const size_t heads = sizeof(float) * (size_t)cfg->max_minibatch * (cfg->n_out + 1);
+    bool ok = e->arena.alloc((void **)&e->partial, sizeof(float) * (size_t)e->max_ctas * e->nparams) == cudaSuccess &&
+              e->arena.alloc((void **)&e->partial_stats, sizeof(float) * (size_t)e->max_ctas * kLrnStatStride) == cudaSuccess &&
+              e->arena.alloc((void **)&e->next_online, heads) == cudaSuccess && e->arena.alloc((void **)&e->next_target, heads) == cudaSuccess;
+    if (ok) ok = cudaFuncSetAttribute(ppo_grad_kernel<8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<8, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<32, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<8, 8, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<8, 16, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<32, 8, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
+                 cudaFuncSetAttribute(ppo_grad_kernel<32, 16, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess;
+    if (!ok) { delete e; cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the DQN learner failed (allocation / shared memory opt-in)"); }
+    *out = e;
+    return PAINTRL_OK;
+}
+
+void paintrl_dqn_destroy(PaintrlDqnHandle h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    cudaDeviceSynchronize();
+    delete h;
+}
+
+int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
+                     const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
+                     const uint8_t *done_dev, float *grad_dev, float *stats_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (!params_dev || !target_params_dev || !idx_dev || !obs_dev || !actions_dev || !reward_dev || !next_obs_dev || !done_dev ||
+        !grad_dev || !stats_dev)
+        return fail(PAINTRL_E_INVALID, "null buffer");
+    if (n <= 0 || n > h->cfg.max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+    CUDA_TRY(cudaSetDevice(h->device));
+    PpoGradArgs a{};
+    a.obs_dim = h->cfg.obs_dim; a.n_out = h->cfg.n_out; a.discrete = 1; a.n = n; a.nparams = h->nparams;
+    a.idx = idx_dev; a.partial = h->partial; a.partial_stats = h->partial_stats;
+    // the head on s' under the online, then the target parameters: the forward-only path of the same kernel
+    a.forward_only = 1; a.obs = next_obs_dev;
+    a.params = params_dev; a.fwd_out = h->next_online;
+    int rc = ppo_launch(a, stream);
+    if (rc != PAINTRL_OK) return rc;
+    a.params = target_params_dev; a.fwd_out = h->next_target;
+    rc = ppo_launch(a, stream);
+    if (rc != PAINTRL_OK) return rc;
+    a.forward_only = 0; a.obs = obs_dev; a.params = params_dev; a.fwd_out = nullptr;
+    a.actions = actions_dev; a.reward = reward_dev; a.done = done_dev; a.next_online = h->next_online; a.next_target = h->next_target;
+    a.gamma = h->cfg.gamma; a.inv_n = 1.f / (float)n;
+    rc = ppo_launch(a, stream, kLossDqn);
+    if (rc != PAINTRL_OK) return rc;
+    const int nparts = (n + kPolRows - 1) / kPolRows;
+    ppo_reduce_kernel<<<(h->nparams + 255) / 256, 256, 0, as_stream(stream)>>>(h->partial, nparts, h->nparams, grad_dev, h->partial_stats,
+                                                                                a.inv_n, stats_dev, kDqnStats);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_reduce_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
+}
+
+int paintrl_clip_grad_norm(float *grad_dev, int32_t n, float max_norm, float *norm_out_dev, void *stream) {
+    if (!grad_dev || !norm_out_dev) return fail(PAINTRL_E_INVALID, "null buffer");
+    if (n <= 0) return fail(PAINTRL_E_INVALID, "n must be positive");
+    if (!(max_norm > 0.f)) return fail(PAINTRL_E_INVALID, "max_norm must be positive");
+    clip_grad_norm_kernel<<<1, kClipThreads, 0, as_stream(stream)>>>(grad_dev, n, max_norm, norm_out_dev);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("clip_grad_norm_kernel: ") + cudaGetErrorString(err));
     return PAINTRL_OK;
 }
 

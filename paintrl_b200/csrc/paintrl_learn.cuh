@@ -23,6 +23,13 @@
 //   output    one partial gradient per CTA (every entry written, no atomics); ppo_reduce_kernel adds the partials in CTA
 //             order, so a training run is reproducible bit for bit
 //
+// The loss stage is a template parameter (LOSS): kLossPpo above, or kLossDqn, double DQN on the head read as a dueling
+// Q-network (dqn_q_values, paintrl_policy.cuh): per sample td = Q(s, a) - y with y = r + gamma (1 - done)
+// Q_target(s', argmax_o Q_online(s', o)), Huber loss (delta 1) averaged over the minibatch, and dout = g ([o == a] -
+// 1 / n_out) for the n_out advantage columns and g for the value column, g = clamp(td, -1, 1) / n.  The head outputs on
+// s' under the online and the target parameters come from two forward-only launches of the PPO instantiation before the
+// gradient launch (paintrl_dqn_grad).  Forward, backward, the cross-sample sums and the partials are the same code.
+//
 // Flat parameter layout (PaintrlPolicyConfig's tensors, row-major): w1 [obs][256] | b1 [256] | w2 [256][128] | b2 [128]
 // | w3 [128][n_out + 1] | b3 [n_out + 1].
 #pragma once
@@ -31,7 +38,9 @@
 namespace paintrl {
 
 constexpr int kLrnStats = 6;                   // policy loss, value loss, KL, entropy, clip fraction, mean ratio
+constexpr int kDqnStats = 4;                   // Huber loss, |td|, Q(s, a), target y
 constexpr int kLrnStatStride = 8;
+constexpr int kLossPpo = 0, kLossDqn = 1;
 
 __host__ __device__ constexpr int ppo_num_params(int obs_dim, int n_out) {
     return obs_dim * kPolH1 + kPolH1 + kPolH1 * kPolH2 + kPolH2 + kPolH2 * (n_out + 1) + (n_out + 1);
@@ -49,6 +58,12 @@ struct PpoGradArgs {
     float *partial;                            // [gridDim.x][nparams]
     float *partial_stats;                      // [gridDim.x][kLrnStatStride]
     float *fwd_out;                            // forward_only: [n][n_out + 1]
+    // kLossDqn: reward float32 [rows], done uint8 [rows]; the head outputs on s' under the online and the target
+    // parameters, [n][n_out + 1] in minibatch order
+    const float *reward;
+    const unsigned char *done;
+    const float *next_online, *next_target;
+    float gamma;
 };
 
 // dynamic shared memory.  R0 (160 KB) is reused by phase:
@@ -94,7 +109,7 @@ __device__ __forceinline__ uint4 lrn_pack8(const float *f) {
 }
 
 // MO / MX: the compile-time caps of policy_act_kernel (observation and output register arrays)
-template <int MO, int MX>
+template <int MO, int MX, int LOSS = kLossPpo>
 __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a) {
     extern __shared__ __align__(1024) unsigned char lrn_smem[];
     __nv_bfloat16 *sA = reinterpret_cast<__nv_bfloat16 *>(lrn_smem);
@@ -232,6 +247,36 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
         if (valid && a.forward_only) {
 #pragma unroll
             for (int o = 0; o < MX; ++o) if (o < nout1) a.fwd_out[(size_t)j * nout1 + o] = out[o];
+        } else if (valid && LOSS == kLossDqn) {
+            const int act = (int)reinterpret_cast<const long long *>(a.actions)[src];
+            float q[MX], nx[MX], qn[MX];
+            dqn_q_values<MX>(out, a.n_out, q);
+#pragma unroll
+            for (int o = 0; o < MX; ++o) nx[o] = o < nout1 ? __ldg(&a.next_online[(size_t)j * nout1 + o]) : 0.f;
+            const int an = dqn_q_values<MX>(nx, a.n_out, qn);
+#pragma unroll
+            for (int o = 0; o < MX; ++o) nx[o] = o < nout1 ? __ldg(&a.next_target[(size_t)j * nout1 + o]) : 0.f;
+            dqn_q_values<MX>(nx, a.n_out, qn);
+            float qsa = 0.f, qnext = 0.f;
+#pragma unroll
+            for (int o = 0; o < MX; ++o) {
+                if (o == act) qsa = q[o];
+                if (o == an) qnext = qn[o];
+            }
+            const float nd = a.done[src] ? 0.f : 1.f;
+            const float y = __ldg(&a.reward[src]) + a.gamma * nd * qnext;
+            const float td = qsa - y, atd = fabsf(td);
+            const float g = fminf(fmaxf(td, -1.f), 1.f) * a.inv_n;
+            const float inv_nout = 1.f / (float)a.n_out;
+#pragma unroll
+            for (int o = 0; o < MX; ++o) {
+                if (o < a.n_out) dout[o] = g * ((o == act ? 1.f : 0.f) - inv_nout);
+                else if (o == a.n_out) dout[o] = g;
+            }
+            st[0] = atd <= 1.f ? 0.5f * td * td : atd - 0.5f;
+            st[1] = atd;
+            st[2] = qsa;
+            st[3] = y;
         } else if (valid) {
             float v = 0.f;
 #pragma unroll
@@ -468,20 +513,46 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 512;" ::"r"(tmem) : "memory");
 }
 
-// grad[p] = sum over CTAs, in CTA order, of the partial gradients; stats[s] = the minibatch means
+// grad[p] = sum over CTAs, in CTA order, of the partial gradients; stats[s] = the minibatch means of the first nstats
 __global__ void ppo_reduce_kernel(const float *partial, int nparts, int nparams, float *grad, const float *partial_stats, float inv_n,
-                                  float *stats) {
+                                  float *stats, int nstats) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;
     if (p < nparams) {
         float s = 0.f;
         for (int c = 0; c < nparts; ++c) s += partial[(size_t)c * nparams + p];
         grad[p] = s;
     }
-    if (blockIdx.x == 0 && threadIdx.x < kLrnStats) {
+    if (blockIdx.x == 0 && (int)threadIdx.x < nstats) {
         float s = 0.f;
         for (int c = 0; c < nparts; ++c) s += partial_stats[c * kLrnStatStride + threadIdx.x];
         stats[threadIdx.x] = s * inv_n;
     }
+}
+
+// Global-norm gradient clipping (torch.nn.utils.clip_grad_norm_'s rule): norm = sqrt(sum g^2), and when norm > max_norm
+// every entry is multiplied by max_norm / (norm + 1e-6).  One CTA: each thread sums a fixed stride of squares, then a
+// shared-memory tree in a fixed order -- no float atomics, the same norm on every run.  Under max_norm nothing is written.
+constexpr int kClipThreads = 1024;
+__global__ void __launch_bounds__(kClipThreads) clip_grad_norm_kernel(float *grad, int n, float max_norm, float *norm_out) {
+    __shared__ float red[kClipThreads];
+    const int tid = threadIdx.x;
+    float s = 0.f;
+    for (int i = tid; i < n; i += kClipThreads) {
+        const float g = grad[i];
+        s += g * g;
+    }
+    red[tid] = s;
+    __syncthreads();
+#pragma unroll 1
+    for (int w = kClipThreads / 2; w > 0; w >>= 1) {
+        if (tid < w) red[tid] += red[tid + w];
+        __syncthreads();
+    }
+    const float norm = sqrtf(red[0]);
+    if (tid == 0) norm_out[0] = norm;
+    if (!(norm > max_norm)) return;
+    const float scale = max_norm / (norm + 1e-6f);
+    for (int i = tid; i < n; i += kClipThreads) grad[i] *= scale;
 }
 
 // Adam with bias correction, torch.optim.Adam's arithmetic: m <- lerp(m, g, 1 - beta1), v <- beta2 v + (1 - beta2) g^2,

@@ -51,6 +51,7 @@ struct PolicyIO {
     float *logp, *value;      // [B]
     float *logits;            // [B][n_out + 1] or nullptr (tests)
     int sample;               // 0: value / logits only (bootstrap), 1: sample actions
+    const float *epsilon;     // [1] exploration probability of the epsilon-greedy instantiations (EPS), device memory
 };
 
 __device__ __forceinline__ unsigned long long pol_mix(unsigned long long x) {
@@ -78,11 +79,41 @@ __device__ __forceinline__ float pol_tanh(float x) {
     return y;
 }
 
+// The head read as a dueling Q-network (RLlib DQN's dueling combination, without its per-stream hidden layers):
+// out[0, n_out) are the advantages A, out[n_out] the state value V, and q[o] = V + (A[o] - mean A) with the mean
+// summed in column order and divided by n_out.  Returns the greedy action: the first maximum over q, i.e. the lowest
+// index on ties.  The epsilon-greedy act kernel and the double-DQN target both use this, so "greedy" is one rule.
+template <int MX>
+__device__ __forceinline__ int dqn_q_values(const float *out, int n_out, float *q) {
+    float sa = 0.f, v = 0.f;
+#pragma unroll
+    for (int o = 0; o < MX; ++o) {
+        if (o < n_out) sa += out[o];
+        else if (o == n_out) v = out[o];
+    }
+    const float ma = sa / (float)n_out;
+    float best = -INFINITY;
+    int arg = 0;
+#pragma unroll
+    for (int o = 0; o < MX; ++o) {
+        q[o] = 0.f;
+        if (o < n_out) {
+            q[o] = v + (out[o] - ma);
+            if (q[o] > best) { best = q[o]; arg = o; }
+        }
+    }
+    return arg;
+}
+
 // dynamic shared memory: A (64 KB) | B (64 KB) | w1 | b1 | b2 | w3 | b3 | barriers
 // MO / MX: compile-time caps of the observation and output loops (register arrays, fully unrolled): 8 / 8 for the
 // reference's spaces (6-18 observations are 8 or 32; 4 logits + value), 32 / 16 in general.  The shared-memory layout
 // does not depend on them.
-template <int MO, int MX>
+// EPS: epsilon-greedy over the dueling Q values instead of sampling the logits (discrete engines; DQN).  Draw k = 0 of
+// the environment's counter decides (explore when pol_uniform(.., 0) < *io.epsilon), draw k = 1 picks the random
+// action min((int)(pol_uniform(.., 1) * n_out), n_out - 1); otherwise the action is dqn_q_values' greedy one.  logp
+// is not written.
+template <int MO, int MX, bool EPS = false>
 __global__ void __launch_bounds__(kPolThreads, 1) policy_act_kernel(PolicyParams pp, PolicyIO io) {
     extern __shared__ __align__(1024) unsigned char pol_smem[];
     __nv_bfloat16 *sA = reinterpret_cast<__nv_bfloat16 *>(pol_smem);
@@ -238,6 +269,14 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_act_kernel(PolicyParams
     if (!io.sample) return;
     const unsigned ctr = pp.counters[env];
     pp.counters[env] = ctr + 1u;
+    if constexpr (EPS) {
+        float q[MX];
+        int act = dqn_q_values<MX>(out, pp.n_out, q);
+        if (pol_uniform(pp.seed, (unsigned)env, ctr, 0u) < __ldg(io.epsilon))
+            act = min((int)(pol_uniform(pp.seed, (unsigned)env, ctr, 1u) * (float)pp.n_out), pp.n_out - 1);
+        io.act_discrete[env] = act;
+        return;
+    }
     if (pp.discrete) {
         // log-softmax + Gumbel-max
         float mx = -INFINITY;

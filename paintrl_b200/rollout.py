@@ -61,6 +61,16 @@ class NativePolicy(object):
         _capi.check(self._lib.paintrl_policy_act(self._h, p(obs), B, p(actions), p(logp), p(value), p(logits), int(bool(sample)),
                                                  ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
 
+    def act_epsilon_into(self, obs, actions, value, epsilon, logits=None):
+        """Epsilon-greedy actions over the head read as a dueling Q-network (`paintrl_policy_act_epsilon`, discrete
+        engines only): `epsilon` is a one-element float32 CUDA tensor the kernel reads on every launch."""
+        if not self.discrete:
+            raise ValueError('epsilon-greedy actions need a discrete policy')
+        B = obs.shape[0]
+        p = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        _capi.check(self._lib.paintrl_policy_act_epsilon(self._h, p(obs), B, p(actions), p(value), p(logits), p(epsilon),
+                                                         ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+
     def set_params(self, params):
         """Pack a flat FP32 parameter vector (w1 | b1 | w2 | b2 | w3 | b3, a contiguous CUDA tensor of this device) into
         this engine's device weights, in place and on the current stream: a captured rollout graph samples with the new
@@ -164,13 +174,17 @@ class RolloutFragment(object):
 class RolloutWorker(object):
     """Collects fragments from a `BatchedPaintEnv` created with `auto_reset=True`."""
 
-    def __init__(self, env, policy, fragment_length=100, use_cuda_graph=False, use_native_policy=True, keep_logits=False):
+    def __init__(self, env, policy, fragment_length=100, use_cuda_graph=False, use_native_policy=True, keep_logits=False,
+                 epsilon=None):
         """`use_cuda_graph`: after one eager fragment, capture the whole T-step loop (policy kernels and the
         two step kernels per step, ~25 launches each) into one CUDA graph and replay it per fragment -- the
         fragment buffers are persistent, so every address in the loop is static.  Small batches are
         launch-bound without it.
         `keep_logits`: the policy kernel also writes its logits | means and value into `fragment.logits`
-        [T, B, n_out + 1] (what `ppo.PPOLearner` needs for the KL term); needs the native policy."""
+        [T, B, n_out + 1] (what `ppo.PPOLearner` needs for the KL term); needs the native policy.
+        `epsilon`: a one-element float32 CUDA tensor; the native policy then acts epsilon-greedily on its head read as a
+        dueling Q-network (`dqn.DQNLearner`), reading epsilon on every step, inside a captured graph too, and
+        `fragment.logp` is not written.  Needs the native policy and discrete actions."""
         if not env.cfg.auto_reset:
             raise ValueError('RolloutWorker needs an environment created with auto_reset=True')
         self.env, self.policy, self.T = env, policy, int(fragment_length)
@@ -179,6 +193,12 @@ class RolloutWorker(object):
         self.keep_logits = bool(keep_logits)
         if self.keep_logits and getattr(policy, 'native', None) is None:
             raise ValueError('keep_logits needs the native policy kernel (obs_dim <= 32, n_out <= 15, hidden layers 256, 128)')
+        self.epsilon = epsilon
+        if epsilon is not None:
+            if getattr(policy, 'native', None) is None or env.cfg.action_mode != 'discrete':
+                raise ValueError('epsilon-greedy collection needs the native policy kernel and discrete actions')
+            if not (torch.is_tensor(epsilon) and epsilon.is_cuda and epsilon.dtype == torch.float32 and epsilon.numel() == 1):
+                raise ValueError('epsilon must be a one-element float32 CUDA tensor')
         self.use_cuda_graph = bool(use_cuda_graph)
         self._graph, self._eager_fragments, self.graph_error = None, 0, None
         shape = () if env.cfg.action_mode == 'discrete' else (env.action_dim,)
@@ -207,7 +227,9 @@ class RolloutWorker(object):
         f.obs[0].copy_(self._carry)
         native = pol.native
         for t in range(self.T):
-            if native is not None:
+            if native is not None and self.epsilon is not None:
+                native.act_epsilon_into(f.obs[t], f.actions[t], f.value[t], self.epsilon, logits=None if f.logits is None else f.logits[t])
+            elif native is not None:
                 # one launch: obs[t] -> actions[t], logp[t], value[t] written in place (no torch kernels in the loop)
                 native.act_into(f.obs[t], f.actions[t], f.logp[t], f.value[t], logits=None if f.logits is None else f.logits[t])
             else:

@@ -1,6 +1,7 @@
-"""Train the rollout policy with PPO on one GPU: collection and learning both on the device.
+"""Train the rollout policy with PPO or double DQN on one GPU: collection and learning both on the device.
 
     python -m paintrl_b200.train --part 0 --envs 4096 --fragment 100 --samples 8000000 --seed 0 --checkpoint door.pt
+    python -m paintrl_b200.train --algo dqn --envs 4096 --samples 2000000 --checkpoint door_dqn.pt
 
 Environment: BASELINE config C2 (RGB, section-4 observation, discrete-4 actions, late termination, anchor start points,
 auto-reset) on the chosen part.  Policy: paint_ppo.py's [256, 128] MLP, sampled by the act kernel inside a captured
@@ -8,7 +9,10 @@ CUDA graph; the learner (`ppo.PPOLearner`) refreshes the kernel's weights in pla
 
 Per iteration one JSON line: env-steps so far, the ended episodes' mean return, mean coverage ratio (episode `reward`
 total x 100 / the part's max points; RGB) and mean length / 235 (the zigzag baseline's steps to full coverage), and the
-collection and learner times (host clock around work that ends in a device synchronisation).
+collection and learner times (host clock around work that ends in a device synchronisation).  With --algo dqn
+(`dqn.DQNLearner`) the act kernel is epsilon-greedy on the head read as a dueling Q-network, epsilon follows the
+schedule of `dqn.epsilon_at` over the --samples budget and is written before every collection, and each line also
+carries epsilon and the learner's DQN statistics.
 """
 import argparse
 import json
@@ -53,21 +57,38 @@ def max_points(env):
 class Trainer(object):
     """One environment batch, one policy, one worker, one learner; `iteration()` collects a fragment and learns on it."""
 
-    def __init__(self, part=0, num_envs=4096, fragment_length=100, seed=0, device='cuda:0', config=None, use_cuda_graph=True):
-        from .ppo import PPOConfig, PPOLearner
+    def __init__(self, part=0, num_envs=4096, fragment_length=100, seed=0, device='cuda:0', config=None, use_cuda_graph=True,
+                 algo='ppo', total_samples=2000000):
         from .rollout import MlpPolicy, RolloutWorker
+        if algo not in ('ppo', 'dqn'):
+            raise ValueError('algo must be ppo or dqn, not %r' % (algo,))
+        self.algo, self.total_samples = algo, int(total_samples)
         self.device = torch.device(device)
         self.env = make_env(part, num_envs, seed, self.device)
         self.policy = MlpPolicy(self.env.obs_dim, 4 if self.env.cfg.action_mode == 'discrete' else self.env.action_dim,
                                 device=self.device, seed=seed, discrete=self.env.cfg.action_mode == 'discrete')
-        self.worker = RolloutWorker(self.env, self.policy, fragment_length=fragment_length, use_cuda_graph=use_cuda_graph, keep_logits=True)
-        self.learner = PPOLearner(self.policy, config if config is not None else PPOConfig(seed=seed))
+        if algo == 'ppo':
+            from .ppo import PPOConfig, PPOLearner
+            self.epsilon = None
+            self.worker = RolloutWorker(self.env, self.policy, fragment_length=fragment_length, use_cuda_graph=use_cuda_graph, keep_logits=True)
+            self.learner = PPOLearner(self.policy, config if config is not None else PPOConfig(seed=seed))
+        else:
+            from .dqn import DQNConfig, DQNLearner
+            self.epsilon = torch.ones(1, dtype=torch.float32, device=self.device)
+            self.worker = RolloutWorker(self.env, self.policy, fragment_length=fragment_length, use_cuda_graph=use_cuda_graph,
+                                        epsilon=self.epsilon)
+            self.learner = DQNLearner(self.policy, config if config is not None else DQNConfig(seed=seed))
         self.lengths = EpisodeLengths(num_envs, self.device)
         self.max_points = max_points(self.env)
         self.env_steps = 0
         self.worker.start((torch.arange(num_envs) % self.env.n_starts).numpy().astype('int32'))
 
     def iteration(self):
+        eps = None
+        if self.algo == 'dqn':
+            from .dqn import epsilon_at
+            eps = epsilon_at(self.learner.cfg, self.env_steps, self.total_samples)
+            self.epsilon.fill_(eps)
         torch.cuda.synchronize(self.device)
         t0 = time.perf_counter()
         frag, st = self.worker.collect()
@@ -76,16 +97,22 @@ class Trainer(object):
         ls = self.learner.update(frag)                            # ends in the read of its statistics
         t2 = time.perf_counter()
         self.env_steps += int(st['env_steps'])
-        eps = st['episodes']
-        return dict(env_steps=self.env_steps, episodes=int(eps),
-                    mean_return=st['sum_return'] / eps if eps else None,
-                    coverage=st['sum_reward'] * 100.0 / self.max_points / eps if eps else None,
-                    length_ratio=ep_len / eps / ZIGZAG_STEPS if eps else None,
-                    collect_s=t1 - t0, learn_s=t2 - t1, learner=ls)
+        n_ep = st['episodes']
+        r = dict(env_steps=self.env_steps, episodes=int(n_ep),
+                 mean_return=st['sum_return'] / n_ep if n_ep else None,
+                 coverage=st['sum_reward'] * 100.0 / self.max_points / n_ep if n_ep else None,
+                 length_ratio=ep_len / n_ep / ZIGZAG_STEPS if n_ep else None,
+                 collect_s=t1 - t0, learn_s=t2 - t1, learner=ls)
+        if eps is not None:
+            r['epsilon'] = eps
+        return r
 
     def save(self, path):
-        torch.save({'learner': self.learner.state_dict(), 'obs_dim': self.policy.obs_dim, 'n_out': self.policy.n_out,
-                    'discrete': self.policy.discrete, 'env_settings': dict(C2_SETTINGS, Part_NO=self.env.cfg.part_no)}, path)
+        ck = {'learner': self.learner.state_dict(), 'obs_dim': self.policy.obs_dim, 'n_out': self.policy.n_out,
+              'discrete': self.policy.discrete, 'env_settings': dict(C2_SETTINGS, Part_NO=self.env.cfg.part_no)}
+        if self.algo != 'ppo':
+            ck['algo'] = self.algo
+        torch.save(ck, path)
 
     def close(self):
         self.learner.close()
@@ -93,12 +120,18 @@ class Trainer(object):
 
 
 def load_policy(path, device):
-    """A trained `rollout.MlpPolicy` from a checkpoint of this script."""
+    """A trained `rollout.MlpPolicy` from a checkpoint of this script (PPO, or DQN when it records algo 'dqn').  For a
+    DQN policy the argmax of the head outputs' first n_out columns is the greedy action: Q differs from them by a
+    per-state constant, so only the tie rule can differ (the first maximum of the advantages vs. of Q)."""
     from .ppo import check_state_dict, unflatten_into
     from .rollout import MlpPolicy
     ck = torch.load(path, map_location='cpu', weights_only=False)
     pol = MlpPolicy(ck['obs_dim'], ck['n_out'], device=device, discrete=ck['discrete'])
-    check_state_dict(ck['learner'], ck['obs_dim'], ck['n_out'], ck['discrete'])
+    if ck.get('algo', 'ppo') == 'dqn':
+        from .dqn import check_state_dict as check_dqn_state_dict
+        check_dqn_state_dict(ck['learner'], ck['obs_dim'], ck['n_out'])
+    else:
+        check_state_dict(ck['learner'], ck['obs_dim'], ck['n_out'], ck['discrete'])
     unflatten_into(pol, ck['learner']['params'].to(device))
     return pol
 
@@ -113,13 +146,21 @@ def main(argv=None):
     ap.add_argument('--seed', type=int, default=0)
     ap.add_argument('--minibatch', type=int, default=None, help='SGD minibatch (multiple of 128)')
     ap.add_argument('--sgd-iters', type=int, default=None)
-    ap.add_argument('--lr', type=float, default=1e-3, help='Adam learning rate (RLlib default 5e-5; 1e-3 learns faster on the door, '
-                    'profiles/ppo_door_b200.json)')
+    ap.add_argument('--lr', type=float, default=None, help='Adam learning rate; PPO: 1e-3 (RLlib default 5e-5; 1e-3 learns faster on '
+                    'the door, profiles/ppo_door_b200.json); DQN: DQNConfig\'s 5e-4')
     ap.add_argument('--checkpoint', default=None, help='write the learner state here at the end')
+    ap.add_argument('--algo', choices=('ppo', 'dqn'), default='ppo', help='learner: PPO (default) or double DQN with a dueling head')
     args = ap.parse_args(argv)
-    from .ppo import PPOConfig
-    kw = {k: v for k, v in (('minibatch_size', args.minibatch), ('num_sgd_iter', args.sgd_iters), ('lr', args.lr)) if v is not None}
-    tr = Trainer(args.part, args.envs, args.fragment, args.seed, config=PPOConfig(seed=args.seed, **kw))
+    if args.algo == 'dqn':
+        from .dqn import DQNConfig
+        kw = {k: v for k, v in (('minibatch_size', args.minibatch), ('lr', args.lr)) if v is not None}
+        tr = Trainer(args.part, args.envs, args.fragment, args.seed, config=DQNConfig(seed=args.seed, **kw), algo='dqn',
+                     total_samples=args.samples)
+    else:
+        from .ppo import PPOConfig
+        lr = args.lr if args.lr is not None else 1e-3
+        kw = {k: v for k, v in (('minibatch_size', args.minibatch), ('num_sgd_iter', args.sgd_iters), ('lr', lr)) if v is not None}
+        tr = Trainer(args.part, args.envs, args.fragment, args.seed, config=PPOConfig(seed=args.seed, **kw))
     iters = args.iters if args.iters is not None else -(-args.samples // (args.envs * args.fragment))
     t0 = time.perf_counter()
     for it in range(iters):
