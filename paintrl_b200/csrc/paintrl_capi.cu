@@ -7,6 +7,7 @@
 #include <cstring>
 #include <numeric>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #include "../../include/paintrl.h"
@@ -87,6 +88,44 @@ struct DeviceArena {
         return n;
     }
 };
+
+// The prologue of every create function: a device must exist, the index must name one, and it becomes current.
+int select_device(int device) {
+    int count = 0;
+    cudaError_t err = cudaGetDeviceCount(&count);
+    if (err != cudaSuccess || count == 0)
+        return fail(PAINTRL_E_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(err));
+    if (device < 0 || device >= count) return fail(PAINTRL_E_INVALID, "device index out of range");
+    CUDA_TRY(cudaSetDevice(device));
+    return PAINTRL_OK;
+}
+
+// The <MO, MX> instantiation of policy_act_kernel and ppo_grad_kernel for (obs_dim, n_out): f(MO, MX) is called with
+// std::integral_constant arguments.  8 / 8 covers the reference's spaces; the other three take the rest up to 32 / 16.
+template <class F>
+void with_caps(int obs_dim, int n_out, F &&f) {
+    using k8 = std::integral_constant<int, 8>;
+    using k16 = std::integral_constant<int, 16>;
+    using k32 = std::integral_constant<int, 32>;
+    const bool small_obs = obs_dim <= 8, small_out = n_out + 1 <= 8;
+    if (small_obs && small_out) f(k8(), k8());
+    else if (small_obs) f(k8(), k16());
+    else if (small_out) f(k32(), k8());
+    else f(k32(), k16());
+}
+
+template <class K>
+bool opt_in_smem(K *kernel, size_t bytes) {
+    return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes) == cudaSuccess;
+}
+
+template <class E>
+void destroy_engine(E *h) {
+    if (!h) return;
+    cudaSetDevice(h->device);
+    cudaDeviceSynchronize();
+    delete h;
+}
 
 }  // namespace
 
@@ -1198,12 +1237,8 @@ int paintrl_policy_create(const PaintrlPolicyConfig *cfg, int32_t device, Paintr
     if (cfg->n_out <= 0 || cfg->n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the policy kernel takes 1..15 action outputs");
     if (cfg->capacity <= 0) return fail(PAINTRL_E_INVALID, "capacity must be positive");
     if (!cfg->w1 || !cfg->b1 || !cfg->w2 || !cfg->b2 || !cfg->w3 || !cfg->b3) return fail(PAINTRL_E_INVALID, "null weight pointer");
-    int count = 0;
-    cudaError_t err = cudaGetDeviceCount(&count);
-    if (err != cudaSuccess || count == 0)
-        return fail(PAINTRL_E_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(err));
-    if (device < 0 || device >= count) return fail(PAINTRL_E_INVALID, "device index out of range");
-    CUDA_TRY(cudaSetDevice(device));
+    int rc = select_device(device);
+    if (rc != PAINTRL_OK) return rc;
     PaintrlPolicyEngine *e = new PaintrlPolicyEngine();
     e->device = device;
     e->capacity = cfg->capacity;
@@ -1215,33 +1250,33 @@ int paintrl_policy_create(const PaintrlPolicyConfig *cfg, int32_t device, Paintr
     // W2 [256 in][128 out] FP32 -> BF16 B operand [n = out][k = in] in the tensor core's canonical K-major layout
     std::vector<__nv_bfloat16> w2p((size_t)kPolH1 * kPolH2);
     for (int n = 0; n < kPolH2; ++n)
-        for (int k = 0; k < kPolH1; ++k) {
-            const size_t byte = (size_t)(k / 8) * (kPolH2 / 8) * 128 + (size_t)(n / 8) * 128 + (size_t)(n % 8) * 16 + (size_t)(k % 8) * 2;
-            w2p[byte / 2] = __float2bfloat16_rn(cfg->w2[(size_t)k * kPolH2 + n]);
-        }
+        for (int k = 0; k < kPolH1; ++k) w2p[pol_w2_byte(k, n) / 2] = __float2bfloat16_rn(cfg->w2[(size_t)k * kPolH2 + n]);
     bool ok = e->arena.upload(w1, &pp.w1) == cudaSuccess && e->arena.upload(b1, &pp.b1) == cudaSuccess &&
               e->arena.upload(w2p, &pp.w2_packed) == cudaSuccess && e->arena.upload(b2, &pp.b2) == cudaSuccess &&
               e->arena.upload(w3, &pp.w3) == cudaSuccess && e->arena.upload(b3, &pp.b3) == cudaSuccess &&
               e->arena.alloc((void **)&pp.counters, sizeof(unsigned) * (size_t)cfg->capacity) == cudaSuccess;
     if (ok) ok = cudaMemset(pp.counters, 0, sizeof(unsigned) * (size_t)cfg->capacity) == cudaSuccess;
-    if (ok) ok = cudaFuncSetAttribute(policy_act_kernel<8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<8, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<32, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<8, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<8, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<32, 8, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(policy_act_kernel<32, 16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kPolSmemBytes) == cudaSuccess;
+    with_caps(pp.obs_dim, pp.n_out, [&](auto mo, auto mx) {
+        ok = ok && opt_in_smem(policy_act_kernel<mo, mx, false>, kPolSmemBytes) && opt_in_smem(policy_act_kernel<mo, mx, true>, kPolSmemBytes);
+    });
     if (!ok) { delete e; cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the policy engine failed (allocation / shared memory opt-in)"); }
     *out = e;
     return PAINTRL_OK;
 }
 
-void paintrl_policy_destroy(PaintrlPolicyHandle h) {
-    if (!h) return;
-    cudaSetDevice(h->device);
-    cudaDeviceSynchronize();
-    delete h;
+void paintrl_policy_destroy(PaintrlPolicyHandle h) { destroy_engine(h); }
+
+static int policy_launch(PaintrlPolicyHandle h, const PolicyIO &io, bool epsilon_greedy, void *stream) {
+    const dim3 pgrid((io.batch + kPolRows - 1) / kPolRows);
+    cudaStream_t s = as_stream(stream);
+    with_caps(h->pp.obs_dim, h->pp.n_out, [&](auto mo, auto mx) {
+        if (epsilon_greedy) policy_act_kernel<mo, mx, true><<<pgrid, kPolThreads, kPolSmemBytes, s>>>(h->pp, io);
+        else policy_act_kernel<mo, mx, false><<<pgrid, kPolThreads, kPolSmemBytes, s>>>(h->pp, io);
+    });
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("policy_act_kernel: ") + cudaGetErrorString(err));
+    h->launches++;
+    return PAINTRL_OK;
 }
 
 int paintrl_policy_act(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, void *actions_dev, float *logp_dev, float *value_dev,
@@ -1255,16 +1290,7 @@ int paintrl_policy_act(PaintrlPolicyHandle h, const double *obs_dev, int32_t bat
     io.act_discrete = h->pp.discrete ? reinterpret_cast<long long *>(actions_dev) : nullptr;
     io.act_continuous = h->pp.discrete ? nullptr : reinterpret_cast<double *>(actions_dev);
     io.logp = logp_dev; io.value = value_dev; io.logits = logits_dev; io.sample = sample ? 1 : 0;
-    const dim3 pgrid((batch + kPolRows - 1) / kPolRows);
-    const bool small_obs = h->pp.obs_dim <= 8, small_out = h->pp.n_out + 1 <= 8;
-    if (small_obs && small_out) policy_act_kernel<8, 8><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    else if (small_obs) policy_act_kernel<8, 16><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    else if (small_out) policy_act_kernel<32, 8><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    else policy_act_kernel<32, 16><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("policy_act_kernel: ") + cudaGetErrorString(err));
-    h->launches++;
-    return PAINTRL_OK;
+    return policy_launch(h, io, false, stream);
 }
 
 int paintrl_policy_act_epsilon(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, void *actions_dev, float *value_dev,
@@ -1278,22 +1304,13 @@ int paintrl_policy_act_epsilon(PaintrlPolicyHandle h, const double *obs_dev, int
     io.obs = obs_dev; io.batch = batch;
     io.act_discrete = reinterpret_cast<long long *>(actions_dev);
     io.value = value_dev; io.logits = logits_dev; io.sample = 1; io.epsilon = epsilon_dev;
-    const dim3 pgrid((batch + kPolRows - 1) / kPolRows);
-    const bool small_obs = h->pp.obs_dim <= 8, small_out = h->pp.n_out + 1 <= 8;
-    if (small_obs && small_out) policy_act_kernel<8, 8, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    else if (small_obs) policy_act_kernel<8, 16, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    else if (small_out) policy_act_kernel<32, 8, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    else policy_act_kernel<32, 16, true><<<pgrid, kPolThreads, kPolSmemBytes, as_stream(stream)>>>(h->pp, io);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("policy_act_kernel: ") + cudaGetErrorString(err));
-    h->launches++;
-    return PAINTRL_OK;
+    return policy_launch(h, io, true, stream);
 }
 
 /* ---- the PPO learner, see paintrl_learn.cuh ---- */
 int32_t paintrl_policy_num_params(int32_t obs_dim, int32_t n_out) {
     if (obs_dim <= 0 || obs_dim > kPolMaxObs || n_out <= 0 || n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the policy kernel takes observations of 1..32 entries and 1..15 action outputs");
-    return ppo_num_params(obs_dim, n_out);
+    return pol_num_params(obs_dim, n_out);
 }
 
 int paintrl_policy_set_params(PaintrlPolicyHandle h, const float *params_dev, void *stream) {
@@ -1301,7 +1318,7 @@ int paintrl_policy_set_params(PaintrlPolicyHandle h, const float *params_dev, vo
     if (!params_dev) return fail(PAINTRL_E_INVALID, "null parameter buffer");
     CUDA_TRY(cudaSetDevice(h->device));
     const PolicyParams &pp = h->pp;
-    const int n = ppo_num_params(pp.obs_dim, pp.n_out);
+    const int n = pol_num_params(pp.obs_dim, pp.n_out);
     policy_pack_kernel<<<(n + 255) / 256, 256, 0, as_stream(stream)>>>(params_dev, pp.obs_dim, pp.n_out, const_cast<float *>(pp.w1),
                                                                         const_cast<float *>(pp.b1), const_cast<__nv_bfloat16 *>(pp.w2_packed),
                                                                         const_cast<float *>(pp.b2), const_cast<float *>(pp.w3), const_cast<float *>(pp.b3));
@@ -1310,75 +1327,92 @@ int paintrl_policy_set_params(PaintrlPolicyHandle h, const float *params_dev, vo
     return PAINTRL_OK;
 }
 
-struct PaintrlPpoEngine {
+// What the PPO and the DQN learner handles share: the network shape, the per-CTA partial gradients and statistics that
+// ppo_reduce_kernel sums, and the arena that owns them.
+struct LearnerEngine {
     int device = 0;
-    PaintrlPpoConfig cfg{};
+    int obs_dim = 0, n_out = 0, max_minibatch = 0;
     int nparams = 0, max_ctas = 0;
     float *partial = nullptr, *partial_stats = nullptr;
     DeviceArena arena;
 };
 
-int paintrl_ppo_create(const PaintrlPpoConfig *cfg, int32_t device, PaintrlPpoHandle *out) {
-    if (!cfg || !out) return fail(PAINTRL_E_INVALID, "null argument");
-    if (cfg->abi_version != PAINTRL_ABI_VERSION) return fail(PAINTRL_E_INVALID, "ABI version mismatch");
-    if (cfg->obs_dim <= 0 || cfg->obs_dim > kPolMaxObs) return fail(PAINTRL_E_INVALID, "the learner kernel takes observations of 1..32 entries");
-    if (cfg->n_out <= 0 || cfg->n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the learner kernel takes 1..15 action outputs");
-    if (cfg->max_minibatch <= 0) return fail(PAINTRL_E_INVALID, "max_minibatch must be positive");
-    if (!(cfg->clip_param > 0.f) || !(cfg->vf_clip_param > 0.f) || !(cfg->vf_loss_coeff >= 0.f) || !(cfg->entropy_coeff >= 0.f))
-        return fail(PAINTRL_E_INVALID, "clip_param and vf_clip_param must be positive, vf_loss_coeff and entropy_coeff non-negative");
-    int count = 0;
-    cudaError_t err = cudaGetDeviceCount(&count);
-    if (err != cudaSuccess || count == 0)
-        return fail(PAINTRL_E_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(err));
-    if (device < 0 || device >= count) return fail(PAINTRL_E_INVALID, "device index out of range");
-    CUDA_TRY(cudaSetDevice(device));
-    PaintrlPpoEngine *e = new PaintrlPpoEngine();
-    e->device = device;
-    e->cfg = *cfg;
-    e->nparams = ppo_num_params(cfg->obs_dim, cfg->n_out);
-    e->max_ctas = (cfg->max_minibatch + kPolRows - 1) / kPolRows;
-    bool ok = e->arena.alloc((void **)&e->partial, sizeof(float) * (size_t)e->max_ctas * e->nparams) == cudaSuccess &&
-              e->arena.alloc((void **)&e->partial_stats, sizeof(float) * (size_t)e->max_ctas * kLrnStatStride) == cudaSuccess;
-    if (ok) ok = cudaFuncSetAttribute(ppo_grad_kernel<8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<8, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<32, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess;
-    if (!ok) { delete e; cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the learner failed (allocation / shared memory opt-in)"); }
-    *out = e;
+struct PaintrlPpoEngine : LearnerEngine {
+    PaintrlPpoConfig cfg{};
+};
+
+static int learner_check(int abi_version, int obs_dim, int n_out, int max_minibatch) {
+    if (abi_version != PAINTRL_ABI_VERSION) return fail(PAINTRL_E_INVALID, "ABI version mismatch");
+    if (obs_dim <= 0 || obs_dim > kPolMaxObs) return fail(PAINTRL_E_INVALID, "the learner kernel takes observations of 1..32 entries");
+    if (n_out <= 0 || n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the learner kernel takes 1..15 action outputs");
+    if (max_minibatch <= 0) return fail(PAINTRL_E_INVALID, "max_minibatch must be positive");
     return PAINTRL_OK;
 }
 
-void paintrl_ppo_destroy(PaintrlPpoHandle h) {
-    if (!h) return;
-    cudaSetDevice(h->device);
-    cudaDeviceSynchronize();
-    delete h;
+// Device, shape, the partial buffers and the shared-memory opt-in of both loss stages for this shape.  The caller
+// deletes e when this fails.
+static int learner_init(LearnerEngine *e, int device, int obs_dim, int n_out, int max_minibatch) {
+    int rc = select_device(device);
+    if (rc != PAINTRL_OK) return rc;
+    e->device = device;
+    e->obs_dim = obs_dim; e->n_out = n_out; e->max_minibatch = max_minibatch;
+    e->nparams = pol_num_params(obs_dim, n_out);
+    e->max_ctas = (max_minibatch + kPolRows - 1) / kPolRows;
+    bool ok = e->arena.alloc((void **)&e->partial, sizeof(float) * (size_t)e->max_ctas * e->nparams) == cudaSuccess &&
+              e->arena.alloc((void **)&e->partial_stats, sizeof(float) * (size_t)e->max_ctas * kLrnStatStride) == cudaSuccess;
+    with_caps(obs_dim, n_out, [&](auto mo, auto mx) {
+        ok = ok && opt_in_smem(ppo_grad_kernel<mo, mx, kLossPpo>, kLrnSmemBytes) && opt_in_smem(ppo_grad_kernel<mo, mx, kLossDqn>, kLrnSmemBytes);
+    });
+    if (!ok) { cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the learner failed (allocation / shared memory opt-in)"); }
+    return PAINTRL_OK;
 }
 
-static int ppo_launch(const PpoGradArgs &a, void *stream, int loss = kLossPpo) {
+// the launch arguments every learner call fills the same way
+static PpoGradArgs learner_args(const LearnerEngine *h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev) {
+    PpoGradArgs a{};
+    a.obs_dim = h->obs_dim; a.n_out = h->n_out; a.n = n; a.nparams = h->nparams;
+    a.params = params_dev; a.idx = idx_dev; a.obs = obs_dev;
+    a.partial = h->partial; a.partial_stats = h->partial_stats;
+    return a;
+}
+
+static int learner_launch(const PpoGradArgs &a, void *stream, int loss = kLossPpo) {
     const dim3 grid((a.n + kPolRows - 1) / kPolRows);
-    const bool small_obs = a.obs_dim <= 8, small_out = a.n_out + 1 <= 8;
     cudaStream_t s = as_stream(stream);
-    if (loss == kLossDqn) {
-        if (small_obs && small_out) ppo_grad_kernel<8, 8, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
-        else if (small_obs) ppo_grad_kernel<8, 16, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
-        else if (small_out) ppo_grad_kernel<32, 8, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
-        else ppo_grad_kernel<32, 16, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
-    } else if (small_obs && small_out) ppo_grad_kernel<8, 8><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
-    else if (small_obs) ppo_grad_kernel<8, 16><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
-    else if (small_out) ppo_grad_kernel<32, 8><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
-    else ppo_grad_kernel<32, 16><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    with_caps(a.obs_dim, a.n_out, [&](auto mo, auto mx) {
+        if (loss == kLossDqn) ppo_grad_kernel<mo, mx, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+        else ppo_grad_kernel<mo, mx, kLossPpo><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+    });
     cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_grad_kernel: ") + cudaGetErrorString(err));
     return PAINTRL_OK;
 }
 
-static void ppo_args(PaintrlPpoHandle h, PpoGradArgs &a, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev) {
-    a = PpoGradArgs{};
-    a.obs_dim = h->cfg.obs_dim; a.n_out = h->cfg.n_out; a.discrete = h->cfg.discrete ? 1 : 0; a.n = n; a.nparams = h->nparams;
-    a.params = params_dev; a.idx = idx_dev; a.obs = obs_dev;
-    a.partial = h->partial; a.partial_stats = h->partial_stats;
+// grad = the CTA-order sum of the partial gradients of a launch over n samples; stats = the means of its first nstats
+static int learner_reduce(const LearnerEngine *h, int32_t n, float inv_n, float *grad_dev, float *stats_dev, int nstats, void *stream) {
+    const int nparts = (n + kPolRows - 1) / kPolRows;
+    ppo_reduce_kernel<<<(h->nparams + 255) / 256, 256, 0, as_stream(stream)>>>(h->partial, nparts, h->nparams, grad_dev, h->partial_stats,
+                                                                                inv_n, stats_dev, nstats);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_reduce_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
 }
+
+int paintrl_ppo_create(const PaintrlPpoConfig *cfg, int32_t device, PaintrlPpoHandle *out) {
+    if (!cfg || !out) return fail(PAINTRL_E_INVALID, "null argument");
+    int rc = learner_check(cfg->abi_version, cfg->obs_dim, cfg->n_out, cfg->max_minibatch);
+    if (rc != PAINTRL_OK) return rc;
+    if (!(cfg->clip_param > 0.f) || !(cfg->vf_clip_param > 0.f) || !(cfg->vf_loss_coeff >= 0.f) || !(cfg->entropy_coeff >= 0.f))
+        return fail(PAINTRL_E_INVALID, "clip_param and vf_clip_param must be positive, vf_loss_coeff and entropy_coeff non-negative");
+    PaintrlPpoEngine *e = new PaintrlPpoEngine();
+    e->cfg = *cfg;
+    rc = learner_init(e, device, cfg->obs_dim, cfg->n_out, cfg->max_minibatch);
+    if (rc != PAINTRL_OK) { delete e; return rc; }
+    *out = e;
+    return PAINTRL_OK;
+}
+
+void paintrl_ppo_destroy(PaintrlPpoHandle h) { destroy_engine(h); }
 
 int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
                      const void *actions_dev, const float *logp_old_dev, const float *value_old_dev, const float *logits_old_dev,
@@ -1387,36 +1421,31 @@ int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t 
     if (!params_dev || !idx_dev || !obs_dev || !actions_dev || !logp_old_dev || !value_old_dev || !logits_old_dev || !adv_dev ||
         !vtarg_dev || !grad_dev || !stats_dev)
         return fail(PAINTRL_E_INVALID, "null buffer");
-    if (n <= 0 || n > h->cfg.max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+    if (n <= 0 || n > h->max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
     if (!(kl_coeff >= 0.f)) return fail(PAINTRL_E_INVALID, "kl_coeff must be non-negative");
     CUDA_TRY(cudaSetDevice(h->device));
-    PpoGradArgs a;
-    ppo_args(h, a, params_dev, idx_dev, n, obs_dev);
+    PpoGradArgs a = learner_args(h, params_dev, idx_dev, n, obs_dev);
+    a.discrete = h->cfg.discrete ? 1 : 0;
     a.actions = actions_dev; a.logp_old = logp_old_dev; a.value_old = value_old_dev; a.logits_old = logits_old_dev;
     a.adv = adv_dev; a.vtarg = vtarg_dev;
     a.clip = h->cfg.clip_param; a.vf_clip = h->cfg.vf_clip_param; a.vf_coeff = h->cfg.vf_loss_coeff; a.ent_coeff = h->cfg.entropy_coeff;
     a.kl_coeff = kl_coeff; a.inv_n = 1.f / (float)n;
-    int rc = ppo_launch(a, stream);
+    int rc = learner_launch(a, stream);
     if (rc != PAINTRL_OK) return rc;
-    const int nparts = (n + kPolRows - 1) / kPolRows;
-    ppo_reduce_kernel<<<(h->nparams + 255) / 256, 256, 0, as_stream(stream)>>>(h->partial, nparts, h->nparams, grad_dev, h->partial_stats,
-                                                                                a.inv_n, stats_dev, kLrnStats);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_reduce_kernel: ") + cudaGetErrorString(err));
-    return PAINTRL_OK;
+    return learner_reduce(h, n, a.inv_n, grad_dev, stats_dev, kLrnStats, stream);
 }
 
 int paintrl_ppo_forward(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
                         float *out_dev, void *stream) {
     if (!h) return fail(PAINTRL_E_INVALID, "null handle");
     if (!params_dev || !idx_dev || !obs_dev || !out_dev) return fail(PAINTRL_E_INVALID, "null buffer");
-    if (n <= 0 || n > h->cfg.max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+    if (n <= 0 || n > h->max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
     CUDA_TRY(cudaSetDevice(h->device));
-    PpoGradArgs a;
-    ppo_args(h, a, params_dev, idx_dev, n, obs_dev);
+    PpoGradArgs a = learner_args(h, params_dev, idx_dev, n, obs_dev);
+    a.discrete = h->cfg.discrete ? 1 : 0;
     a.forward_only = 1;
     a.fwd_out = out_dev;
-    return ppo_launch(a, stream);
+    return learner_launch(a, stream);
 }
 
 int paintrl_adam_step(float *params_dev, const float *grad_dev, float *m_dev, float *v_dev, int32_t n_params, float lr, float beta1,
@@ -1435,56 +1464,31 @@ int paintrl_adam_step(float *params_dev, const float *grad_dev, float *m_dev, fl
 }
 
 /* ---- double DQN on the learner kernel's loss template, see paintrl_learn.cuh ---- */
-struct PaintrlDqnEngine {
-    int device = 0;
+struct PaintrlDqnEngine : LearnerEngine {
     PaintrlDqnConfig cfg{};
-    int nparams = 0, max_ctas = 0;
-    float *partial = nullptr, *partial_stats = nullptr;
     float *next_online = nullptr, *next_target = nullptr;   // [max_minibatch][n_out + 1]: the head on s'
-    DeviceArena arena;
 };
 
 int paintrl_dqn_create(const PaintrlDqnConfig *cfg, int32_t device, PaintrlDqnHandle *out) {
     if (!cfg || !out) return fail(PAINTRL_E_INVALID, "null argument");
-    if (cfg->abi_version != PAINTRL_ABI_VERSION) return fail(PAINTRL_E_INVALID, "ABI version mismatch");
-    if (cfg->obs_dim <= 0 || cfg->obs_dim > kPolMaxObs) return fail(PAINTRL_E_INVALID, "the learner kernel takes observations of 1..32 entries");
-    if (cfg->n_out <= 0 || cfg->n_out + 1 > kPolMaxOut) return fail(PAINTRL_E_INVALID, "the learner kernel takes 1..15 action outputs");
-    if (cfg->max_minibatch <= 0) return fail(PAINTRL_E_INVALID, "max_minibatch must be positive");
+    int rc = learner_check(cfg->abi_version, cfg->obs_dim, cfg->n_out, cfg->max_minibatch);
+    if (rc != PAINTRL_OK) return rc;
     if (!(cfg->gamma > 0.f && cfg->gamma <= 1.f)) return fail(PAINTRL_E_INVALID, "gamma must be in (0, 1]");
-    int count = 0;
-    cudaError_t err = cudaGetDeviceCount(&count);
-    if (err != cudaSuccess || count == 0)
-        return fail(PAINTRL_E_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(err));
-    if (device < 0 || device >= count) return fail(PAINTRL_E_INVALID, "device index out of range");
-    CUDA_TRY(cudaSetDevice(device));
     PaintrlDqnEngine *e = new PaintrlDqnEngine();
-    e->device = device;
     e->cfg = *cfg;
-    e->nparams = ppo_num_params(cfg->obs_dim, cfg->n_out);
-    e->max_ctas = (cfg->max_minibatch + kPolRows - 1) / kPolRows;
+    rc = learner_init(e, device, cfg->obs_dim, cfg->n_out, cfg->max_minibatch);
     const size_t heads = sizeof(float) * (size_t)cfg->max_minibatch * (cfg->n_out + 1);
-    bool ok = e->arena.alloc((void **)&e->partial, sizeof(float) * (size_t)e->max_ctas * e->nparams) == cudaSuccess &&
-              e->arena.alloc((void **)&e->partial_stats, sizeof(float) * (size_t)e->max_ctas * kLrnStatStride) == cudaSuccess &&
-              e->arena.alloc((void **)&e->next_online, heads) == cudaSuccess && e->arena.alloc((void **)&e->next_target, heads) == cudaSuccess;
-    if (ok) ok = cudaFuncSetAttribute(ppo_grad_kernel<8, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<8, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<32, 8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<32, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<8, 8, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<8, 16, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<32, 8, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess &&
-                 cudaFuncSetAttribute(ppo_grad_kernel<32, 16, kLossDqn>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kLrnSmemBytes) == cudaSuccess;
-    if (!ok) { delete e; cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the DQN learner failed (allocation / shared memory opt-in)"); }
+    if (rc == PAINTRL_OK &&
+        (e->arena.alloc((void **)&e->next_online, heads) != cudaSuccess || e->arena.alloc((void **)&e->next_target, heads) != cudaSuccess)) {
+        cudaGetLastError();
+        rc = fail(PAINTRL_E_CUDA, "setting up the DQN learner failed (allocation)");
+    }
+    if (rc != PAINTRL_OK) { delete e; return rc; }
     *out = e;
     return PAINTRL_OK;
 }
 
-void paintrl_dqn_destroy(PaintrlDqnHandle h) {
-    if (!h) return;
-    cudaSetDevice(h->device);
-    cudaDeviceSynchronize();
-    delete h;
-}
+void paintrl_dqn_destroy(PaintrlDqnHandle h) { destroy_engine(h); }
 
 int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
                      const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
@@ -1493,30 +1497,23 @@ int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *t
     if (!params_dev || !target_params_dev || !idx_dev || !obs_dev || !actions_dev || !reward_dev || !next_obs_dev || !done_dev ||
         !grad_dev || !stats_dev)
         return fail(PAINTRL_E_INVALID, "null buffer");
-    if (n <= 0 || n > h->cfg.max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+    if (n <= 0 || n > h->max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
     CUDA_TRY(cudaSetDevice(h->device));
-    PpoGradArgs a{};
-    a.obs_dim = h->cfg.obs_dim; a.n_out = h->cfg.n_out; a.discrete = 1; a.n = n; a.nparams = h->nparams;
-    a.idx = idx_dev; a.partial = h->partial; a.partial_stats = h->partial_stats;
     // the head on s' under the online, then the target parameters: the forward-only path of the same kernel
-    a.forward_only = 1; a.obs = next_obs_dev;
-    a.params = params_dev; a.fwd_out = h->next_online;
-    int rc = ppo_launch(a, stream);
+    PpoGradArgs a = learner_args(h, params_dev, idx_dev, n, next_obs_dev);
+    a.discrete = 1;
+    a.forward_only = 1; a.fwd_out = h->next_online;
+    int rc = learner_launch(a, stream);
     if (rc != PAINTRL_OK) return rc;
     a.params = target_params_dev; a.fwd_out = h->next_target;
-    rc = ppo_launch(a, stream);
+    rc = learner_launch(a, stream);
     if (rc != PAINTRL_OK) return rc;
     a.forward_only = 0; a.obs = obs_dev; a.params = params_dev; a.fwd_out = nullptr;
     a.actions = actions_dev; a.reward = reward_dev; a.done = done_dev; a.next_online = h->next_online; a.next_target = h->next_target;
     a.gamma = h->cfg.gamma; a.inv_n = 1.f / (float)n;
-    rc = ppo_launch(a, stream, kLossDqn);
+    rc = learner_launch(a, stream, kLossDqn);
     if (rc != PAINTRL_OK) return rc;
-    const int nparts = (n + kPolRows - 1) / kPolRows;
-    ppo_reduce_kernel<<<(h->nparams + 255) / 256, 256, 0, as_stream(stream)>>>(h->partial, nparts, h->nparams, grad_dev, h->partial_stats,
-                                                                                a.inv_n, stats_dev, kDqnStats);
-    cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("ppo_reduce_kernel: ") + cudaGetErrorString(err));
-    return PAINTRL_OK;
+    return learner_reduce(h, n, a.inv_n, grad_dev, stats_dev, kDqnStats, stream);
 }
 
 int paintrl_clip_grad_norm(float *grad_dev, int32_t n, float max_norm, float *norm_out_dev, void *stream) {
@@ -1625,18 +1622,14 @@ int paintrl_create(const PaintrlPartPack *pack, const PaintrlConfig *cfg, int32_
     if (cfg->color_mode == PAINTRL_COLOR_RGB && (pack->status_init > 255 || pack->status_init < 0))
         return fail(PAINTRL_E_INVALID, "status_init out of uint8 range");
 
-    int count = 0;
-    cudaError_t err = cudaGetDeviceCount(&count);
-    if (err != cudaSuccess || count == 0)
-        return fail(PAINTRL_E_CUDA, std::string("no CUDA device (there is no CPU fallback): ") + cudaGetErrorString(err));
-    if (device < 0 || device >= count) return fail(PAINTRL_E_INVALID, "device index out of range");
-    CUDA_TRY(cudaSetDevice(device));
+    int rc = select_device(device);
+    if (rc != PAINTRL_OK) return rc;
 
     PaintrlEngine *e = new PaintrlEngine();
     e->device = device;
     e->num_envs = num_envs;
     e->color = cfg->color_mode == PAINTRL_COLOR_RGB ? 0 : 1;
-    int rc = build_tables(e, pack, cfg);
+    rc = build_tables(e, pack, cfg);
     if (rc != PAINTRL_OK) { delete e; return rc; }
 
     DevConfig &c = e->cfg;
@@ -1696,7 +1689,7 @@ int paintrl_create(const PaintrlPartPack *pack, const PaintrlConfig *cfg, int32_
               e->arena.alloc((void **)&e->slot_out[1], (sizeof(double) * (2 * od + 3) + 1) * (size_t)num_envs) == cudaSuccess &&
               e->arena.alloc((void **)&e->stage_out, (sizeof(double) * (2 * od + 3) + 1) * (size_t)num_envs) == cudaSuccess;
     if (!ok) { delete e; return fail(PAINTRL_E_CUDA, "device allocation failed (state / status planes)"); }
-    err = cudaMemset(e->states, 0, sizeof(EnvState) * (size_t)num_envs);
+    cudaError_t err = cudaMemset(e->states, 0, sizeof(EnvState) * (size_t)num_envs);
     if (err == cudaSuccess) err = cudaMemset(e->moves, 0xff, sizeof(MoveOut) * (size_t)num_envs);   // miss_cache = none
     if (err == cudaSuccess) err = cudaMemset(e->env_stats, 0, sizeof(EnvStat) * (size_t)num_envs);
     if (err == cudaSuccess) err = cudaMemset(e->bits, 0, bits_bytes);

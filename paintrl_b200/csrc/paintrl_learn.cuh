@@ -6,10 +6,10 @@
 // (four threads per sample, each owning a quarter of the sample's hidden features).  Samples are rows of a flattened
 // T x B fragment read through an index list, so the learner shuffles without copying.
 //
-//   forward   exactly policy_act_kernel's arithmetic: layer 1 FP32 FFMA + tanh.approx -> BF16 h1 (canonical K-major,
-//             the act kernel's layout), layer 2 on tcgen05.mma (BF16 x BF16 -> FP32, the same sixteen K steps) into TMEM
-//             columns [0, 128), head in FP32 with the same four partial sums added in the same order -- so logits and
-//             value equal paintrl_policy_act's bit for bit
+//   forward   calls policy_act_kernel's forward functions (paintrl_policy.cuh): layer 1 FP32 FFMA + tanh.approx -> BF16
+//             h1 (canonical K-major), layer 2 on tcgen05.mma (BF16 x BF16 -> FP32, sixteen K steps) into TMEM columns
+//             [0, 128), head in FP32 as four partial sums added in the same order -- so logits and value equal
+//             paintrl_policy_act's bit for bit
 //   loss      RLlib PPO (ray 0.x ppo_policy): clipped surrogate + kl_coeff KL(old || new) + vf_loss_coeff clipped
 //             value loss - entropy_coeff H, averaged over the minibatch; its gradient with respect to the head outputs
 //             (dout) is computed per sample in FP32
@@ -30,8 +30,7 @@
 // s' under the online and the target parameters come from two forward-only launches of the PPO instantiation before the
 // gradient launch (paintrl_dqn_grad).  Forward, backward, the cross-sample sums and the partials are the same code.
 //
-// Flat parameter layout (PaintrlPolicyConfig's tensors, row-major): w1 [obs][256] | b1 [256] | w2 [256][128] | b2 [128]
-// | w3 [128][n_out + 1] | b3 [n_out + 1].
+// Parameters arrive flat, in pol_num_params' layout (paintrl_policy.cuh).
 #pragma once
 #include "paintrl_policy.cuh"
 
@@ -41,10 +40,6 @@ constexpr int kLrnStats = 6;                   // policy loss, value loss, KL, e
 constexpr int kDqnStats = 4;                   // Huber loss, |td|, Q(s, a), target y
 constexpr int kLrnStatStride = 8;
 constexpr int kLossPpo = 0, kLossDqn = 1;
-
-__host__ __device__ constexpr int ppo_num_params(int obs_dim, int n_out) {
-    return obs_dim * kPolH1 + kPolH1 + kPolH1 * kPolH2 + kPolH2 + kPolH2 * (n_out + 1) + (n_out + 1);
-}
 
 struct PpoGradArgs {
     int obs_dim, n_out, discrete, n, nparams;
@@ -75,44 +70,11 @@ constexpr size_t kLrnSmemBytes = (size_t)kLrnR0 +
                                  sizeof(float) * (kPolMaxObs * kPolH1 + kPolH1 + kPolH2 + kPolH2 * kPolMaxOut + kPolMaxOut +
                                                   kPolRows * kPolMaxOut + kPolRows * kLrnStatStride) + 64;
 
-__device__ __forceinline__ void lrn_wait(unsigned long long *bar, unsigned parity) {
-    const unsigned b = (unsigned)__cvta_generic_to_shared(bar);
-    asm volatile("{\n.reg .pred p;\nWAITL_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra DONEL_%=;\nbra WAITL_%=;\nDONEL_%=:\n}" ::"r"(b),
-                 "r"(parity) : "memory");
-}
-
-__device__ __forceinline__ void lrn_mma(unsigned tmem, unsigned long long da, unsigned long long db, unsigned idesc, unsigned accumulate) {
-    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(tmem), "l"(da), "l"(db),
-                 "r"(idesc), "r"(accumulate)
-                 : "memory");
-}
-
-__device__ __forceinline__ void lrn_ld16(unsigned addr, float *v) {
-    unsigned r[16];
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-                   "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                 : "r"(addr)
-                 : "memory");
-    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-    for (int c = 0; c < 16; ++c) v[c] = __uint_as_float(r[c]);
-}
-
-__device__ __forceinline__ uint4 lrn_pack8(const float *f) {
-    __nv_bfloat162 p0 = __floats2bfloat162_rn(f[0], f[1]), p1 = __floats2bfloat162_rn(f[2], f[3]);
-    __nv_bfloat162 p2 = __floats2bfloat162_rn(f[4], f[5]), p3 = __floats2bfloat162_rn(f[6], f[7]);
-    uint4 v;
-    v.x = *reinterpret_cast<unsigned *>(&p0); v.y = *reinterpret_cast<unsigned *>(&p1);
-    v.z = *reinterpret_cast<unsigned *>(&p2); v.w = *reinterpret_cast<unsigned *>(&p3);
-    return v;
-}
-
 // MO / MX: the compile-time caps of policy_act_kernel (observation and output register arrays)
 template <int MO, int MX, int LOSS = kLossPpo>
 __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a) {
     extern __shared__ __align__(1024) unsigned char lrn_smem[];
-    __nv_bfloat16 *sA = reinterpret_cast<__nv_bfloat16 *>(lrn_smem);
+    unsigned char *sA = lrn_smem;
     unsigned char *sB = lrn_smem + kPolRows * kPolH1 * 2;
     unsigned char *sD = sB + kPolH2 * kPolH1 * 2;
     float *spart = reinterpret_cast<float *>(sD);                     // [kPolSplit - 1][kPolRows][kPolMaxOut]
@@ -120,12 +82,8 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
     float *sDZ2 = sH2 + kPolRows * kLrnPadH2;
     float *sDZ1 = reinterpret_cast<float *>(lrn_smem);                // [128][kLrnPadH1]
     float *sX = reinterpret_cast<float *>(lrn_smem + 147456);         // [128][kPolMaxObs]
-    float *sw1 = reinterpret_cast<float *>(lrn_smem + kLrnR0);
-    float *sb1 = sw1 + kPolMaxObs * kPolH1;
-    float *sb2 = sb1 + kPolH1;
-    float *sw3 = sb2 + kPolH2;
-    float *sb3 = sw3 + kPolH2 * kPolMaxOut;
-    float *sdout = sb3 + kPolMaxOut;                                  // [128][kPolMaxOut] dLoss / d(logits | value)
+    const PolTables st(reinterpret_cast<float *>(lrn_smem + kLrnR0));
+    float *sdout = reinterpret_cast<float *>(st.end());               // [128][kPolMaxOut] dLoss / d(logits | value)
     float *sstat = sdout + kPolRows * kPolMaxOut;                     // [128][kLrnStatStride]
     unsigned long long *bar_mma = reinterpret_cast<unsigned long long *>(sstat + kPolRows * kLrnStatStride);
     unsigned *tmem_slot = reinterpret_cast<unsigned *>(bar_mma + 1);
@@ -155,90 +113,35 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
         float f[8];
 #pragma unroll
         for (int q = 0; q < 8; ++q) f[q] = __ldg(&P[off_w2 + (kg * 8 + q) * kPolH2 + n]);
-        *reinterpret_cast<uint4 *>(sB + kg * (kPolH2 / 8) * 128 + (n >> 3) * 128 + (n & 7) * 16) = lrn_pack8(f);
+        *reinterpret_cast<uint4 *>(sB + pol_w2_byte(kg * 8, n)) = pol_pack8(f);
     }
-    for (int i = tid; i < a.obs_dim * kPolH1; i += kPolThreads) sw1[i] = __ldg(&P[i]);
-    for (int i = tid; i < kPolH1; i += kPolThreads) sb1[i] = __ldg(&P[off_b1 + i]);
-    for (int i = tid; i < kPolH2; i += kPolThreads) sb2[i] = __ldg(&P[off_b2 + i]);
-    for (int i = tid; i < kPolH2 * nout1; i += kPolThreads) sw3[i] = __ldg(&P[off_w3 + i]);
-    if (tid < nout1) sb3[tid] = __ldg(&P[off_b3 + tid]);
+    pol_stage_tables(st, P, P, P, P, P, a.obs_dim, nout1, tid, off_b1, off_b2, off_w3, off_b3);
     float x[MO];
-#pragma unroll
-    for (int i = 0; i < MO; ++i) x[i] = (i < a.obs_dim && valid) ? (float)a.obs[(size_t)src * a.obs_dim + i] : 0.f;
+    pol_load_x<MO>(x, a.obs, src, a.obs_dim, valid);
     __syncthreads();
 
-    // ---- layer 1 (policy_act_kernel's loop)
-    {
-        unsigned char *rowbase = reinterpret_cast<unsigned char *>(sA) + (row >> 3) * 128 + (row & 7) * 16;
-        for (int kj = part * (kPolH1 / 8 / kPolSplit); kj < (part + 1) * (kPolH1 / 8 / kPolSplit); ++kj) {
-            float h[8];
-#pragma unroll
-            for (int c = 0; c < 8; ++c) h[c] = sb1[kj * 8 + c];
-#pragma unroll
-            for (int i = 0; i < MO; ++i) {
-                if (i < a.obs_dim) {
-                    const float xi = x[i];
-                    const float *wr = sw1 + i * kPolH1 + kj * 8;
-#pragma unroll
-                    for (int c = 0; c < 8; ++c) h[c] = fmaf(xi, wr[c], h[c]);
-                }
-            }
-#pragma unroll
-            for (int c = 0; c < 8; ++c) h[c] = pol_tanh(h[c]);
-            *reinterpret_cast<uint4 *>(rowbase + kj * (kPolRows / 8) * 128) = lrn_pack8(h);
-        }
-    }
+    pol_layer1<MO>(sA, st, x, a.obs_dim, row, part);
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const unsigned tmem = *tmem_slot;
-    const unsigned base_idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(kPolRows >> 4) << 24);   // D F32, A / B BF16, M 128
     const unsigned a0 = (unsigned)__cvta_generic_to_shared(sA), b0 = (unsigned)__cvta_generic_to_shared(sB),
                    d0 = (unsigned)__cvta_generic_to_shared(sD);
 
-    // ---- layer 2: z2 [128 x 128] = h1 W2, both operands K-major (policy_act_kernel's sixteen steps)
-    if (tid == 0) {
-        const unsigned idesc = base_idesc | ((unsigned)(kPolH2 >> 3) << 17);
-#pragma unroll 1
-        for (int ks = 0; ks < kPolH1 / 16; ++ks)
-            lrn_mma(tmem, pol_smem_desc(a0 + ks * 2 * (kPolRows / 8) * 128, (kPolRows / 8) * 128, 128),
-                    pol_smem_desc(b0 + ks * 2 * (kPolH2 / 8) * 128, (kPolH2 / 8) * 128, 128), idesc, ks > 0 ? 1u : 0u);
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"((unsigned)__cvta_generic_to_shared(bar_mma)) : "memory");
-    }
-    lrn_wait(bar_mma, 0);
+    if (tid == 0) pol_layer2(tmem, a0, b0, bar_mma);   // z2 [128 x 128] = h1 W2
+    pol_wait(bar_mma, 0);
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
-    // ---- head (policy_act_kernel's epilogue)
     const unsigned lane_base = tmem + ((unsigned)((warp & 3) * 32) << 16);
     float out[MX];
-#pragma unroll
-    for (int o = 0; o < MX; ++o) out[o] = (o < nout1 && part == 0) ? sb3[o] : 0.f;
-#pragma unroll 1
-    for (int c0 = part * (kPolH2 / kPolSplit); c0 < (part + 1) * (kPolH2 / kPolSplit); c0 += 16) {
-        float z[16];
-        lrn_ld16(lane_base + (unsigned)c0, z);
-#pragma unroll
-        for (int c = 0; c < 16; ++c) {
-            const float h2 = pol_tanh(z[c] + sb2[c0 + c]);
-            const float *wr = sw3 + (c0 + c) * nout1;
-#pragma unroll
-            for (int o = 0; o < MX; ++o)
-                if (o < nout1) out[o] = fmaf(h2, wr[o], out[o]);
-        }
-    }
-    if (part > 0) {
-#pragma unroll
-        for (int o = 0; o < MX; ++o) spart[((part - 1) * kPolRows + row) * kPolMaxOut + o] = out[o];
-    }
+    pol_head_partial<MX>(out, lane_base, st, nout1, part);
+    pol_head_store<MX>(spart, out, row, part);
     __syncthreads();
 
     // ---- loss and its gradient with respect to the head outputs (one thread per sample)
     if (part == 0) {
-#pragma unroll
-        for (int q = 0; q < kPolSplit - 1; ++q)
-#pragma unroll
-            for (int o = 0; o < MX; ++o) out[o] += spart[(q * kPolRows + row) * kPolMaxOut + o];
+        pol_head_combine<MX>(out, spart, row);
         float dout[MX], st[kLrnStats];
 #pragma unroll
         for (int o = 0; o < MX; ++o) dout[o] = 0.f;
@@ -380,11 +283,11 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
             for (int h = 0; h < 2; ++h) {
                 const int c0 = part * (kPolH2 / kPolSplit) + h * 16;
                 float z[16];
-                lrn_ld16(lane_base + (unsigned)c0, z);
+                pol_ld16(lane_base + (unsigned)c0, z);
 #pragma unroll
                 for (int c = 0; c < 16; ++c) {
-                    const float h2 = pol_tanh(z[c] + sb2[c0 + c]);
-                    const float *wr = sw3 + (c0 + c) * nout1;
+                    const float h2 = pol_tanh(z[c] + st.b2[c0 + c]);
+                    const float *wr = st.w3 + (c0 + c) * nout1;
                     float dh = 0.f;
 #pragma unroll
                     for (int o = 0; o < MX; ++o)
@@ -392,8 +295,8 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
                     h2v[h * 16 + c] = h2;
                     dz2v[h * 16 + c] = dh * (1.f - h2 * h2);
                 }
-                *reinterpret_cast<uint4 *>(rowbase + (c0 >> 3) * (kPolRows / 8) * 128) = lrn_pack8(&dz2v[h * 16]);
-                *reinterpret_cast<uint4 *>(rowbase + ((c0 >> 3) + 1) * (kPolRows / 8) * 128) = lrn_pack8(&dz2v[h * 16 + 8]);
+                *reinterpret_cast<uint4 *>(rowbase + (c0 >> 3) * (kPolRows / 8) * 128) = pol_pack8(&dz2v[h * 16]);
+                *reinterpret_cast<uint4 *>(rowbase + ((c0 >> 3) + 1) * (kPolRows / 8) * 128) = pol_pack8(&dz2v[h * 16 + 8]);
             }
         }
         asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
@@ -404,21 +307,21 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
             // dh1 [128 x 256] = dz2 W2^T: A = dz2 [sample][feature] K-major; B = the W2 tile read as [k][n], n the
             // reduction: MN-major (8 consecutive k per 16-byte row), MN groups of 8 k every 2 KB (SBO), K groups of 8 n
             // every 128 B (LBO)
-            const unsigned id1 = base_idesc | (1u << 16) | ((unsigned)(kPolH1 >> 3) << 17);
+            const unsigned id1 = kPolIdescBase | (1u << 16) | ((unsigned)(kPolH1 >> 3) << 17);
 #pragma unroll 1
             for (int ks = 0; ks < kPolH2 / 16; ++ks)
-                lrn_mma(tmem, pol_smem_desc(d0 + ks * 2 * (kPolRows / 8) * 128, (kPolRows / 8) * 128, 128),
+                pol_mma(tmem, pol_smem_desc(d0 + ks * 2 * (kPolRows / 8) * 128, (kPolRows / 8) * 128, 128),
                         pol_smem_desc(b0 + ks * 2 * 128, 128, (kPolH2 / 8) * 128), id1, ks > 0 ? 1u : 0u);
             // dW2^T [128 n x 256 k] = dz2^T h1, the reduction over samples: both tiles MN-major (8 consecutive features
             // per 16-byte row), feature groups every 2 KB (SBO), sample groups every 128 B (LBO)
-            const unsigned id2 = base_idesc | (1u << 15) | (1u << 16) | ((unsigned)(kPolH1 >> 3) << 17);
+            const unsigned id2 = kPolIdescBase | (1u << 15) | (1u << 16) | ((unsigned)(kPolH1 >> 3) << 17);
 #pragma unroll 1
             for (int ks = 0; ks < kPolRows / 16; ++ks)
-                lrn_mma(tmem + 256, pol_smem_desc(d0 + ks * 2 * 128, 128, (kPolRows / 8) * 128),
+                pol_mma(tmem + 256, pol_smem_desc(d0 + ks * 2 * 128, 128, (kPolRows / 8) * 128),
                         pol_smem_desc(a0 + ks * 2 * 128, 128, (kPolRows / 8) * 128), id2, ks > 0 ? 1u : 0u);
-            asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"((unsigned)__cvta_generic_to_shared(bar_mma)) : "memory");
+            pol_commit(bar_mma);
         }
-        lrn_wait(bar_mma, 1);
+        pol_wait(bar_mma, 1);
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
         // ---- dW3, db2, db3 and the statistics: h2 / dz2 through shared memory, summed in sample order
@@ -457,7 +360,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
 #pragma unroll 1
             for (int k0 = part * (kPolH1 / kPolSplit); k0 < (part + 1) * (kPolH1 / kPolSplit); k0 += 16) {
                 float g[16];
-                lrn_ld16(lane_base + 256u + (unsigned)k0, g);
+                pol_ld16(lane_base + 256u + (unsigned)k0, g);
 #pragma unroll
                 for (int c = 0; c < 16; ++c) pg[off_w2 + (k0 + c) * kPolH2 + n] = g[c];
             }
@@ -467,8 +370,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
         asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
         // ---- layer 1 backward: dz1 = dh1 * (1 - h1^2), h1 recomputed in FP32 with the forward's arithmetic
-#pragma unroll
-        for (int i = 0; i < MO; ++i) x[i] = (i < a.obs_dim && valid) ? (float)a.obs[(size_t)src * a.obs_dim + i] : 0.f;
+        pol_load_x<MO>(x, a.obs, src, a.obs_dim, valid);
         if (part == 0) {
 #pragma unroll
             for (int i = 0; i < MO; ++i) sX[row * kPolMaxObs + i] = x[i];
@@ -476,13 +378,13 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
 #pragma unroll 1
         for (int k0 = part * (kPolH1 / kPolSplit); k0 < (part + 1) * (kPolH1 / kPolSplit); k0 += 16) {
             float g[16];
-            lrn_ld16(lane_base + (unsigned)k0, g);
+            pol_ld16(lane_base + (unsigned)k0, g);
 #pragma unroll
             for (int c = 0; c < 16; ++c) {
-                float h = sb1[k0 + c];
+                float h = st.b1[k0 + c];
 #pragma unroll
                 for (int i = 0; i < MO; ++i)
-                    if (i < a.obs_dim) h = fmaf(x[i], sw1[i * kPolH1 + k0 + c], h);
+                    if (i < a.obs_dim) h = fmaf(x[i], st.w1[i * kPolH1 + k0 + c], h);
                 h = pol_tanh(h);
                 sDZ1[row * kLrnPadH1 + k0 + c] = valid ? g[c] * (1.f - h * h) : 0.f;
             }
@@ -581,9 +483,8 @@ __global__ void policy_pack_kernel(const float *params, int obs_dim, int n_out, 
         if (p < off_b1) w1[p] = f;
         else if (p < off_w2) b1[p - off_b1] = f;
         else if (p < off_b2) {
-            const int e = p - off_w2, k = e / kPolH2, n = e % kPolH2;
-            const size_t byte = (size_t)(k / 8) * (kPolH2 / 8) * 128 + (size_t)(n / 8) * 128 + (size_t)(n % 8) * 16 + (size_t)(k % 8) * 2;
-            w2p[byte / 2] = __float2bfloat16_rn(f);
+            const int e = p - off_w2;
+            w2p[pol_w2_byte(e / kPolH2, e % kPolH2) / 2] = __float2bfloat16_rn(f);
         } else if (p < off_w3) b2[p - off_b2] = f;
         else if (p < off_b3) w3[p - off_w3] = f;
         else b3[p - off_b3] = f;

@@ -73,10 +73,176 @@ __device__ __forceinline__ unsigned long long pol_smem_desc(unsigned smem_byte_a
            ((unsigned long long)(sbo_bytes >> 4) << 32) | (1ull << 46);
 }
 
+// Flat parameter layout (PaintrlPolicyConfig's tensors, row-major), the learner's and policy_pack_kernel's input:
+// w1 [obs][256] | b1 [256] | w2 [256][128] | b2 [128] | w3 [128][n_out + 1] | b3 [n_out + 1]
+__host__ __device__ constexpr int pol_num_params(int obs_dim, int n_out) {
+    return obs_dim * kPolH1 + kPolH1 + kPolH1 * kPolH2 + kPolH2 + kPolH2 * (n_out + 1) + (n_out + 1);
+}
+
+// Byte offset of W2 element (k = input feature, n = output feature) in the canonical K-major B tile [n][k] above.  The
+// host packing (paintrl_policy_create), policy_pack_kernel and the learner's W2 staging all place W2 through this.
+__host__ __device__ constexpr size_t pol_w2_byte(int k, int n) {
+    return (size_t)(k / 8) * (kPolH2 / 8) * 128 + (size_t)(n / 8) * 128 + (size_t)(n % 8) * 16 + (size_t)(k % 8) * 2;
+}
+
 __device__ __forceinline__ float pol_tanh(float x) {
     float y;
     asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
+}
+
+// ---- the forward pass, called step for step by policy_act_kernel and ppo_grad_kernel (paintrl_learn.cuh), so that the
+// learner's head outputs equal the act kernel's bit for bit.  The two kernels lay out shared memory differently; these
+// functions take the shared-memory pointers.
+
+// the FP32 tables in shared memory: w1 [obs_dim][256] | b1 [256] | b2 [128] | w3 [128][n_out + 1] | b3 [n_out + 1]
+struct PolTables {
+    float *w1, *b1, *b2, *w3, *b3;
+    __device__ explicit PolTables(float *base)
+        : w1(base), b1(w1 + kPolMaxObs * kPolH1), b2(b1 + kPolH1), w3(b2 + kPolH2), b3(w3 + kPolH2 * kPolMaxOut) {}
+    __device__ void *end() const { return b3 + kPolMaxOut; }
+};
+
+// Each source table is read at its pointer plus an element offset: the act kernel passes the engine's five arrays, the
+// learner its flat parameter vector five times with the layout's offsets.  obs_dim here and obs / obs_dim in
+// pol_load_x are references to the kernels' launch-parameter fields; passed so, both kernels compile to the code they
+// compiled to when each had its own copy of these loops.
+__device__ __forceinline__ void pol_stage_tables(const PolTables &s, const float *w1, const float *b1, const float *b2, const float *w3,
+                                                 const float *b3, const int &obs_dim, int nout1, int tid, int o_b1 = 0, int o_b2 = 0,
+                                                 int o_w3 = 0, int o_b3 = 0) {
+    for (int i = tid; i < obs_dim * kPolH1; i += kPolThreads) s.w1[i] = __ldg(&w1[i]);
+    for (int i = tid; i < kPolH1; i += kPolThreads) s.b1[i] = __ldg(&b1[o_b1 + i]);
+    for (int i = tid; i < kPolH2; i += kPolThreads) s.b2[i] = __ldg(&b2[o_b2 + i]);
+    for (int i = tid; i < kPolH2 * nout1; i += kPolThreads) s.w3[i] = __ldg(&w3[o_w3 + i]);
+    if (tid < nout1) s.b3[tid] = __ldg(&b3[o_b3 + tid]);
+}
+
+// observation row `src` as FP32, zero past obs_dim and for rows past the batch
+template <int MO>
+__device__ __forceinline__ void pol_load_x(float (&x)[MO], const double *const &obs, int src, const int &obs_dim, bool valid) {
+#pragma unroll
+    for (int i = 0; i < MO; ++i) x[i] = (i < obs_dim && valid) ? (float)obs[(size_t)src * obs_dim + i] : 0.f;
+}
+
+__device__ __forceinline__ uint4 pol_pack8(const float *f) {
+    __nv_bfloat162 p0 = __floats2bfloat162_rn(f[0], f[1]), p1 = __floats2bfloat162_rn(f[2], f[3]);
+    __nv_bfloat162 p2 = __floats2bfloat162_rn(f[4], f[5]), p3 = __floats2bfloat162_rn(f[6], f[7]);
+    uint4 v;
+    v.x = *reinterpret_cast<unsigned *>(&p0); v.y = *reinterpret_cast<unsigned *>(&p1);
+    v.z = *reinterpret_cast<unsigned *>(&p2); v.w = *reinterpret_cast<unsigned *>(&p3);
+    return v;
+}
+
+// layer 1: h1 = tanh(x W1 + b1) -> BF16 into the A tile sA (canonical layout); this thread's quarter of the row's features
+template <int MO>
+__device__ __forceinline__ void pol_layer1(unsigned char *sA, const PolTables &s, const float (&x)[MO], int obs_dim, int row, int part) {
+    unsigned char *rowbase = sA + (row >> 3) * 128 + (row & 7) * 16;
+    for (int kj = part * (kPolH1 / 8 / kPolSplit); kj < (part + 1) * (kPolH1 / 8 / kPolSplit); ++kj) {
+        float h[8];
+#pragma unroll
+        for (int c = 0; c < 8; ++c) h[c] = s.b1[kj * 8 + c];
+#pragma unroll
+        for (int i = 0; i < MO; ++i) {
+            if (i < obs_dim) {
+                const float xi = x[i];
+                const float *wr = s.w1 + i * kPolH1 + kj * 8;
+#pragma unroll
+                for (int c = 0; c < 8; ++c) h[c] = fmaf(xi, wr[c], h[c]);
+            }
+        }
+        // tanh inside the conversions: written so, this compiles to the act kernel's earlier instruction sequence
+        __nv_bfloat162 p0 = __floats2bfloat162_rn(pol_tanh(h[0]), pol_tanh(h[1]));
+        __nv_bfloat162 p1 = __floats2bfloat162_rn(pol_tanh(h[2]), pol_tanh(h[3]));
+        __nv_bfloat162 p2 = __floats2bfloat162_rn(pol_tanh(h[4]), pol_tanh(h[5]));
+        __nv_bfloat162 p3 = __floats2bfloat162_rn(pol_tanh(h[6]), pol_tanh(h[7]));
+        uint4 v;
+        v.x = *reinterpret_cast<unsigned *>(&p0); v.y = *reinterpret_cast<unsigned *>(&p1);
+        v.z = *reinterpret_cast<unsigned *>(&p2); v.w = *reinterpret_cast<unsigned *>(&p3);
+        *reinterpret_cast<uint4 *>(rowbase + kj * (kPolRows / 8) * 128) = v;
+    }
+}
+
+__device__ __forceinline__ void pol_wait(unsigned long long *bar, unsigned parity) {
+    const unsigned b = (unsigned)__cvta_generic_to_shared(bar);
+    asm volatile("{\n.reg .pred p;\nWAIT_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n@p bra DONE_%=;\nbra WAIT_%=;\nDONE_%=:\n}" ::"r"(b),
+                 "r"(parity) : "memory");
+}
+
+__device__ __forceinline__ void pol_mma(unsigned tmem, unsigned long long da, unsigned long long db, unsigned idesc, unsigned accumulate) {
+    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(tmem), "l"(da), "l"(db),
+                 "r"(idesc), "r"(accumulate)
+                 : "memory");
+}
+
+__device__ __forceinline__ void pol_commit(unsigned long long *bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"((unsigned)__cvta_generic_to_shared(bar)) : "memory");
+}
+
+// instruction descriptor (cute::UMMA::InstrDescriptor) without N: D FP32, A / B BF16, M = 128
+constexpr unsigned kPolIdescBase = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(kPolRows >> 4) << 24);
+
+// layer 2 on the tensor core, issued by one thread: D[128 x 128] = A[128 x 256] B[128 x 256]^T, both K-major, into TMEM
+// columns [0, 128), then a commit that arrives on bar
+__device__ __forceinline__ void pol_layer2(unsigned tmem, unsigned a0, unsigned b0, unsigned long long *bar) {
+    const unsigned idesc = kPolIdescBase | ((unsigned)(kPolH2 >> 3) << 17);   // N = 128
+#pragma unroll 1
+    for (int ks = 0; ks < kPolH1 / 16; ++ks)
+        // K step of 16 = two core matrices along K; LBO = distance between them, SBO = distance between 8-row groups
+        pol_mma(tmem, pol_smem_desc(a0 + ks * 2 * (kPolRows / 8) * 128, (kPolRows / 8) * 128, 128),
+                pol_smem_desc(b0 + ks * 2 * (kPolH2 / 8) * 128, (kPolH2 / 8) * 128, 128), idesc, ks > 0 ? 1u : 0u);
+    pol_commit(bar);
+}
+
+// 16 consecutive FP32 columns of this warp's 32 TMEM lanes (one per thread)
+__device__ __forceinline__ void pol_ld16(unsigned addr, float *v) {
+    unsigned r[16];
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
+                   "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(addr)
+                 : "memory");
+    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+    for (int c = 0; c < 16; ++c) v[c] = __uint_as_float(r[c]);
+}
+
+// the head over this thread's quarter of its row of D (TMEM lane = row): out = (part 0: b3) + sum over the quarter's
+// columns c, in column order, of tanh(z2[c] + b2[c]) w3[c]
+template <int MX>
+__device__ __forceinline__ void pol_head_partial(float (&out)[MX], unsigned lane_base, const PolTables &s, int nout1, int part) {
+#pragma unroll
+    for (int o = 0; o < MX; ++o) out[o] = (o < nout1 && part == 0) ? s.b3[o] : 0.f;
+#pragma unroll 1
+    for (int c0 = part * (kPolH2 / kPolSplit); c0 < (part + 1) * (kPolH2 / kPolSplit); c0 += 16) {
+        float z[16];
+        pol_ld16(lane_base + (unsigned)c0, z);
+#pragma unroll
+        for (int c = 0; c < 16; ++c) {
+            const float h2 = pol_tanh(z[c] + s.b2[c0 + c]);
+            const float *wr = s.w3 + (c0 + c) * nout1;
+#pragma unroll
+            for (int o = 0; o < MX; ++o)
+                if (o < nout1) out[o] = fmaf(h2, wr[o], out[o]);
+        }
+    }
+}
+
+// partial heads of the row's other three threads -> spart [kPolSplit - 1][kPolRows][kPolMaxOut]; after a barrier the
+// row's first thread adds them in part order
+template <int MX>
+__device__ __forceinline__ void pol_head_store(float *spart, const float (&out)[MX], int row, int part) {
+    if (part > 0) {
+#pragma unroll
+        for (int o = 0; o < MX; ++o) spart[((part - 1) * kPolRows + row) * kPolMaxOut + o] = out[o];
+    }
+}
+
+template <int MX>
+__device__ __forceinline__ void pol_head_combine(float (&out)[MX], const float *spart, int row) {
+#pragma unroll
+    for (int q = 0; q < kPolSplit - 1; ++q)
+#pragma unroll
+        for (int o = 0; o < MX; ++o) out[o] += spart[(q * kPolRows + row) * kPolMaxOut + o];
 }
 
 // The head read as a dueling Q-network (RLlib DQN's dueling combination, without its per-stream hidden layers):
@@ -116,14 +282,10 @@ __device__ __forceinline__ int dqn_q_values(const float *out, int n_out, float *
 template <int MO, int MX, bool EPS = false>
 __global__ void __launch_bounds__(kPolThreads, 1) policy_act_kernel(PolicyParams pp, PolicyIO io) {
     extern __shared__ __align__(1024) unsigned char pol_smem[];
-    __nv_bfloat16 *sA = reinterpret_cast<__nv_bfloat16 *>(pol_smem);
+    unsigned char *sA = pol_smem;
     unsigned char *sB = pol_smem + kPolRows * kPolH1 * 2;
-    float *sw1 = reinterpret_cast<float *>(sB + kPolH2 * kPolH1 * 2);
-    float *sb1 = sw1 + kPolMaxObs * kPolH1;
-    float *sb2 = sb1 + kPolH1;
-    float *sw3 = sb2 + kPolH2;
-    float *sb3 = sw3 + kPolH2 * kPolMaxOut;
-    unsigned long long *bar_w = reinterpret_cast<unsigned long long *>(sb3 + kPolMaxOut);   // W2 landed
+    const PolTables st(reinterpret_cast<float *>(sB + kPolH2 * kPolH1 * 2));
+    unsigned long long *bar_w = reinterpret_cast<unsigned long long *>(st.end());              // W2 landed
     unsigned long long *bar_mma = bar_w + 1;                                                 // accumulator ready
     unsigned *tmem_slot = reinterpret_cast<unsigned *>(bar_mma + 1);
     float *spart = reinterpret_cast<float *>(tmem_slot + 2);          // [kPolSplit - 1][kPolRows][kPolMaxOut] partial heads
@@ -149,43 +311,12 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_act_kernel(PolicyParams
         asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], 128;" ::"r"((unsigned)__cvta_generic_to_shared(tmem_slot)) : "memory");
         asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
     }
-    // small FP32 tables
-    for (int i = tid; i < pp.obs_dim * kPolH1; i += kPolThreads) sw1[i] = __ldg(&pp.w1[i]);
-    for (int i = tid; i < kPolH1; i += kPolThreads) sb1[i] = __ldg(&pp.b1[i]);
-    for (int i = tid; i < kPolH2; i += kPolThreads) sb2[i] = __ldg(&pp.b2[i]);
-    for (int i = tid; i < kPolH2 * nout1; i += kPolThreads) sw3[i] = __ldg(&pp.w3[i]);
-    if (tid < nout1) sb3[tid] = __ldg(&pp.b3[tid]);
+    pol_stage_tables(st, pp.w1, pp.b1, pp.b2, pp.w3, pp.b3, pp.obs_dim, nout1, tid);
     float x[MO];
-#pragma unroll
-    for (int i = 0; i < MO; ++i) x[i] = (i < pp.obs_dim && env < io.batch) ? (float)io.obs[(size_t)env * pp.obs_dim + i] : 0.f;
+    pol_load_x<MO>(x, io.obs, env, pp.obs_dim, env < io.batch);
     __syncthreads();
 
-    // ---- layer 1: h1 = tanh(x W1 + b1) -> BF16, canonical layout; this thread's quarter of the row's features
-    {
-        unsigned char *rowbase = reinterpret_cast<unsigned char *>(sA) + (row >> 3) * 128 + (row & 7) * 16;
-        for (int kj = part * (kPolH1 / 8 / kPolSplit); kj < (part + 1) * (kPolH1 / 8 / kPolSplit); ++kj) {
-            float h[8];
-#pragma unroll
-            for (int c = 0; c < 8; ++c) h[c] = sb1[kj * 8 + c];
-#pragma unroll
-            for (int i = 0; i < MO; ++i) {
-                if (i < pp.obs_dim) {
-                    const float xi = x[i];
-                    const float *wr = sw1 + i * kPolH1 + kj * 8;
-#pragma unroll
-                    for (int c = 0; c < 8; ++c) h[c] = fmaf(xi, wr[c], h[c]);
-                }
-            }
-            __nv_bfloat162 p0 = __floats2bfloat162_rn(pol_tanh(h[0]), pol_tanh(h[1]));
-            __nv_bfloat162 p1 = __floats2bfloat162_rn(pol_tanh(h[2]), pol_tanh(h[3]));
-            __nv_bfloat162 p2 = __floats2bfloat162_rn(pol_tanh(h[4]), pol_tanh(h[5]));
-            __nv_bfloat162 p3 = __floats2bfloat162_rn(pol_tanh(h[6]), pol_tanh(h[7]));
-            uint4 v;
-            v.x = *reinterpret_cast<unsigned *>(&p0); v.y = *reinterpret_cast<unsigned *>(&p1);
-            v.z = *reinterpret_cast<unsigned *>(&p2); v.w = *reinterpret_cast<unsigned *>(&p3);
-            *reinterpret_cast<uint4 *>(rowbase + kj * (kPolRows / 8) * 128) = v;
-        }
-    }
+    pol_layer1<MO>(sA, st, x, pp.obs_dim, row, part);
     // the activations were written through the generic proxy; the tensor core reads through the async proxy
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
@@ -193,69 +324,22 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_act_kernel(PolicyParams
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
     const unsigned tmem = *tmem_slot;
 
-    // ---- layer 2 on the tensor core: D[128 x 128] = A[128 x 256] B[128 x 256]^T, one thread issues
     if (tid == 0) {
-        {   // W2 has landed?
-            const unsigned bw = (unsigned)__cvta_generic_to_shared(bar_w);
-            asm volatile("{\n.reg .pred p;\nWAITW_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n@p bra DONEW_%=;\nbra WAITW_%=;\nDONEW_%=:\n}" ::"r"(bw) : "memory");
-        }
-        // instruction descriptor (cute::UMMA::InstrDescriptor): D FP32, A / B BF16, both K-major, N = 128, M = 128
-        const unsigned idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(kPolH2 >> 3) << 17) | ((unsigned)(kPolRows >> 4) << 24);
-        const unsigned a0 = (unsigned)__cvta_generic_to_shared(sA), b0 = (unsigned)__cvta_generic_to_shared(sB);
-#pragma unroll 1
-        for (int ks = 0; ks < kPolH1 / 16; ++ks) {
-            // K step of 16 = two core matrices along K; LBO = distance between them, SBO = distance between 8-row groups
-            const unsigned long long da = pol_smem_desc(a0 + ks * 2 * (kPolRows / 8) * 128, (kPolRows / 8) * 128, 128);
-            const unsigned long long db = pol_smem_desc(b0 + ks * 2 * (kPolH2 / 8) * 128, (kPolH2 / 8) * 128, 128);
-            const unsigned accumulate = ks > 0 ? 1u : 0u;
-            asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\ntcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n}" ::"r"(tmem), "l"(da), "l"(db),
-                         "r"(idesc), "r"(accumulate)
-                         : "memory");
-        }
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"((unsigned)__cvta_generic_to_shared(bar_mma)) : "memory");
+        pol_wait(bar_w, 0);   // W2 has landed
+        pol_layer2(tmem, (unsigned)__cvta_generic_to_shared(sA), (unsigned)__cvta_generic_to_shared(sB), bar_mma);
     }
-    {   // everyone: accumulator ready
-        const unsigned bm = (unsigned)__cvta_generic_to_shared(bar_mma);
-        asm volatile("{\n.reg .pred p;\nWAITM_%=:\nmbarrier.try_wait.parity.shared::cta.b64 p, [%0], 0;\n@p bra DONEM_%=;\nbra WAITM_%=;\nDONEM_%=:\n}" ::"r"(bm) : "memory");
-    }
+    pol_wait(bar_mma, 0);     // everyone: accumulator ready
     asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
 
-    // ---- epilogue: this thread's quarter of its row of D (TMEM lane = row), + b2, tanh, head
+    // ---- epilogue: this thread's quarter of its row of D, + b2, tanh, head; the row's first thread adds the others'
     float out[MX];
-#pragma unroll
-    for (int o = 0; o < MX; ++o) out[o] = (o < nout1 && part == 0) ? sb3[o] : 0.f;
-    const unsigned lane_base = tmem + ((unsigned)((warp & 3) * 32) << 16);
-#pragma unroll 1
-    for (int c0 = part * (kPolH2 / kPolSplit); c0 < (part + 1) * (kPolH2 / kPolSplit); c0 += 16) {
-        unsigned r[16];
-        asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                     : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]),
-                       "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                     : "r"(lane_base + (unsigned)c0)
-                     : "memory");
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-        for (int c = 0; c < 16; ++c) {
-            const float h2 = pol_tanh(__uint_as_float(r[c]) + sb2[c0 + c]);
-            const float *wr = sw3 + (c0 + c) * nout1;
-#pragma unroll
-            for (int o = 0; o < MX; ++o)
-                if (o < nout1) out[o] = fmaf(h2, wr[o], out[o]);
-        }
-    }
-    // partial heads of the row's other three threads -> the row's first thread
-    if (part > 0) {
-#pragma unroll
-        for (int o = 0; o < MX; ++o) spart[((part - 1) * kPolRows + row) * kPolMaxOut + o] = out[o];
-    }
+    pol_head_partial<MX>(out, tmem + ((unsigned)((warp & 3) * 32) << 16), st, nout1, part);
+    pol_head_store<MX>(spart, out, row, part);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     __syncthreads();
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, 128;" ::"r"(tmem) : "memory");
     if (part > 0 || env >= io.batch) return;
-#pragma unroll
-    for (int q = 0; q < kPolSplit - 1; ++q)
-#pragma unroll
-        for (int o = 0; o < MX; ++o) out[o] += spart[(q * kPolRows + row) * kPolMaxOut + o];
+    pol_head_combine<MX>(out, spart, row);
 
     // ---- outputs
     float v = 0.f;                              // out[n_out], selected without dynamic register indexing

@@ -18,13 +18,13 @@ the new weights on its next replay.  `update()` reads its statistics back once, 
     frag, rollout_stats = worker.collect()
     learn_stats = learner.update(frag)
 """
-import ctypes
 import math
 
 import torch
 
 from . import _capi
-from .ppo import check_policy, flat_params, num_params, unflatten_into
+from .learner import Learner, LearnerConfig, _ptr, flat_params, unflatten_into  # noqa: F401
+from .learner import check_state_dict as _check_state_dict
 
 # RLlib DQN's defaults as recalled (lr 5e-4, Adam eps 1e-8, gamma 0.99, grad-norm clip 40, 1-step double-Q dueling
 # targets, epsilon 1.0 -> 0.02 over the first 10 % of the sample budget); they could not be checked against an RLlib or
@@ -38,33 +38,17 @@ _DEFAULTS = dict(lr=5e-4, adam_beta1=0.9, adam_beta2=0.999, adam_eps=1e-8, gamma
 STAT_NAMES = ('loss', 'abs_td', 'q_mean', 'target_mean')
 
 
-class DQNConfig(object):
+class DQNConfig(LearnerConfig):
     """Hyper-parameters of `DQNLearner` (see _DEFAULTS); minibatch_size must be a positive multiple of 128."""
+    _DEFAULTS = _DEFAULTS
 
-    def __init__(self, **kw):
-        unknown = set(kw) - set(_DEFAULTS)
-        if unknown:
-            raise TypeError('unknown DQNConfig fields: %s' % sorted(unknown))
-        for k, v in _DEFAULTS.items():
-            setattr(self, k, type(v)(kw.get(k, v)))
-        if self.minibatch_size <= 0 or self.minibatch_size % 128:
-            raise ValueError('minibatch_size must be a positive multiple of 128 (one learner CTA per 128 samples)')
+    def _check(self):
         if self.replay_capacity <= 0 or self.learning_starts < 0 or self.target_update_freq <= 0:
             raise ValueError('replay_capacity and target_update_freq must be positive, learning_starts non-negative')
         if not self.train_intensity > 0.0 or not 0.0 < self.gamma <= 1.0 or not self.grad_clip > 0.0:
             raise ValueError('train_intensity and grad_clip must be positive and gamma in (0, 1]')
         if not (0.0 <= self.epsilon_final <= 1.0 and 0.0 <= self.epsilon_initial <= 1.0 and 0.0 < self.epsilon_fraction <= 1.0):
             raise ValueError('epsilon_initial and epsilon_final must be in [0, 1] and epsilon_fraction in (0, 1]')
-
-    def to_dict(self):
-        return {k: getattr(self, k) for k in _DEFAULTS}
-
-    @classmethod
-    def from_dict(cls, d):
-        return cls(**d)
-
-    def __repr__(self):
-        return 'DQNConfig(%s)' % ', '.join('%s=%r' % kv for kv in self.to_dict().items())
 
 
 def epsilon_at(cfg, env_steps, total_samples):
@@ -121,56 +105,21 @@ class ReplayBuffer(object):
         return torch.randint(0, self.size, (n,), generator=generator, device=self.device, dtype=torch.int32)
 
 
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr())
-
-
-class DQNLearner(object):
+class DQNLearner(Learner):
     """Double DQN over fragments of a `RolloutWorker`, training `policy` (a discrete `rollout.MlpPolicy`) in place: its
     torch tensors and, when enabled, its native act kernel's weights follow every update.  The target network is a
     second flat parameter vector, copied from the online one every target_update_freq gradient steps."""
+    _CREATE, _DESTROY = 'paintrl_dqn_create', 'paintrl_dqn_destroy'
 
     def __init__(self, policy, config=None):
-        check_policy(policy)
         if not policy.discrete:
             raise ValueError('DQN takes discrete action spaces only')
-        self.cfg = config if config is not None else DQNConfig()
-        self.policy = policy
-        self.device = torch.device(policy.device)
-        if self.device.type != 'cuda':
-            raise ValueError('the learner runs on a CUDA device (no CPU fallback)')
-        self.obs_dim, self.n_out = policy.obs_dim, policy.n_out
-        self._lib = _capi.lib()
-        self.n_params = num_params(self.obs_dim, self.n_out)
-        self.params = flat_params(policy).to(self.device)
+        super().__init__(policy, config if config is not None else DQNConfig())
         self.target = self.params.clone()
-        self.m = torch.zeros_like(self.params)
-        self.v = torch.zeros_like(self.params)
-        self.grad = torch.zeros_like(self.params)
-        self.step = 0                              # gradient steps so far (Adam's step count)
-        self.gen = torch.Generator(device=self.device)
-        self.gen.manual_seed(self.cfg.seed)
-        c = self.cfg
-        dc = _capi.PaintrlDqnConfig(_capi.PAINTRL_ABI_VERSION, self.obs_dim, self.n_out, c.minibatch_size, c.gamma)
-        handle = ctypes.c_void_p()
-        index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        _capi.check(self._lib.paintrl_dqn_create(ctypes.byref(dc), index, ctypes.byref(handle)))
-        self._h = handle
-        self.replay = ReplayBuffer(c.replay_capacity, self.obs_dim, self.device)
+        self.replay = ReplayBuffer(self.cfg.replay_capacity, self.obs_dim, self.device)
 
-    def close(self):
-        if getattr(self, '_h', None):
-            self._lib.paintrl_dqn_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _stream(self):
-        return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+    def _c_config(self):
+        return _capi.PaintrlDqnConfig(_capi.PAINTRL_ABI_VERSION, self.obs_dim, self.n_out, self.cfg.minibatch_size, self.cfg.gamma)
 
     def grad_into(self, buf, idx, grad, stats, params=None, target=None):
         """One `paintrl_dqn_grad` call on rows `idx` (int32) of `buf` (a `ReplayBuffer` or anything with its five
@@ -182,12 +131,6 @@ class DQNLearner(object):
 
     def clip(self, grad, norm_out):
         _capi.check(self._lib.paintrl_clip_grad_norm(_ptr(grad), grad.numel(), self.cfg.grad_clip, _ptr(norm_out), self._stream()))
-
-    def adam(self, grad):
-        self.step += 1
-        c = self.cfg
-        _capi.check(self._lib.paintrl_adam_step(_ptr(self.params), _ptr(grad), _ptr(self.m), _ptr(self.v), self.n_params, c.lr,
-                                                c.adam_beta1, c.adam_beta2, c.adam_eps, self.step, self._stream()))
 
     def sync_target(self):
         self.target.copy_(self.params)
@@ -233,30 +176,14 @@ class DQNLearner(object):
     def state_dict(self):
         """Parameters, target parameters, Adam moments, the step count and the sampling generator.  The replay buffer
         is not part of it: a resumed run refills it (and waits for learning_starts transitions again)."""
-        return {'algo': 'dqn', 'config': self.cfg.to_dict(), 'obs_dim': self.obs_dim, 'n_out': self.n_out, 'discrete': True,
-                'params': self.params.cpu(), 'target_params': self.target.cpu(), 'adam_m': self.m.cpu(), 'adam_v': self.v.cpu(),
-                'step': int(self.step), 'generator': self.gen.get_state()}
+        return dict(self._state_dict(), algo='dqn', target_params=self.target.cpu())
 
     def load_state_dict(self, sd):
         check_state_dict(sd, self.obs_dim, self.n_out)
-        self.params.copy_(sd['params'])
         self.target.copy_(sd['target_params'])
-        self.m.copy_(sd['adam_m'])
-        self.v.copy_(sd['adam_v'])
-        self.step = int(sd['step'])
-        self.gen.set_state(sd['generator'])
-        unflatten_into(self.policy, self.params)
-        if getattr(self.policy, 'native', None) is not None:
-            self.policy.native.set_params(self.params)
+        self._load_state_dict(sd)
 
 
 def check_state_dict(sd, obs_dim, n_out):
     """Raise ValueError when a DQN learner state does not fit a discrete policy of this shape."""
-    if (sd.get('obs_dim'), sd.get('n_out'), bool(sd.get('discrete'))) != (obs_dim, n_out, True):
-        raise ValueError('checkpoint is for obs_dim %r, n_out %r, discrete %r' % (sd.get('obs_dim'), sd.get('n_out'), sd.get('discrete')))
-    n = num_params(obs_dim, n_out)
-    for k in ('params', 'target_params', 'adam_m', 'adam_v'):
-        if k not in sd or tuple(sd[k].shape) != (n,):
-            raise ValueError('%s has shape %s, expected (%d,)' % (k, tuple(sd[k].shape) if k in sd else None, n))
-    if int(sd['step']) < 0:
-        raise ValueError('step must be non-negative')
+    _check_state_dict(sd, obs_dim, n_out, True, ('params', 'target_params', 'adam_m', 'adam_v'))

@@ -13,11 +13,11 @@ synchronisation.
     frag, rollout_stats = worker.collect()
     learn_stats = learner.update(frag)
 """
-import ctypes
-
 import torch
 
 from . import _capi
+from .learner import Learner, LearnerConfig, _ptr, check_policy, flat_params, num_params, unflatten_into  # noqa: F401
+from .learner import check_state_dict as _check_state_dict
 from .rollout import gae
 
 # RLlib PPO's loss and optimiser defaults; num_sgd_iter is paint_ppo.py's (BASELINE.md section 1: train batch 1500,
@@ -29,58 +29,15 @@ _DEFAULTS = dict(lr=5e-5, clip_param=0.3, vf_clip_param=10.0, vf_loss_coeff=1.0,
 STAT_NAMES = ('policy_loss', 'vf_loss', 'kl', 'entropy', 'clip_fraction', 'mean_ratio')
 
 
-class PPOConfig(object):
+class PPOConfig(LearnerConfig):
     """Hyper-parameters of `PPOLearner`.  Defaults: RLlib PPO (clip 0.3, vf_clip 10, vf_loss_coeff 1, entropy 0,
     kl_coeff 0.2 adapted toward kl_target 0.01, gamma 0.99, lambda 1.0, Adam lr 5e-5) and paint_ppo.py's 16 SGD
     iterations; minibatch_size must be a positive multiple of 128."""
+    _DEFAULTS = _DEFAULTS
 
-    def __init__(self, **kw):
-        unknown = set(kw) - set(_DEFAULTS)
-        if unknown:
-            raise TypeError('unknown PPOConfig fields: %s' % sorted(unknown))
-        for k, v in _DEFAULTS.items():
-            setattr(self, k, type(v)(kw.get(k, v)))
-        if self.minibatch_size <= 0 or self.minibatch_size % 128:
-            raise ValueError('minibatch_size must be a positive multiple of 128 (one learner CTA per 128 samples)')
+    def _check(self):
         if self.num_sgd_iter <= 0:
             raise ValueError('num_sgd_iter must be positive')
-
-    def to_dict(self):
-        return {k: getattr(self, k) for k in _DEFAULTS}
-
-    @classmethod
-    def from_dict(cls, d):
-        return cls(**d)
-
-    def __repr__(self):
-        return 'PPOConfig(%s)' % ', '.join('%s=%r' % kv for kv in self.to_dict().items())
-
-
-def num_params(obs_dim, n_out):
-    """Length of the flat parameter vector w1 | b1 | w2 | b2 | w3 | b3 (hidden layers 256, 128)."""
-    return obs_dim * 256 + 256 + 256 * 128 + 128 + 128 * (n_out + 1) + (n_out + 1)
-
-
-def check_policy(policy):
-    """Raise ValueError for a policy the learner kernel does not take."""
-    if len(policy.layers) != 2 or tuple(policy.layers[0][0].shape) != (policy.obs_dim, 256) or tuple(policy.layers[1][0].shape) != (256, 128):
-        raise ValueError('the learner kernel takes hidden layers (256, 128) only')
-    if not 1 <= policy.obs_dim <= 32:
-        raise ValueError('the learner kernel takes observations of 1..32 entries, not %d' % policy.obs_dim)
-    if not 1 <= policy.n_out <= 15:
-        raise ValueError('the learner kernel takes 1..15 action outputs, not %d' % policy.n_out)
-
-
-def flat_params(policy):
-    return torch.cat([w.reshape(-1).to(torch.float32) for w in policy.weights()]).contiguous()
-
-
-def unflatten_into(policy, params):
-    """Copy a flat parameter vector into the policy's own tensors (asynchronous device copies)."""
-    off = 0
-    for w in policy.weights():
-        w.copy_(params[off:off + w.numel()].view(w.shape))
-        off += w.numel()
 
 
 def minibatches(n_rows, size):
@@ -97,53 +54,19 @@ def adapt_kl(kl_coeff, kl, kl_target):
     return kl_coeff
 
 
-def _ptr(t):
-    return ctypes.c_void_p(t.data_ptr())
-
-
-class PPOLearner(object):
+class PPOLearner(Learner):
     """PPO over fragments of a `RolloutWorker(..., keep_logits=True)`, training `policy` (an `rollout.MlpPolicy`) in
     place: its torch tensors and, when enabled, its native act kernel's weights follow every update."""
+    _CREATE, _DESTROY = 'paintrl_ppo_create', 'paintrl_ppo_destroy'
 
     def __init__(self, policy, config=None):
-        check_policy(policy)
-        self.cfg = config if config is not None else PPOConfig()
-        self.policy = policy
-        self.device = torch.device(policy.device)
-        if self.device.type != 'cuda':
-            raise ValueError('the learner runs on a CUDA device (no CPU fallback)')
-        self.obs_dim, self.n_out, self.discrete = policy.obs_dim, policy.n_out, bool(policy.discrete)
-        self._lib = _capi.lib()
-        self.n_params = num_params(self.obs_dim, self.n_out)
-        self.params = flat_params(policy).to(self.device)
-        self.m = torch.zeros_like(self.params)
-        self.v = torch.zeros_like(self.params)
-        self.grad = torch.zeros_like(self.params)
-        self.step = 0
+        super().__init__(policy, config if config is not None else PPOConfig())
         self.kl_coeff = float(self.cfg.kl_coeff)
-        self.gen = torch.Generator(device=self.device)
-        self.gen.manual_seed(self.cfg.seed)
+
+    def _c_config(self):
         c = self.cfg
-        pc = _capi.PaintrlPpoConfig(_capi.PAINTRL_ABI_VERSION, self.obs_dim, self.n_out, int(self.discrete), c.minibatch_size,
-                                    c.clip_param, c.vf_clip_param, c.vf_loss_coeff, c.entropy_coeff)
-        handle = ctypes.c_void_p()
-        index = self.device.index if self.device.index is not None else torch.cuda.current_device()
-        _capi.check(self._lib.paintrl_ppo_create(ctypes.byref(pc), index, ctypes.byref(handle)))
-        self._h = handle
-
-    def close(self):
-        if getattr(self, '_h', None):
-            self._lib.paintrl_ppo_destroy(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def _stream(self):
-        return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        return _capi.PaintrlPpoConfig(_capi.PAINTRL_ABI_VERSION, self.obs_dim, self.n_out, int(self.discrete), c.minibatch_size,
+                                      c.clip_param, c.vf_clip_param, c.vf_loss_coeff, c.entropy_coeff)
 
     def forward(self, obs, idx):
         """The learner kernel's forward pass on rows `idx` (int32) of `obs` (float64 [rows, obs_dim]): float32
@@ -159,12 +82,6 @@ class PPOLearner(object):
             self._h, _ptr(self.params), _ptr(idx), idx.numel(), _ptr(rows['obs']), _ptr(rows['actions']), _ptr(rows['logp']),
             _ptr(rows['value']), _ptr(rows['logits']), _ptr(rows['adv']), _ptr(rows['vtarg']), float(kl_coeff), _ptr(grad),
             _ptr(stats), self._stream()))
-
-    def adam(self, grad):
-        self.step += 1
-        c = self.cfg
-        _capi.check(self._lib.paintrl_adam_step(_ptr(self.params), _ptr(grad), _ptr(self.m), _ptr(self.v), self.n_params, c.lr,
-                                                c.adam_beta1, c.adam_beta2, c.adam_eps, self.step, self._stream()))
 
     def flatten(self, frag):
         """The fragment as T*B rows (views where the buffers allow) plus standardised advantages and value targets."""
@@ -209,30 +126,16 @@ class PPOLearner(object):
         return out
 
     def state_dict(self):
-        return {'config': self.cfg.to_dict(), 'obs_dim': self.obs_dim, 'n_out': self.n_out, 'discrete': self.discrete,
-                'params': self.params.cpu(), 'adam_m': self.m.cpu(), 'adam_v': self.v.cpu(), 'step': int(self.step),
-                'kl_coeff': float(self.kl_coeff), 'generator': self.gen.get_state()}
+        return dict(self._state_dict(), kl_coeff=float(self.kl_coeff))
 
     def load_state_dict(self, sd):
         check_state_dict(sd, self.obs_dim, self.n_out, self.discrete)
-        self.params.copy_(sd['params'])
-        self.m.copy_(sd['adam_m'])
-        self.v.copy_(sd['adam_v'])
-        self.step = int(sd['step'])
         self.kl_coeff = float(sd['kl_coeff'])
-        self.gen.set_state(sd['generator'])
-        unflatten_into(self.policy, self.params)
-        if getattr(self.policy, 'native', None) is not None:
-            self.policy.native.set_params(self.params)
+        self._load_state_dict(sd)
 
 
 def check_state_dict(sd, obs_dim, n_out, discrete):
     """Raise ValueError when a learner state does not fit a policy of this shape."""
-    if (sd.get('obs_dim'), sd.get('n_out'), bool(sd.get('discrete'))) != (obs_dim, n_out, bool(discrete)):
-        raise ValueError('checkpoint is for obs_dim %r, n_out %r, discrete %r' % (sd.get('obs_dim'), sd.get('n_out'), sd.get('discrete')))
-    n = num_params(obs_dim, n_out)
-    for k in ('params', 'adam_m', 'adam_v'):
-        if tuple(sd[k].shape) != (n,):
-            raise ValueError('%s has shape %s, expected (%d,)' % (k, tuple(sd[k].shape), n))
-    if int(sd['step']) < 0 or not float(sd['kl_coeff']) >= 0.0:
-        raise ValueError('step must be non-negative and kl_coeff non-negative')
+    _check_state_dict(sd, obs_dim, n_out, discrete, ('params', 'adam_m', 'adam_v'))
+    if not float(sd['kl_coeff']) >= 0.0:
+        raise ValueError('kl_coeff must be non-negative')
