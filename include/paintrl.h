@@ -424,6 +424,43 @@ void paintrl_dqn_destroy(PaintrlDqnHandle h);
 int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
                      const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
                      const uint8_t *done_dev, float *grad_dev, float *stats_dev, void *stream);
+/* paintrl_dqn_grad with a per-sample importance weight (prioritized replay): weight_dev float32 [n] and td_out_dev
+ * float32 [n], both in minibatch order.  loss = mean w_k Huber(td_k), its gradient per sample
+ * (clamp(td, -1, 1) * w) / n, so all-ones weights give paintrl_dqn_grad's gradient and statistics bit for bit.  td_out_dev
+ * receives td_k = Q(s, a) - y for the priority update; stats_dev float32 [5]: mean weighted Huber loss, mean |td|,
+ * mean Q(s, a), mean y, mean weight.  Bitwise reproducible. */
+int paintrl_dqn_grad_weighted(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev,
+                              int32_t n, const double *obs_dev, const int64_t *actions_dev, const float *reward_dev,
+                              const double *next_obs_dev, const uint8_t *done_dev, const float *weight_dev, float *td_out_dev,
+                              float *grad_dev, float *stats_dev, void *stream);
+
+/*
+ * Prioritized replay (RLlib's PrioritizedReplayBuffer) over a ring of `capacity` rows: a sum tree and a min tree, both
+ * float64 [2 * tree_leaves] in device memory and owned by the caller.  tree_leaves is a power of two >= capacity; node 1
+ * is the root, node i has children 2i and 2i + 1, and row r is leaf tree_leaves + r.  A filled leaf holds p^alpha in
+ * both trees; the caller initialises every leaf and node to 0 in the sum tree and +inf in the min tree.  After every
+ * leaf write the calls below rebuild each internal node from its two children (sum: left + right, min: fmin), so the
+ * trees are a pure function of their leaves.  max_priority_dev is one float64 in device memory (RLlib starts it at 1).
+ * All three are asynchronous on `stream`.
+ *
+ * paintrl_prio_fill: rows [start, start + count) mod capacity get max_priority^alpha, as new transitions do in RLlib.
+ * paintrl_prio_update: for k < n, row idx_dev[k] (int32, in [0, capacity)) gets (|td_k| + eps)^alpha from the float32
+ *   td_dev [n] (paintrl_dqn_grad_weighted's td_out), computed in float64, and max_priority rises to max(|td_k| + eps).
+ *   Duplicate rows must carry identical td (as one minibatch's do).
+ * paintrl_prio_sample: n rows, row k from the float64 uniform u_dev[k] in [0, 1): the leaf where the prefix sum of the
+ *   sum tree passes u * root, never a row of priority 0 (so never one at or beyond size, the filled rows [0, size)).
+ *   idx_out_dev int32 [n]; weight_out_dev float32 [n] = (p_i / p_min)^(-beta) in float64, p_min the min-tree root: RLlib's
+ *   (N P(i))^-beta / max_j (N P(j))^-beta, at most 1.
+ * Requirements: alpha finite and >= 0, eps finite and > 0, beta in [0, 1], size in [1, capacity], count in [1, capacity],
+ * start in [0, capacity), n in [1, 2^24].
+ */
+int paintrl_prio_fill(double *sum_tree_dev, double *min_tree_dev, int32_t tree_leaves, int32_t capacity, int32_t start, int32_t count,
+                      const double *max_priority_dev, double alpha, void *stream);
+int paintrl_prio_update(double *sum_tree_dev, double *min_tree_dev, int32_t tree_leaves, int32_t capacity, const int32_t *idx_dev,
+                        const float *td_dev, int32_t n, double *max_priority_dev, double alpha, double eps, void *stream);
+int paintrl_prio_sample(const double *sum_tree_dev, const double *min_tree_dev, int32_t tree_leaves, int32_t capacity, int32_t size,
+                        const double *u_dev, int32_t n, double beta, int32_t *idx_out_dev, float *weight_out_dev, void *stream);
+
 /* Global-norm clipping of n float32 values in place (torch.nn.utils.clip_grad_norm_'s rule: scaled by
  * max_norm / (norm + 1e-6) only when the L2 norm exceeds max_norm, untouched otherwise).  norm_out_dev float32 [1]
  * receives the norm before clipping.  Fixed-order reduction: the same norm on every run. */

@@ -99,6 +99,7 @@ class PaintrlDqnConfig(ctypes.Structure):
 # name -> (restype, argtypes); every symbol include/paintrl.h declares
 _VP = ctypes.c_void_p
 _I32 = ctypes.c_int32
+_F64 = ctypes.c_double
 SIGNATURES = {
     'paintrl_create': (ctypes.c_int, [ctypes.POINTER(PaintrlPartPack), ctypes.POINTER(PaintrlConfig),
                                       _I32, _I32, ctypes.POINTER(_VP)]),
@@ -145,6 +146,10 @@ SIGNATURES = {
     'paintrl_dqn_create': (ctypes.c_int, [ctypes.POINTER(PaintrlDqnConfig), _I32, ctypes.POINTER(_VP)]),
     'paintrl_dqn_destroy': (None, [_VP]),
     'paintrl_dqn_grad': (ctypes.c_int, [_VP, _VP, _VP, _VP, _I32] + [_VP] * 8),
+    'paintrl_dqn_grad_weighted': (ctypes.c_int, [_VP, _VP, _VP, _VP, _I32] + [_VP] * 10),
+    'paintrl_prio_fill': (ctypes.c_int, [_VP, _VP, _I32, _I32, _I32, _I32, _VP, _F64, _VP]),
+    'paintrl_prio_update': (ctypes.c_int, [_VP, _VP, _I32, _I32, _VP, _VP, _I32, _VP, _F64, _F64, _VP]),
+    'paintrl_prio_sample': (ctypes.c_int, [_VP, _VP, _I32, _I32, _I32, _VP, _I32, _F64, _VP, _VP, _VP]),
     'paintrl_clip_grad_norm': (ctypes.c_int, [_VP, _I32, ctypes.c_float, _VP, _VP]),
     'paintrl_last_error': (ctypes.c_char_p, []),
     'paintrl_abi_version': (_I32, []),

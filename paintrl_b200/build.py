@@ -15,7 +15,7 @@ _DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(_DIR, 'csrc')
 SOURCES = [os.path.join(CSRC, 'paintrl_capi.cu')]
 HEADERS = [os.path.join(CSRC, 'paintrl_device.cuh'), os.path.join(CSRC, 'paintrl_kernels.cuh'), os.path.join(CSRC, 'paintrl_raster.cuh'), os.path.join(CSRC, 'paintrl_param.cuh'), os.path.join(CSRC, 'paintrl_policy.cuh'),
-           os.path.join(CSRC, 'paintrl_learn.cuh'),
+           os.path.join(CSRC, 'paintrl_learn.cuh'), os.path.join(CSRC, 'paintrl_replay.cuh'),
            os.path.join(os.path.dirname(_DIR), 'include', 'paintrl.h')]
 LIB = os.path.join(_DIR, 'libpaintrl_b200.so')
 

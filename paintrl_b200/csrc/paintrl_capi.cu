@@ -16,6 +16,7 @@
 #include "paintrl_param.cuh"
 #include "paintrl_policy.cuh"
 #include "paintrl_learn.cuh"
+#include "paintrl_replay.cuh"
 
 using namespace paintrl;
 
@@ -1349,7 +1350,7 @@ static int learner_check(int abi_version, int obs_dim, int n_out, int max_miniba
     return PAINTRL_OK;
 }
 
-// Device, shape, the partial buffers and the shared-memory opt-in of both loss stages for this shape.  The caller
+// Device, shape, the partial buffers and the shared-memory opt-in of every loss stage for this shape.  The caller
 // deletes e when this fails.
 static int learner_init(LearnerEngine *e, int device, int obs_dim, int n_out, int max_minibatch) {
     int rc = select_device(device);
@@ -1361,7 +1362,8 @@ static int learner_init(LearnerEngine *e, int device, int obs_dim, int n_out, in
     bool ok = e->arena.alloc((void **)&e->partial, sizeof(float) * (size_t)e->max_ctas * e->nparams) == cudaSuccess &&
               e->arena.alloc((void **)&e->partial_stats, sizeof(float) * (size_t)e->max_ctas * kLrnStatStride) == cudaSuccess;
     with_caps(obs_dim, n_out, [&](auto mo, auto mx) {
-        ok = ok && opt_in_smem(ppo_grad_kernel<mo, mx, kLossPpo>, kLrnSmemBytes) && opt_in_smem(ppo_grad_kernel<mo, mx, kLossDqn>, kLrnSmemBytes);
+        ok = ok && opt_in_smem(ppo_grad_kernel<mo, mx, kLossPpo>, kLrnSmemBytes) && opt_in_smem(ppo_grad_kernel<mo, mx, kLossDqn>, kLrnSmemBytes) &&
+             opt_in_smem(ppo_grad_kernel<mo, mx, kLossDqnPer>, kLrnSmemBytes);
     });
     if (!ok) { cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the learner failed (allocation / shared memory opt-in)"); }
     return PAINTRL_OK;
@@ -1381,6 +1383,7 @@ static int learner_launch(const PpoGradArgs &a, void *stream, int loss = kLossPp
     cudaStream_t s = as_stream(stream);
     with_caps(a.obs_dim, a.n_out, [&](auto mo, auto mx) {
         if (loss == kLossDqn) ppo_grad_kernel<mo, mx, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+        else if (loss == kLossDqnPer) ppo_grad_kernel<mo, mx, kLossDqnPer><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
         else ppo_grad_kernel<mo, mx, kLossPpo><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
     });
     cudaError_t err = cudaGetLastError();
@@ -1490,14 +1493,10 @@ int paintrl_dqn_create(const PaintrlDqnConfig *cfg, int32_t device, PaintrlDqnHa
 
 void paintrl_dqn_destroy(PaintrlDqnHandle h) { destroy_engine(h); }
 
-int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
-                     const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
-                     const uint8_t *done_dev, float *grad_dev, float *stats_dev, void *stream) {
-    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
-    if (!params_dev || !target_params_dev || !idx_dev || !obs_dev || !actions_dev || !reward_dev || !next_obs_dev || !done_dev ||
-        !grad_dev || !stats_dev)
-        return fail(PAINTRL_E_INVALID, "null buffer");
-    if (n <= 0 || n > h->max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+// paintrl_dqn_grad and paintrl_dqn_grad_weighted: weight_dev / td_out_dev are null for the unweighted loss
+static int dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
+                    const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
+                    const uint8_t *done_dev, const float *weight_dev, float *td_out_dev, float *grad_dev, float *stats_dev, void *stream) {
     CUDA_TRY(cudaSetDevice(h->device));
     // the head on s' under the online, then the target parameters: the forward-only path of the same kernel
     PpoGradArgs a = learner_args(h, params_dev, idx_dev, n, next_obs_dev);
@@ -1511,9 +1510,112 @@ int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *t
     a.forward_only = 0; a.obs = obs_dev; a.params = params_dev; a.fwd_out = nullptr;
     a.actions = actions_dev; a.reward = reward_dev; a.done = done_dev; a.next_online = h->next_online; a.next_target = h->next_target;
     a.gamma = h->cfg.gamma; a.inv_n = 1.f / (float)n;
-    rc = learner_launch(a, stream, kLossDqn);
+    a.weight = weight_dev; a.td_out = td_out_dev;
+    const bool weighted = weight_dev != nullptr;
+    rc = learner_launch(a, stream, weighted ? kLossDqnPer : kLossDqn);
     if (rc != PAINTRL_OK) return rc;
-    return learner_reduce(h, n, a.inv_n, grad_dev, stats_dev, kDqnStats, stream);
+    return learner_reduce(h, n, a.inv_n, grad_dev, stats_dev, weighted ? kDqnPerStats : kDqnStats, stream);
+}
+
+static int dqn_grad_check(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
+                          const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
+                          const uint8_t *done_dev, float *grad_dev, float *stats_dev) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (!params_dev || !target_params_dev || !idx_dev || !obs_dev || !actions_dev || !reward_dev || !next_obs_dev || !done_dev ||
+        !grad_dev || !stats_dev)
+        return fail(PAINTRL_E_INVALID, "null buffer");
+    if (n <= 0 || n > h->max_minibatch) return fail(PAINTRL_E_INVALID, "n must be in [1, max_minibatch]");
+    return PAINTRL_OK;
+}
+
+int paintrl_dqn_grad(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev, int32_t n,
+                     const double *obs_dev, const int64_t *actions_dev, const float *reward_dev, const double *next_obs_dev,
+                     const uint8_t *done_dev, float *grad_dev, float *stats_dev, void *stream) {
+    const int rc = dqn_grad_check(h, params_dev, target_params_dev, idx_dev, n, obs_dev, actions_dev, reward_dev, next_obs_dev, done_dev,
+                                  grad_dev, stats_dev);
+    if (rc != PAINTRL_OK) return rc;
+    return dqn_grad(h, params_dev, target_params_dev, idx_dev, n, obs_dev, actions_dev, reward_dev, next_obs_dev, done_dev, nullptr,
+                    nullptr, grad_dev, stats_dev, stream);
+}
+
+int paintrl_dqn_grad_weighted(PaintrlDqnHandle h, const float *params_dev, const float *target_params_dev, const int32_t *idx_dev,
+                              int32_t n, const double *obs_dev, const int64_t *actions_dev, const float *reward_dev,
+                              const double *next_obs_dev, const uint8_t *done_dev, const float *weight_dev, float *td_out_dev,
+                              float *grad_dev, float *stats_dev, void *stream) {
+    const int rc = dqn_grad_check(h, params_dev, target_params_dev, idx_dev, n, obs_dev, actions_dev, reward_dev, next_obs_dev, done_dev,
+                                  grad_dev, stats_dev);
+    if (rc != PAINTRL_OK) return rc;
+    if (!weight_dev || !td_out_dev) return fail(PAINTRL_E_INVALID, "null buffer");
+    return dqn_grad(h, params_dev, target_params_dev, idx_dev, n, obs_dev, actions_dev, reward_dev, next_obs_dev, done_dev, weight_dev,
+                    td_out_dev, grad_dev, stats_dev, stream);
+}
+
+/* ---- prioritized replay: the sum / min trees of paintrl_replay.cuh ---- */
+static int prio_check_tree(const double *sum_tree_dev, const double *min_tree_dev, int32_t tree_leaves, int32_t capacity) {
+    if (!sum_tree_dev || !min_tree_dev) return fail(PAINTRL_E_INVALID, "null tree buffer");
+    if (capacity < 1) return fail(PAINTRL_E_INVALID, "capacity must be positive");
+    if (tree_leaves < capacity || (tree_leaves & (tree_leaves - 1)) != 0)
+        return fail(PAINTRL_E_INVALID, "tree_leaves must be a power of two at or above the capacity");
+    return PAINTRL_OK;
+}
+
+// every internal node from its two children: one launch per group of up to log2(kPrioSubtree) levels, bottom up
+static int prio_rebuild(double *sum, double *mn, int L, cudaStream_t s) {
+    for (int base = L; base > 1;) {
+        const int width = std::min(base, kPrioSubtree);
+        prio_build_kernel<<<base / width, kPrioBuildThreads, 0, s>>>(sum, mn, base, width);
+        base /= width;
+    }
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("prio_build_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
+}
+
+int paintrl_prio_fill(double *sum_tree_dev, double *min_tree_dev, int32_t tree_leaves, int32_t capacity, int32_t start, int32_t count,
+                      const double *max_priority_dev, double alpha, void *stream) {
+    int rc = prio_check_tree(sum_tree_dev, min_tree_dev, tree_leaves, capacity);
+    if (rc != PAINTRL_OK) return rc;
+    if (!max_priority_dev) return fail(PAINTRL_E_INVALID, "null buffer");
+    if (start < 0 || start >= capacity) return fail(PAINTRL_E_INVALID, "start must be in [0, capacity)");
+    if (count < 1 || count > capacity) return fail(PAINTRL_E_INVALID, "count must be in [1, capacity]");
+    if (!(alpha >= 0.0 && std::isfinite(alpha))) return fail(PAINTRL_E_INVALID, "alpha must be finite and non-negative");
+    cudaStream_t s = as_stream(stream);
+    prio_fill_kernel<<<(count + kPrioThreads - 1) / kPrioThreads, kPrioThreads, 0, s>>>(sum_tree_dev, min_tree_dev, tree_leaves, capacity,
+                                                                                          start, count, max_priority_dev, alpha);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("prio_fill_kernel: ") + cudaGetErrorString(err));
+    return prio_rebuild(sum_tree_dev, min_tree_dev, tree_leaves, s);
+}
+
+int paintrl_prio_update(double *sum_tree_dev, double *min_tree_dev, int32_t tree_leaves, int32_t capacity, const int32_t *idx_dev,
+                        const float *td_dev, int32_t n, double *max_priority_dev, double alpha, double eps, void *stream) {
+    int rc = prio_check_tree(sum_tree_dev, min_tree_dev, tree_leaves, capacity);
+    if (rc != PAINTRL_OK) return rc;
+    if (!idx_dev || !td_dev || !max_priority_dev) return fail(PAINTRL_E_INVALID, "null buffer");
+    if (n < 1 || n > kPrioMaxBatch) return fail(PAINTRL_E_INVALID, "n must be in [1, 2^24]");
+    if (!(alpha >= 0.0 && std::isfinite(alpha))) return fail(PAINTRL_E_INVALID, "alpha must be finite and non-negative");
+    if (!(eps > 0.0 && std::isfinite(eps))) return fail(PAINTRL_E_INVALID, "eps must be finite and positive");
+    cudaStream_t s = as_stream(stream);
+    prio_update_kernel<<<(n + kPrioThreads - 1) / kPrioThreads, kPrioThreads, 0, s>>>(sum_tree_dev, min_tree_dev, tree_leaves, idx_dev,
+                                                                                        td_dev, n, max_priority_dev, alpha, eps);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("prio_update_kernel: ") + cudaGetErrorString(err));
+    return prio_rebuild(sum_tree_dev, min_tree_dev, tree_leaves, s);
+}
+
+int paintrl_prio_sample(const double *sum_tree_dev, const double *min_tree_dev, int32_t tree_leaves, int32_t capacity, int32_t size,
+                        const double *u_dev, int32_t n, double beta, int32_t *idx_out_dev, float *weight_out_dev, void *stream) {
+    int rc = prio_check_tree(sum_tree_dev, min_tree_dev, tree_leaves, capacity);
+    if (rc != PAINTRL_OK) return rc;
+    if (!u_dev || !idx_out_dev || !weight_out_dev) return fail(PAINTRL_E_INVALID, "null buffer");
+    if (size < 1 || size > capacity) return fail(PAINTRL_E_INVALID, "size must be in [1, capacity]");
+    if (n < 1 || n > kPrioMaxBatch) return fail(PAINTRL_E_INVALID, "n must be in [1, 2^24]");
+    if (!(beta >= 0.0 && beta <= 1.0)) return fail(PAINTRL_E_INVALID, "beta must be in [0, 1]");
+    prio_sample_kernel<<<(n + kPrioThreads - 1) / kPrioThreads, kPrioThreads, 0, as_stream(stream)>>>(
+        sum_tree_dev, min_tree_dev, tree_leaves, u_dev, n, beta, idx_out_dev, weight_out_dev);
+    cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return fail(PAINTRL_E_CUDA, std::string("prio_sample_kernel: ") + cudaGetErrorString(err));
+    return PAINTRL_OK;
 }
 
 int paintrl_clip_grad_norm(float *grad_dev, int32_t n, float max_norm, float *norm_out_dev, void *stream) {

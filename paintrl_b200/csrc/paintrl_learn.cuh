@@ -29,6 +29,9 @@
 // 1 / n_out) for the n_out advantage columns and g for the value column, g = clamp(td, -1, 1) / n.  The head outputs on
 // s' under the online and the target parameters come from two forward-only launches of the PPO instantiation before the
 // gradient launch (paintrl_dqn_grad).  Forward, backward, the cross-sample sums and the partials are the same code.
+// kLossDqnPer is kLossDqn with a per-sample importance weight w (prioritized replay, paintrl_replay.cuh): g =
+// (clamp(td, -1, 1) * w) * inv_n, so w = 1 gives kLossDqn's bits; the Huber statistic is weighted the same way, a fifth
+// statistic is w, and td goes to td_out in minibatch order for the priority update.
 //
 // Parameters arrive flat, in pol_num_params' layout (paintrl_policy.cuh).
 #pragma once
@@ -38,8 +41,9 @@ namespace paintrl {
 
 constexpr int kLrnStats = 6;                   // policy loss, value loss, KL, entropy, clip fraction, mean ratio
 constexpr int kDqnStats = 4;                   // Huber loss, |td|, Q(s, a), target y
+constexpr int kDqnPerStats = 5;                // weighted Huber loss, |td|, Q(s, a), target y, importance weight
 constexpr int kLrnStatStride = 8;
-constexpr int kLossPpo = 0, kLossDqn = 1;
+constexpr int kLossPpo = 0, kLossDqn = 1, kLossDqnPer = 2;
 
 struct PpoGradArgs {
     int obs_dim, n_out, discrete, n, nparams;
@@ -59,6 +63,9 @@ struct PpoGradArgs {
     const unsigned char *done;
     const float *next_online, *next_target;
     float gamma;
+    // kLossDqnPer: importance weights float32 [n] in, TD errors float32 [n] out, both in minibatch order
+    const float *weight;
+    float *td_out;
 };
 
 // dynamic shared memory.  R0 (160 KB) is reused by phase:
@@ -150,7 +157,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
         if (valid && a.forward_only) {
 #pragma unroll
             for (int o = 0; o < MX; ++o) if (o < nout1) a.fwd_out[(size_t)j * nout1 + o] = out[o];
-        } else if (valid && LOSS == kLossDqn) {
+        } else if (valid && LOSS != kLossPpo) {
             const int act = (int)reinterpret_cast<const long long *>(a.actions)[src];
             float q[MX], nx[MX], qn[MX];
             dqn_q_values<MX>(out, a.n_out, q);
@@ -169,7 +176,14 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
             const float nd = a.done[src] ? 0.f : 1.f;
             const float y = __ldg(&a.reward[src]) + a.gamma * nd * qnext;
             const float td = qsa - y, atd = fabsf(td);
-            const float g = fminf(fmaxf(td, -1.f), 1.f) * a.inv_n;
+            float c = fminf(fmaxf(td, -1.f), 1.f);
+            float w = 1.f;
+            if (LOSS == kLossDqnPer) {
+                w = __ldg(&a.weight[j]);
+                c = c * w;
+                a.td_out[j] = td;
+            }
+            const float g = c * a.inv_n;
             const float inv_nout = 1.f / (float)a.n_out;
 #pragma unroll
             for (int o = 0; o < MX; ++o) {
@@ -180,6 +194,10 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
             st[1] = atd;
             st[2] = qsa;
             st[3] = y;
+            if (LOSS == kLossDqnPer) {
+                st[0] = st[0] * w;
+                st[4] = w;
+            }
         } else if (valid) {
             float v = 0.f;
 #pragma unroll

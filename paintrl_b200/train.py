@@ -2,6 +2,7 @@
 
     python -m paintrl_b200.train --part 0 --envs 4096 --fragment 100 --samples 8000000 --seed 0 --checkpoint door.pt
     python -m paintrl_b200.train --algo dqn --envs 4096 --samples 2000000 --checkpoint door_dqn.pt
+    python -m paintrl_b200.train --algo dqn --prioritized-replay --n-step 3 --samples 2000000 --checkpoint door_apex.pt
 
 Environment: BASELINE config C2 (RGB, section-4 observation, discrete-4 actions, late termination, anchor start points,
 auto-reset) on the chosen part.  Policy: paint_ppo.py's [256, 128] MLP, sampled by the act kernel inside a captured
@@ -12,7 +13,9 @@ total x 100 / the part's max points; RGB) and mean length / 235 (the zigzag base
 collection and learner times (host clock around work that ends in a device synchronisation).  With --algo dqn
 (`dqn.DQNLearner`) the act kernel is epsilon-greedy on the head read as a dueling Q-network, epsilon follows the
 schedule of `dqn.epsilon_at` over the --samples budget and is written before every collection, and each line also
-carries epsilon and the learner's DQN statistics.
+carries epsilon and the learner's DQN statistics.  --prioritized-replay and --n-step turn on `dqn.DQNConfig`'s
+prioritized replay and n-step returns (Ape-X DQN's replay side); the statistics then include the mean importance
+weight, weight_mean.
 """
 import argparse
 import json
@@ -150,10 +153,16 @@ def main(argv=None):
                     'the door, profiles/ppo_door_b200.json); DQN: DQNConfig\'s 5e-4')
     ap.add_argument('--checkpoint', default=None, help='write the learner state here at the end')
     ap.add_argument('--algo', choices=('ppo', 'dqn'), default='ppo', help='learner: PPO (default) or double DQN with a dueling head')
+    ap.add_argument('--prioritized-replay', action='store_true', help='DQN: proportional prioritized replay (alpha 0.6, beta 0.4)')
+    ap.add_argument('--n-step', type=int, default=None, help='DQN: n-step returns (default 1; Ape-X uses 3)')
     args = ap.parse_args(argv)
+    if args.algo != 'dqn' and (args.prioritized_replay or args.n_step is not None):
+        ap.error('--prioritized-replay and --n-step apply to --algo dqn')
     if args.algo == 'dqn':
         from .dqn import DQNConfig
-        kw = {k: v for k, v in (('minibatch_size', args.minibatch), ('lr', args.lr)) if v is not None}
+        kw = {k: v for k, v in (('minibatch_size', args.minibatch), ('lr', args.lr), ('n_step', args.n_step)) if v is not None}
+        if args.prioritized_replay:
+            kw['prioritized_replay'] = True
         tr = Trainer(args.part, args.envs, args.fragment, args.seed, config=DQNConfig(seed=args.seed, **kw), algo='dqn',
                      total_samples=args.samples)
     else:
