@@ -7,7 +7,8 @@
 Without an argument it trains for 10 iterations of 4096 environments x 100 steps (about 4 M env-steps, a few seconds
 on a B200) and writes /tmp/paintrl_door_ppo.pt; with one it loads that checkpoint instead, PPO or DQN
 (`python -m paintrl_b200.train --algo dqn ...`): for a DQN policy the argmax of the head's first n_out columns is the
-greedy Q action, up to the tie rule.
+greedy Q action, up to the tie rule.  A continuous checkpoint (`--action-mode continuous`) drives with its mean action;
+the gym.Env is set to the spaces the checkpoint records.
 """
 import os
 import sys
@@ -32,11 +33,20 @@ else:
     tr.close()
 
 policy = train.load_policy(path, device)
+spaces = train.checkpoint_spaces(torch.load(path, map_location='cpu', weights_only=False))
+PaintGymEnv.change_obs_mode(spaces['obs_mode'], spaces['obs_grad'])
+PaintGymEnv.change_action_mode(spaces['action_shape'], spaces['action_mode'], spaces['granularity'])
 env = PaintGymEnv('', with_robot=False, renders=False, rollout=True, extra_config=dict(DEFAULT_EXTRA_CONFIG))
 obs, done, total, steps = env.reset(), False, 0.0, 0
 while not done:
-    logits, _ = policy.forward(torch.as_tensor(obs, device=device)[None])
-    obs, reward, done, info = env.step(int(logits.argmax()))          # greedy action
+    out, _ = policy.forward(torch.as_tensor(obs, device=device)[None])
+    if policy.discrete:
+        action = int(out.argmax())                                    # greedy action
+    elif policy.dist == 'diag_gaussian':
+        action = out[0, :policy.action_dim].double().cpu().numpy()   # mean action
+    else:
+        action = torch.tanh(out[0]).double().cpu().numpy()
+    obs, reward, done, info = env.step(action)
     total += reward
     steps += 1
 print('gym.Env episode with the trained policy: %d steps, return %.2f, last info %s' % (steps, total, info))

@@ -391,6 +391,29 @@ int paintrl_adam_step(float *params_dev, const float *grad_dev, float *m_dev, fl
                       float beta1, float beta2, float eps, int32_t step, void *stream);
 
 /*
+ * PPO with a learned log-std (RLlib's DiagGaussian for a Box action space) on a continuous engine with n_out = 2 A:
+ * head column o is the mean mu_o and column A + o is log sigma_o of action dimension o < A, then the value.  Both calls
+ * return PAINTRL_E_INVALID for a discrete handle or an odd n_out.
+ *
+ * paintrl_policy_act_diag_gaussian: a_o = fl(fl(sigma_o z_o) + mu_o), sigma_o = expf(log sigma_o), z_o the Box-Muller
+ * draw paintrl_policy_act's continuous head uses (pol_uniform k = 2o, 2o + 1); no tanh and no clamp (the environment
+ * clips).  actions_dev float64 [batch, A] (FP32 values), logp_dev float32 [batch] = log N(a; mu, diag sigma^2) computed
+ * from those FP32 actions by the function the learner also uses, value_dev float32 [batch], logits_dev float32
+ * [batch, n_out + 1] or NULL.  Always samples; the bootstrap value comes from paintrl_policy_act with sample = 0.
+ *
+ * paintrl_ppo_grad_diag_gaussian: paintrl_ppo_grad's arguments and loss on this distribution, actions float64 [rows][A]:
+ * KL(old || new) = sum_o (log sigma_o - log sigma_old,o + (sigma_old,o^2 + (mu_old,o - mu_o)^2) / (2 sigma_o^2) - 1/2)
+ * and H = sum_o (log sigma_o + log(2 pi e) / 2).  The same six statistics; the first minibatch after a collection has
+ * ratios of exactly 1.
+ */
+int paintrl_policy_act_diag_gaussian(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, double *actions_dev, float *logp_dev,
+                                     float *value_dev, float *logits_dev, void *stream);
+int paintrl_ppo_grad_diag_gaussian(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                                   const void *actions_dev, const float *logp_old_dev, const float *value_old_dev,
+                                   const float *logits_old_dev, const float *adv_dev, const float *vtarg_dev, float kl_coeff,
+                                   float *grad_dev, float *stats_dev, void *stream);
+
+/*
  * Double DQN with a dueling head on the same network (RLlib DQN's dueling combination, without its extra hidden layer
  * per stream): the n_out head outputs are the advantages A, the value column is V, and Q(s, a) = V + A_a - mean_o A_o.
  * "Greedy" is the first maximum of Q (the lowest action index on ties), in the act kernel and in the target alike.

@@ -143,6 +143,8 @@ SIGNATURES = {
     'paintrl_ppo_forward': (ctypes.c_int, [_VP, _VP, _VP, _I32, _VP, _VP, _VP]),
     'paintrl_adam_step': (ctypes.c_int, [_VP, _VP, _VP, _VP, _I32, ctypes.c_float, ctypes.c_float, ctypes.c_float, ctypes.c_float, _I32, _VP]),
     'paintrl_policy_act_epsilon': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP, _VP]),
+    'paintrl_policy_act_diag_gaussian': (ctypes.c_int, [_VP, _VP, _I32, _VP, _VP, _VP, _VP, _VP]),
+    'paintrl_ppo_grad_diag_gaussian': (ctypes.c_int, [_VP, _VP, _VP, _I32] + [_VP] * 7 + [ctypes.c_float, _VP, _VP, _VP]),
     'paintrl_dqn_create': (ctypes.c_int, [ctypes.POINTER(PaintrlDqnConfig), _I32, ctypes.POINTER(_VP)]),
     'paintrl_dqn_destroy': (None, [_VP]),
     'paintrl_dqn_grad': (ctypes.c_int, [_VP, _VP, _VP, _VP, _I32] + [_VP] * 8),

@@ -1258,7 +1258,8 @@ int paintrl_policy_create(const PaintrlPolicyConfig *cfg, int32_t device, Paintr
               e->arena.alloc((void **)&pp.counters, sizeof(unsigned) * (size_t)cfg->capacity) == cudaSuccess;
     if (ok) ok = cudaMemset(pp.counters, 0, sizeof(unsigned) * (size_t)cfg->capacity) == cudaSuccess;
     with_caps(pp.obs_dim, pp.n_out, [&](auto mo, auto mx) {
-        ok = ok && opt_in_smem(policy_act_kernel<mo, mx, false>, kPolSmemBytes) && opt_in_smem(policy_act_kernel<mo, mx, true>, kPolSmemBytes);
+        ok = ok && opt_in_smem(policy_act_kernel<mo, mx, false>, kPolSmemBytes) && opt_in_smem(policy_act_kernel<mo, mx, true>, kPolSmemBytes) &&
+             (pp.discrete || opt_in_smem(policy_act_kernel<mo, mx, false, true>, kPolSmemBytes));
     });
     if (!ok) { delete e; cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the policy engine failed (allocation / shared memory opt-in)"); }
     *out = e;
@@ -1267,11 +1268,15 @@ int paintrl_policy_create(const PaintrlPolicyConfig *cfg, int32_t device, Paintr
 
 void paintrl_policy_destroy(PaintrlPolicyHandle h) { destroy_engine(h); }
 
-static int policy_launch(PaintrlPolicyHandle h, const PolicyIO &io, bool epsilon_greedy, void *stream) {
+// how policy_act_kernel picks actions: the engine's own head, epsilon-greedy (EPS) or the diagonal Gaussian (DIAG)
+enum PolicyMode { kActSample, kActEpsilon, kActDiag };
+
+static int policy_launch(PaintrlPolicyHandle h, const PolicyIO &io, PolicyMode mode, void *stream) {
     const dim3 pgrid((io.batch + kPolRows - 1) / kPolRows);
     cudaStream_t s = as_stream(stream);
     with_caps(h->pp.obs_dim, h->pp.n_out, [&](auto mo, auto mx) {
-        if (epsilon_greedy) policy_act_kernel<mo, mx, true><<<pgrid, kPolThreads, kPolSmemBytes, s>>>(h->pp, io);
+        if (mode == kActEpsilon) policy_act_kernel<mo, mx, true><<<pgrid, kPolThreads, kPolSmemBytes, s>>>(h->pp, io);
+        else if (mode == kActDiag) policy_act_kernel<mo, mx, false, true><<<pgrid, kPolThreads, kPolSmemBytes, s>>>(h->pp, io);
         else policy_act_kernel<mo, mx, false><<<pgrid, kPolThreads, kPolSmemBytes, s>>>(h->pp, io);
     });
     cudaError_t err = cudaGetLastError();
@@ -1291,7 +1296,7 @@ int paintrl_policy_act(PaintrlPolicyHandle h, const double *obs_dev, int32_t bat
     io.act_discrete = h->pp.discrete ? reinterpret_cast<long long *>(actions_dev) : nullptr;
     io.act_continuous = h->pp.discrete ? nullptr : reinterpret_cast<double *>(actions_dev);
     io.logp = logp_dev; io.value = value_dev; io.logits = logits_dev; io.sample = sample ? 1 : 0;
-    return policy_launch(h, io, false, stream);
+    return policy_launch(h, io, kActSample, stream);
 }
 
 int paintrl_policy_act_epsilon(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, void *actions_dev, float *value_dev,
@@ -1305,7 +1310,22 @@ int paintrl_policy_act_epsilon(PaintrlPolicyHandle h, const double *obs_dev, int
     io.obs = obs_dev; io.batch = batch;
     io.act_discrete = reinterpret_cast<long long *>(actions_dev);
     io.value = value_dev; io.logits = logits_dev; io.sample = 1; io.epsilon = epsilon_dev;
-    return policy_launch(h, io, true, stream);
+    return policy_launch(h, io, kActEpsilon, stream);
+}
+
+int paintrl_policy_act_diag_gaussian(PaintrlPolicyHandle h, const double *obs_dev, int32_t batch, double *actions_dev, float *logp_dev,
+                                     float *value_dev, float *logits_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (h->pp.discrete) return fail(PAINTRL_E_INVALID, "diagonal-Gaussian actions need a continuous policy engine");
+    if (h->pp.n_out % 2) return fail(PAINTRL_E_INVALID, "diagonal-Gaussian actions need an even n_out (a mean and a log-std per action dimension)");
+    if (!obs_dev || !actions_dev || !logp_dev || !value_dev) return fail(PAINTRL_E_INVALID, "null I/O buffer");
+    if (batch <= 0 || batch > h->capacity) return fail(PAINTRL_E_INVALID, "batch exceeds the policy engine's capacity");
+    CUDA_TRY(cudaSetDevice(h->device));
+    PolicyIO io{};
+    io.obs = obs_dev; io.batch = batch;
+    io.act_continuous = actions_dev;
+    io.logp = logp_dev; io.value = value_dev; io.logits = logits_dev; io.sample = 1;
+    return policy_launch(h, io, kActDiag, stream);
 }
 
 /* ---- the PPO learner, see paintrl_learn.cuh ---- */
@@ -1363,7 +1383,7 @@ static int learner_init(LearnerEngine *e, int device, int obs_dim, int n_out, in
               e->arena.alloc((void **)&e->partial_stats, sizeof(float) * (size_t)e->max_ctas * kLrnStatStride) == cudaSuccess;
     with_caps(obs_dim, n_out, [&](auto mo, auto mx) {
         ok = ok && opt_in_smem(ppo_grad_kernel<mo, mx, kLossPpo>, kLrnSmemBytes) && opt_in_smem(ppo_grad_kernel<mo, mx, kLossDqn>, kLrnSmemBytes) &&
-             opt_in_smem(ppo_grad_kernel<mo, mx, kLossDqnPer>, kLrnSmemBytes);
+             opt_in_smem(ppo_grad_kernel<mo, mx, kLossDqnPer>, kLrnSmemBytes) && opt_in_smem(ppo_grad_kernel<mo, mx, kLossPpoDiag>, kLrnSmemBytes);
     });
     if (!ok) { cudaGetLastError(); return fail(PAINTRL_E_CUDA, "setting up the learner failed (allocation / shared memory opt-in)"); }
     return PAINTRL_OK;
@@ -1383,6 +1403,7 @@ static int learner_launch(const PpoGradArgs &a, void *stream, int loss = kLossPp
     cudaStream_t s = as_stream(stream);
     with_caps(a.obs_dim, a.n_out, [&](auto mo, auto mx) {
         if (loss == kLossDqn) ppo_grad_kernel<mo, mx, kLossDqn><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
+        else if (loss == kLossPpoDiag) ppo_grad_kernel<mo, mx, kLossPpoDiag><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
         else if (loss == kLossDqnPer) ppo_grad_kernel<mo, mx, kLossDqnPer><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
         else ppo_grad_kernel<mo, mx, kLossPpo><<<grid, kPolThreads, kLrnSmemBytes, s>>>(a);
     });
@@ -1417,10 +1438,10 @@ int paintrl_ppo_create(const PaintrlPpoConfig *cfg, int32_t device, PaintrlPpoHa
 
 void paintrl_ppo_destroy(PaintrlPpoHandle h) { destroy_engine(h); }
 
-int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
-                     const void *actions_dev, const float *logp_old_dev, const float *value_old_dev, const float *logits_old_dev,
-                     const float *adv_dev, const float *vtarg_dev, float kl_coeff, float *grad_dev, float *stats_dev, void *stream) {
-    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+// paintrl_ppo_grad (loss kLossPpo) and paintrl_ppo_grad_diag_gaussian (kLossPpoDiag), after their handle checks
+static int ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                    const void *actions_dev, const float *logp_old_dev, const float *value_old_dev, const float *logits_old_dev,
+                    const float *adv_dev, const float *vtarg_dev, float kl_coeff, float *grad_dev, float *stats_dev, void *stream, int loss) {
     if (!params_dev || !idx_dev || !obs_dev || !actions_dev || !logp_old_dev || !value_old_dev || !logits_old_dev || !adv_dev ||
         !vtarg_dev || !grad_dev || !stats_dev)
         return fail(PAINTRL_E_INVALID, "null buffer");
@@ -1433,9 +1454,28 @@ int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t 
     a.adv = adv_dev; a.vtarg = vtarg_dev;
     a.clip = h->cfg.clip_param; a.vf_clip = h->cfg.vf_clip_param; a.vf_coeff = h->cfg.vf_loss_coeff; a.ent_coeff = h->cfg.entropy_coeff;
     a.kl_coeff = kl_coeff; a.inv_n = 1.f / (float)n;
-    int rc = learner_launch(a, stream);
+    int rc = learner_launch(a, stream, loss);
     if (rc != PAINTRL_OK) return rc;
     return learner_reduce(h, n, a.inv_n, grad_dev, stats_dev, kLrnStats, stream);
+}
+
+int paintrl_ppo_grad(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                     const void *actions_dev, const float *logp_old_dev, const float *value_old_dev, const float *logits_old_dev,
+                     const float *adv_dev, const float *vtarg_dev, float kl_coeff, float *grad_dev, float *stats_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    return ppo_grad(h, params_dev, idx_dev, n, obs_dev, actions_dev, logp_old_dev, value_old_dev, logits_old_dev, adv_dev, vtarg_dev,
+                    kl_coeff, grad_dev, stats_dev, stream, kLossPpo);
+}
+
+int paintrl_ppo_grad_diag_gaussian(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,
+                                   const void *actions_dev, const float *logp_old_dev, const float *value_old_dev,
+                                   const float *logits_old_dev, const float *adv_dev, const float *vtarg_dev, float kl_coeff,
+                                   float *grad_dev, float *stats_dev, void *stream) {
+    if (!h) return fail(PAINTRL_E_INVALID, "null handle");
+    if (h->cfg.discrete) return fail(PAINTRL_E_INVALID, "the diagonal-Gaussian loss needs a continuous learner handle");
+    if (h->n_out % 2) return fail(PAINTRL_E_INVALID, "the diagonal-Gaussian loss needs an even n_out (a mean and a log-std per action dimension)");
+    return ppo_grad(h, params_dev, idx_dev, n, obs_dev, actions_dev, logp_old_dev, value_old_dev, logits_old_dev, adv_dev, vtarg_dev,
+                    kl_coeff, grad_dev, stats_dev, stream, kLossPpoDiag);
 }
 
 int paintrl_ppo_forward(PaintrlPpoHandle h, const float *params_dev, const int32_t *idx_dev, int32_t n, const double *obs_dev,

@@ -32,6 +32,13 @@
 // kLossDqnPer is kLossDqn with a per-sample importance weight w (prioritized replay, paintrl_replay.cuh): g =
 // (clamp(td, -1, 1) * w) * inv_n, so w = 1 gives kLossDqn's bits; the Huber statistic is weighted the same way, a fifth
 // statistic is w, and td goes to td_out in minibatch order for the priority update.
+// kLossPpoDiag is kLossPpo on the diagonal-Gaussian head of A = n_out / 2 dimensions (RLlib's DiagGaussian; mean in
+// column o, log sigma in column A + o, actions float64 [rows][A]): logp from pol_diag_logp (the act kernel's own
+// function), KL(old || new) = sum (log sigma - log sigma_old + (sigma_old^2 + (mu_old - mu)^2) / (2 sigma^2) - 1/2),
+// H = sum (log sigma + log(2 pi e) / 2), and per dimension, with q = (sigma_old^2 + (mu - mu_old)^2) / sigma^2,
+//   dout[mu]        = s (g_logp u / sigma + kl_coeff (mu - mu_old) / sigma^2)
+//   dout[log sigma] = s (g_logp (u^2 - 1) + kl_coeff (1 - q) - ent_coeff)
+// The clipped surrogate, the value loss and the six statistics are kLossPpo's.
 //
 // Parameters arrive flat, in pol_num_params' layout (paintrl_policy.cuh).
 #pragma once
@@ -43,7 +50,7 @@ constexpr int kLrnStats = 6;                   // policy loss, value loss, KL, e
 constexpr int kDqnStats = 4;                   // Huber loss, |td|, Q(s, a), target y
 constexpr int kDqnPerStats = 5;                // weighted Huber loss, |td|, Q(s, a), target y, importance weight
 constexpr int kLrnStatStride = 8;
-constexpr int kLossPpo = 0, kLossDqn = 1, kLossDqnPer = 2;
+constexpr int kLossPpo = 0, kLossDqn = 1, kLossDqnPer = 2, kLossPpoDiag = 3;
 
 struct PpoGradArgs {
     int obs_dim, n_out, discrete, n, nparams;
@@ -51,7 +58,7 @@ struct PpoGradArgs {
     const float *params;                       // flat FP32 parameters
     const int *idx;                            // [n] rows of the flattened fragment
     const double *obs;                         // [rows][obs_dim]
-    const void *actions;                       // int64 [rows] (discrete) | float64 [rows][n_out]
+    const void *actions;                       // int64 [rows] (discrete) | float64 [rows][n_out] | [rows][n_out / 2] (kLossPpoDiag)
     const float *logp_old, *value_old, *logits_old, *adv, *vtarg;   // [rows], logits_old [rows][n_out + 1]
     float clip, vf_clip, vf_coeff, ent_coeff, kl_coeff, inv_n;
     float *partial;                            // [gridDim.x][nparams]
@@ -157,7 +164,7 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
         if (valid && a.forward_only) {
 #pragma unroll
             for (int o = 0; o < MX; ++o) if (o < nout1) a.fwd_out[(size_t)j * nout1 + o] = out[o];
-        } else if (valid && LOSS != kLossPpo) {
+        } else if (valid && (LOSS == kLossDqn || LOSS == kLossDqnPer)) {
             const int act = (int)reinterpret_cast<const long long *>(a.actions)[src];
             float q[MX], nx[MX], qn[MX];
             dqn_q_values<MX>(out, a.n_out, q);
@@ -208,7 +215,30 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
             float logp = 0.f, kl = 0.f, ent = 0.f;
             float lse = 0.f, lseo = 0.f;
             int act = 0;
-            if (a.discrete) {
+            // kLossPpoDiag: the row's head in its sdout slots (mu at [o], log sigma at [A + o]), its FP32 actions in ad
+            float *head = sdout + row * kPolMaxOut;
+            const int adim = a.n_out >> 1;
+            const float *lgo = a.logits_old + (size_t)src * nout1;
+            float ad[MX / 2];
+            if (LOSS == kLossPpoDiag) {
+#pragma unroll
+                for (int o = 0; o < MX; ++o) if (o < nout1) head[o] = out[o];
+                const double *ac = reinterpret_cast<const double *>(a.actions) + (size_t)src * adim;
+#pragma unroll
+                for (int o = 0; o < MX / 2; ++o) ad[o] = o < adim ? (float)ac[o] : 0.f;
+                logp = pol_diag_logp<MX>(head, ad, adim);
+#pragma unroll
+                for (int o = 0; o < MX / 2; ++o) {
+                    if (o < adim) {
+                        const float mu = head[o], ls = head[adim + o], muo = __ldg(&lgo[o]), lso = __ldg(&lgo[adim + o]);
+                        const float sig = pol_diag_sigma(ls), sigo = pol_diag_sigma(lso);
+                        const float d = mu - muo;
+                        const float q = (sigo * sigo + d * d) / (sig * sig);
+                        kl += ((ls - lso) + 0.5f * q) - 0.5f;
+                        ent += ls + 1.4189385332046727f;             // log sigma + log(2 pi e) / 2
+                    }
+                }
+            } else if (a.discrete) {
                 // log-softmax exactly as policy_act_kernel computes the sampled action's log-probability
                 float mx = -INFINITY, mo = -INFINITY;
 #pragma unroll
@@ -253,6 +283,26 @@ __global__ void __launch_bounds__(kPolThreads, 1) ppo_grad_kernel(PpoGradArgs a)
             const float vf2 = (vcl - R) * (vcl - R);
             const float g_v = vf1 >= vf2 ? 2.f * (v - R) : (fabsf(dv) <= a.vf_clip ? 2.f * (vcl - R) : 0.f);
             const float s = a.inv_n;
+            if (LOSS == kLossPpoDiag) {
+#pragma unroll
+                for (int o = 0; o < MX / 2; ++o) {
+                    if (o < adim) {
+                        const float mu = head[o], ls = head[adim + o], muo = __ldg(&lgo[o]), lso = __ldg(&lgo[adim + o]);
+                        const float sig = pol_diag_sigma(ls), sigo = pol_diag_sigma(lso);
+                        const float u = __fdiv_rn(__fsub_rn(ad[o], mu), sig);
+                        const float d = mu - muo;
+                        const float is2 = 1.f / (sig * sig);
+                        const float q = (sigo * sigo + d * d) * is2;
+                        head[o] = s * (g_logp * (u / sig) + a.kl_coeff * (d * is2));
+                        head[adim + o] = s * ((g_logp * (u * u - 1.f) + a.kl_coeff * (1.f - q)) - a.ent_coeff);
+                    }
+                }
+#pragma unroll
+                for (int o = 0; o < MX; ++o) {
+                    if (o < a.n_out) dout[o] = head[o];
+                    else if (o == a.n_out) dout[o] = s * a.vf_coeff * g_v;
+                }
+            } else
 #pragma unroll
             for (int o = 0; o < MX; ++o) {
                 if (o < a.n_out) {

@@ -13,9 +13,10 @@
 //            activations, B = the weights (pre-packed by the host in the same canonical layout, brought in with one
 //            cp.async.bulk), accumulator in TMEM (128 lanes x 128 columns)
 //   epilogue tcgen05.ld of each thread's row, + bias, tanh, the 128 x (n_out + 1) head in FP32 FFMA
-//   sampling discrete: Gumbel-max over the logits; continuous: tanh(mean) + unit Gaussian noise; log-probability and
-//            value; counter-based random numbers (per-environment counters in device memory, so a captured CUDA graph
-//            draws fresh noise on every replay)
+//   sampling discrete: Gumbel-max over the logits; continuous: tanh(mean) + unit Gaussian noise, or mean + sigma x unit
+//            noise with a learned log-std (the DIAG instantiations); log-probability and value; counter-based random
+//            numbers (per-environment counters in device memory, so a captured CUDA graph draws fresh noise on every
+//            replay)
 //
 // Shared-memory operand layout (no swizzle, K-major; cute::UMMA "INTERLEAVE"): 8 x 8 BF16 core matrices of 128
 // contiguous bytes (row r at +16 r); core (mi, kj) of an [rows x 256] operand sits at kj * (rows / 8) * 128 + mi * 128,
@@ -47,7 +48,7 @@ struct PolicyIO {
     const double *obs;        // [B][obs_dim]
     int batch;
     long long *act_discrete;  // [B]               (discrete)
-    double *act_continuous;   // [B][n_out]        (continuous)
+    double *act_continuous;   // [B][n_out]        (continuous; [B][n_out / 2] for DIAG)
     float *logp, *value;      // [B]
     float *logits;            // [B][n_out + 1] or nullptr (tests)
     int sample;               // 0: value / logits only (bootstrap), 1: sample actions
@@ -271,6 +272,29 @@ __device__ __forceinline__ int dqn_q_values(const float *out, int n_out, float *
     return arg;
 }
 
+// The head read as a diagonal Gaussian over A = n_out / 2 action dimensions (RLlib's DiagGaussian): mean mu_o in
+// column o, log sigma_o in column A + o.  `head` is the row's outputs in shared memory, so the runtime column offset A
+// needs no dynamic register indexing.  The act kernel and the learner's kLossPpoDiag stage both call these two
+// functions; with explicit round-to-nearest operations (never contracted into FMAs) they give the same bits in both
+// kernels, so the first PPO minibatch after a collection sees ratios of exactly 1.
+__device__ __forceinline__ float pol_diag_sigma(float log_sigma) { return expf(log_sigma); }
+
+// log N(a; mu, diag sigma^2) = sum over o, in order, of (-u_o^2 / 2 - log sigma_o), u_o = (a_o - mu_o) / sigma_o, then
+// minus A log(2 pi) / 2
+template <int MX>
+__device__ __forceinline__ float pol_diag_logp(const float *head, const float (&a)[MX / 2], int A) {
+    float lp = 0.f;
+#pragma unroll
+    for (int o = 0; o < MX / 2; ++o) {
+        if (o < A) {
+            const float ls = head[A + o];
+            const float u = __fdiv_rn(__fsub_rn(a[o], head[o]), pol_diag_sigma(ls));
+            lp = __fsub_rn(__fsub_rn(lp, __fmul_rn(__fmul_rn(0.5f, u), u)), ls);
+        }
+    }
+    return __fsub_rn(lp, __fmul_rn((float)A, 0.9189385332046727f));
+}
+
 // dynamic shared memory: A (64 KB) | B (64 KB) | w1 | b1 | b2 | w3 | b3 | barriers
 // MO / MX: compile-time caps of the observation and output loops (register arrays, fully unrolled): 8 / 8 for the
 // reference's spaces (6-18 observations are 8 or 32; 4 logits + value), 32 / 16 in general.  The shared-memory layout
@@ -279,7 +303,11 @@ __device__ __forceinline__ int dqn_q_values(const float *out, int n_out, float *
 // the environment's counter decides (explore when pol_uniform(.., 0) < *io.epsilon), draw k = 1 picks the random
 // action min((int)(pol_uniform(.., 1) * n_out), n_out - 1); otherwise the action is dqn_q_values' greedy one.  logp
 // is not written.
-template <int MO, int MX, bool EPS = false>
+// DIAG: the diagonal-Gaussian head (continuous engines with an even n_out, PPO with a learned log-std).  For each of
+// the A = n_out / 2 dimensions, z is the Box-Muller draw of the N(tanh mu, I) head (k = 2o, 2o + 1) and the action is
+// a = fl(fl(sigma z) + mu), no tanh and no clamp; A actions per row go to act_continuous, and logp is pol_diag_logp
+// of those FP32 actions.
+template <int MO, int MX, bool EPS = false, bool DIAG = false>
 __global__ void __launch_bounds__(kPolThreads, 1) policy_act_kernel(PolicyParams pp, PolicyIO io) {
     extern __shared__ __align__(1024) unsigned char pol_smem[];
     unsigned char *sA = pol_smem;
@@ -359,6 +387,27 @@ __global__ void __launch_bounds__(kPolThreads, 1) policy_act_kernel(PolicyParams
         if (pol_uniform(pp.seed, (unsigned)env, ctr, 0u) < __ldg(io.epsilon))
             act = min((int)(pol_uniform(pp.seed, (unsigned)env, ctr, 1u) * (float)pp.n_out), pp.n_out - 1);
         io.act_discrete[env] = act;
+        return;
+    }
+    if constexpr (DIAG) {
+        // the row's head into its first partial-head slot, free since the combine
+        float *head = spart + (size_t)row * kPolMaxOut;
+#pragma unroll
+        for (int o = 0; o < MX; ++o) if (o < nout1) head[o] = out[o];
+        const int A = pp.n_out >> 1;
+        float a[MX / 2];
+#pragma unroll
+        for (int o = 0; o < MX / 2; ++o) {
+            a[o] = 0.f;
+            if (o < A) {
+                const float u1 = pol_uniform(pp.seed, (unsigned)env, ctr, (unsigned)(2 * o));
+                const float u2 = pol_uniform(pp.seed, (unsigned)env, ctr, (unsigned)(2 * o + 1));
+                const float z = sqrtf(-2.f * __logf(u1)) * __cosf(6.2831853071795865f * u2);      // Box-Muller
+                a[o] = __fadd_rn(__fmul_rn(pol_diag_sigma(head[A + o]), z), head[o]);
+                io.act_continuous[(size_t)env * A + o] = (double)a[o];
+            }
+        }
+        io.logp[env] = pol_diag_logp<MX>(head, a, A);
         return;
     }
     if (pp.discrete) {

@@ -98,6 +98,7 @@ class Learner(object):
         if self.device.type != 'cuda':
             raise ValueError('the learner runs on a CUDA device (no CPU fallback)')
         self.obs_dim, self.n_out, self.discrete = policy.obs_dim, policy.n_out, bool(policy.discrete)
+        self.dist = getattr(policy, 'dist', None) or ('categorical' if self.discrete else 'tanh_gaussian')
         self._lib = _capi.lib()
         self.n_params = num_params(self.obs_dim, self.n_out)
         self.params = flat_params(policy).to(self.device)

@@ -77,8 +77,10 @@ class PPOLearner(Learner):
         return out
 
     def grad_into(self, rows, idx, kl_coeff, grad, stats):
-        """One `paintrl_ppo_grad` call: `rows` is the dict `flatten()` returns."""
-        _capi.check(self._lib.paintrl_ppo_grad(
+        """One `paintrl_ppo_grad` call (`paintrl_ppo_grad_diag_gaussian` for a diagonal-Gaussian policy): `rows` is the
+        dict `flatten()` returns."""
+        fn = self._lib.paintrl_ppo_grad_diag_gaussian if self.dist == 'diag_gaussian' else self._lib.paintrl_ppo_grad
+        _capi.check(fn(
             self._h, _ptr(self.params), _ptr(idx), idx.numel(), _ptr(rows['obs']), _ptr(rows['actions']), _ptr(rows['logp']),
             _ptr(rows['value']), _ptr(rows['logits']), _ptr(rows['adv']), _ptr(rows['vtarg']), float(kl_coeff), _ptr(grad),
             _ptr(stats), self._stream()))
@@ -126,16 +128,25 @@ class PPOLearner(Learner):
         return out
 
     def state_dict(self):
-        return dict(self._state_dict(), kl_coeff=float(self.kl_coeff))
+        return dict(self._state_dict(), kl_coeff=float(self.kl_coeff), dist=self.dist)
 
     def load_state_dict(self, sd):
-        check_state_dict(sd, self.obs_dim, self.n_out, self.discrete)
+        check_state_dict(sd, self.obs_dim, self.n_out, self.discrete, self.dist)
         self.kl_coeff = float(sd['kl_coeff'])
         self._load_state_dict(sd)
 
 
-def check_state_dict(sd, obs_dim, n_out, discrete):
-    """Raise ValueError when a learner state does not fit a policy of this shape."""
+def state_dist(sd):
+    """The action distribution a PPO learner state was trained with; states written before `dist` was recorded hold
+    the distribution every policy had then."""
+    return sd.get('dist') or ('categorical' if sd.get('discrete') else 'tanh_gaussian')
+
+
+def check_state_dict(sd, obs_dim, n_out, discrete, dist=None):
+    """Raise ValueError when a learner state does not fit a policy of this shape (and of distribution `dist`, when
+    given)."""
     _check_state_dict(sd, obs_dim, n_out, discrete, ('params', 'adam_m', 'adam_v'))
     if not float(sd['kl_coeff']) >= 0.0:
         raise ValueError('kl_coeff must be non-negative')
+    if dist is not None and state_dist(sd) != dist:
+        raise ValueError('checkpoint is for the %s distribution, not %s' % (state_dist(sd), dist))

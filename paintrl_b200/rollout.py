@@ -71,6 +71,17 @@ class NativePolicy(object):
         _capi.check(self._lib.paintrl_policy_act_epsilon(self._h, p(obs), B, p(actions), p(value), p(logits), p(epsilon),
                                                          ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
 
+    def act_diag_gaussian_into(self, obs, actions, logp, value, logits=None):
+        """Sample the diagonal-Gaussian head (`paintrl_policy_act_diag_gaussian`, continuous engines with an even n_out):
+        head columns [0, A) are the means and [A, 2A) the log-stds, A = n_out / 2; actions float64 [B, A] hold the FP32
+        values mean + std * noise, and logp is their log-probability as the learner computes it."""
+        if self.discrete or self.n_out % 2:
+            raise ValueError('diagonal-Gaussian actions need a continuous policy with an even n_out')
+        B = obs.shape[0]
+        p = lambda t: None if t is None else ctypes.c_void_p(t.data_ptr())
+        _capi.check(self._lib.paintrl_policy_act_diag_gaussian(self._h, p(obs), B, p(actions), p(logp), p(value), p(logits),
+                                                               ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
+
     def set_params(self, params):
         """Pack a flat FP32 parameter vector (w1 | b1 | w2 | b2 | w3 | b3, a contiguous CUDA tensor of this device) into
         this engine's device weights, in place and on the current stream: a captured rollout graph samples with the new
@@ -79,13 +90,31 @@ class NativePolicy(object):
                                                         ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)))
 
 
+DISTS = ('categorical', 'tanh_gaussian', 'diag_gaussian')
+
+
+def default_dist(discrete):
+    """The distribution of a policy built without `dist`: what every policy was before `dist` existed."""
+    return 'categorical' if discrete else 'tanh_gaussian'
+
+
 class MlpPolicy(object):
     """Fully connected policy of paint_ppo.py:179-183: obs -> 256 -> 128 -> {logits | mean, value},
     tanh activations (RLlib's fcnet default), value branch sharing the hidden layers
-    (`vf_share_layers`).  Random-init FP32 weights; discrete actions are sampled with the Gumbel-max
-    trick, continuous ones from a unit-variance Gaussian around tanh(mean)."""
+    (`vf_share_layers`).  Random-init FP32 weights.  `dist` names the action distribution:
+    'categorical' (discrete; Gumbel-max sampling of n_out logits), 'tanh_gaussian' (continuous; unit-variance
+    Gaussian around tanh(mean), n_out means) or 'diag_gaussian' (continuous; RLlib's DiagGaussian, mean + exp(log_std)
+    noise with a learned log-std: `n_out` is then the action dimension A, and the head has 2A outputs, means then
+    log-stds, so `self.n_out` is 2A and `self.action_dim` is A)."""
 
-    def __init__(self, obs_dim, n_out, hiddens=(256, 128), device=None, seed=0, discrete=True):
+    def __init__(self, obs_dim, n_out, hiddens=(256, 128), device=None, seed=0, discrete=True, dist=None):
+        dist = default_dist(discrete) if dist is None else dist
+        if dist not in DISTS or (dist == 'categorical') != bool(discrete):
+            raise ValueError('dist %r does not fit discrete=%r (categorical is the discrete one)' % (dist, discrete))
+        self.dist = dist
+        self.action_dim = int(n_out) if not discrete else 1
+        if dist == 'diag_gaussian':
+            n_out = 2 * int(n_out)
         gen = torch.Generator(device='cpu')
         gen.manual_seed(seed)
         dims = [obs_dim] + list(hiddens)
@@ -138,6 +167,13 @@ class MlpPolicy(object):
     def act(self, obs):
         """Sample one action per environment: (actions, log-probability, value)."""
         out, value = self.forward(obs)
+        if self.dist == 'diag_gaussian':
+            A = self.action_dim
+            mean, log_std = out[:, :A], out[:, A:]
+            noise = torch.randn(mean.shape, generator=self.gen, device=out.device)
+            a = mean + torch.exp(log_std) * noise
+            logp = (-0.5 * noise * noise - log_std).sum(dim=1) - A * 0.5 * math.log(2 * math.pi)
+            return a.to(torch.float64), logp, value
         if self.discrete:
             logp_all = torch.log_softmax(out, dim=1)
             u = torch.rand(out.shape, generator=self.gen, device=out.device).clamp_(1e-10, 1.0)
@@ -187,6 +223,10 @@ class RolloutWorker(object):
         `fragment.logp` is not written.  Needs the native policy and discrete actions."""
         if not env.cfg.auto_reset:
             raise ValueError('RolloutWorker needs an environment created with auto_reset=True')
+        self.diag = getattr(policy, 'dist', None) == 'diag_gaussian'
+        if self.diag and (env.cfg.action_mode != 'continuous' or policy.action_dim != env.action_dim):
+            raise ValueError('a diagonal-Gaussian policy of %d action dimensions does not fit this environment (%s, %d)'
+                             % (policy.action_dim, env.cfg.action_mode, env.action_dim))
         self.env, self.policy, self.T = env, policy, int(fragment_length)
         if use_native_policy and hasattr(policy, 'enable_native'):
             policy.enable_native(env.num_envs)
@@ -229,6 +269,8 @@ class RolloutWorker(object):
         for t in range(self.T):
             if native is not None and self.epsilon is not None:
                 native.act_epsilon_into(f.obs[t], f.actions[t], f.value[t], self.epsilon, logits=None if f.logits is None else f.logits[t])
+            elif native is not None and self.diag:
+                native.act_diag_gaussian_into(f.obs[t], f.actions[t], f.logp[t], f.value[t], logits=None if f.logits is None else f.logits[t])
             elif native is not None:
                 # one launch: obs[t] -> actions[t], logp[t], value[t] written in place (no torch kernels in the loop)
                 native.act_into(f.obs[t], f.actions[t], f.logp[t], f.value[t], logits=None if f.logits is None else f.logits[t])
